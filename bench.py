@@ -44,6 +44,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the tree may be read-only: no __pycache__ next to the sources this imports
 
 METRIC = "Mrays/s @1080p x16spp, 8 bounces"
 UNIT = "Mrays/s"
@@ -76,10 +77,16 @@ def parse_args():
     ap.add_argument("--exchange", default="auto", choices=["auto", "peer", "gather"],
                     help="N > 1: fused peer/multicast stores from the render kernel, or NCCL all-gather + scatter")
     ap.add_argument("--flags", type=int, default=0, help="MM_FLAG_* for experiments (2 = literal divides for every ray, 64 = reciprocal-multiply slab arithmetic)")
-    ap.add_argument("--frames", type=int, default=120, help="cfg5: frames per fly-through")
     ap.add_argument("--screen", default="f32", choices=["f32", "rgba8"],
                     help="cfg5: fp32 screen and frames (default), or the reference's RGBA8Unorm screen: quantised stores, 4-byte texels read back")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the frame the last timed step computed as DIR/<name>.npy (float32), "
+                         "to compare two builds output for output")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path (--impl ours)")
     w = WORKLOADS[a.workload]
     for k in ("maze", "width", "height", "spp", "bounces"):
         if getattr(a, k) is None:
@@ -153,6 +160,28 @@ N_CORES = len(os.sched_getaffinity(0))       # the host cores this process may u
 
 def sha(a):
     return hashlib.sha256(memoryview(a).cast("B")).hexdigest()
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: each array as out_dir/<name>.npy in float32, at most DUMP_BYTES in all.  An array over its share
+    (a 4K frame) is stored as a fixed seeded sample of its pixels, [n, channels], with their flat pixel indices beside it
+    as <name>_index.npy (float64, exact)."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // len(arrays) - 4096                    # room for the .npy headers
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, dtype=np.float32)
+        if a.nbytes > share:
+            px = a.reshape(-1, a.shape[-1])
+            n = share // (px.shape[1] * 4 + 8)
+            idx = np.sort(np.random.default_rng(0).choice(len(px), n, replace=False))
+            np.save(os.path.join(out_dir, f"{name}_index.npy"), idx.astype(np.float64))
+            a = px[idx]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 # ---- CPU legs (oracle; the only place bench.py executes oracle/) -----------------------------------------------------------
@@ -393,6 +422,8 @@ def run_ours(a):
         sampler.start()
     step_ms, kernel_mean, rays_timed = time_frames(r, frame, u, a.steps, a.warmup, flush, dist, torch)
     clocks = sampler.stop() if sampler else None
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, {"frame": frame.image.cpu().numpy()})        # the last timed step's whole frame
     total_ms = torch.tensor([sum(step_ms)], dtype=torch.float64, device=dev)
     rays_all = torch.tensor([float(rays_timed)], dtype=torch.float64, device=dev)
     keys = ("paths", "rays", "inner_visits", "leaf_visits", "rect_tests", "hits", "literal_rays")
@@ -700,7 +731,8 @@ def run_flythroughs(a, mm, torch, dist, rank, world, local):
     across the GPUs (no exchange until the final collect).  One fly-through = the reference's frame loop (reference
     src/main.rs:767-895) run headless: scripted WASD + yaw -> mm_move_camera (collision) / mm_update_quat_angle -> pop 1/64 of the
     screen's chunk origins (progressive refresh, main.rs:778-784) -> mm_render into the persistent screen -> mm_present (5-tap
-    blur) -> frame read back to pinned host memory.  A step = one frame on every GPU; --steps is ignored, --frames counts."""
+    blur) -> frame read back to pinned host memory.  A step = one frame on every GPU: --warmup untimed frames, then the
+    fly-through again from its start for --steps timed frames."""
     import math
     import numpy as np
 
@@ -757,12 +789,21 @@ def run_flythroughs(a, mm, torch, dist, rank, world, local):
         r.wait_present()
         return rays
 
+    if a.warmup:
+        fly(rank, a.warmup)
     if dist is not None:
         dist.barrier()
     torch.cuda.synchronize()
     t0 = time.perf_counter()
-    rays = fly(rank, a.frames)
+    rays = fly(rank, a.steps)
     dt = time.perf_counter() - t0
+    if a.dump_outputs and rank == 0:
+        last = hf if (a.steps - 1) & 1 else hf2                                  # the alternating read-back frames
+        if rgba8:
+            H, W = a.height, a.width
+            dump_outputs(a.dump_outputs, {"texels": last.array.reshape(-1).view(np.uint8)[:H * W * 4].reshape(H, W, 4)})
+        else:
+            dump_outputs(a.dump_outputs, {"frame": last.array})
     # parity: the first 3 frames of this rank's fly-through against the oracle + the blur model, on a fresh renderer state —
     # AFTER the timed run: the oracle's OpenMP workers keep spinning for a while and would steal the cores the frame loop needs
     parity_ok = None
@@ -797,7 +838,7 @@ def run_flythroughs(a, mm, torch, dist, rank, world, local):
         r.upload_scene(sc, noise)
         fly(rank, 3, check)
         parity_ok = ok[0]
-    tot = np.array([rays, a.frames, dt, 1.0 if parity_ok in (True, None) else 0.0], dtype=np.float64)
+    tot = np.array([rays, a.steps, dt, 1.0 if parity_ok in (True, None) else 0.0], dtype=np.float64)
     if dist is not None:
         t = torch.tensor(tot, device=f"cuda:{local}")
         mx, mn = t.clone(), t.clone()
@@ -808,9 +849,9 @@ def run_flythroughs(a, mm, torch, dist, rank, world, local):
         dist.destroy_process_group()
     if rank == 0:
         print(json.dumps({"metric": "frames/s, fly-throughs with temporal accumulation (BASELINE configs[4])", "value": round(tot[1] / tot[2], 2), "unit": "frames/s",
-                          "n_gpus": world, "steps": int(a.frames), "warmup": 0, "ms_per_step": round(1e3 * tot[2] / a.frames, 4), "higher_is_better": True,
+                          "n_gpus": world, "steps": a.steps, "warmup": a.warmup, "ms_per_step": round(1e3 * tot[2] / a.steps, 4), "higher_is_better": True,
                           "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
-                          "config": {"workload": f"{world} fly-through(s) x {a.frames} frames, {a.maze}x{a.maze} maze, {a.width}x{a.height}, {a.spp} spp, {a.bounces} bounces, "
+                          "config": {"workload": f"{world} fly-through(s) x {a.steps} frames, {a.maze}x{a.maze} maze, {a.width}x{a.height}, {a.spp} spp, {a.bounces} bounces, "
                                                  f"1/64 of the screen ({per_frame} chunks) re-rendered per frame + 5-tap present blur, every frame read back to pinned host memory "
                                                  f"(mm_present_async: the read-back overlaps the next frame's dispatch)",
                                      "workload_id": "cfg5", "parallelism": "one fly-through per GPU, no exchange until the final collect"},
@@ -819,7 +860,7 @@ def run_flythroughs(a, mm, torch, dist, rank, world, local):
                           "screen": "RGBA8Unorm like the reference's (main.rs:702-709): quantised stores, texel bytes read back" if rgba8 else "fp32",
                           "e2e": {"value": round(tot[1] / tot[2], 2), "unit": "frames/s", "h2d_bytes_per_step": per_frame * 8 + 92,
                                   "d2h_bytes_per_step": a.width * a.height * (4 if rgba8 else 16)},
-                          "gpu_launches": int(2 * a.frames)}), flush=True)
+                          "gpu_launches": int(2 * a.steps)}), flush=True)
     return 0
 
 

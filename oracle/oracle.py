@@ -3,12 +3,14 @@
 import ctypes as C
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB = os.path.join(_HERE, "libmm_oracle.so")
 _lib = None
+_native_dir = None
 
 
 class _Counters(C.Structure):
@@ -51,13 +53,15 @@ def lib():
 
 
 def use_native():
-    """bench.py only: build oracle/_native/libmm_oracle.so on THIS machine (g++ -march=native, same source, still no
-    contraction and no fast-math) and use it for every later call.  Returns a one-line description of what is in use.
-    Must run before the first lib() call of the process."""
-    global _LIB, _lib
-    native = os.path.join(_HERE, "_native", "libmm_oracle.so")
+    """bench.py only: build libmm_oracle.so for THIS machine (g++ -march=native, same source, still no contraction and
+    no fast-math) in a temporary directory, so that the tree may be read-only, and use it for every later call.  Returns
+    a one-line description of what is in use.  Must run before the first lib() call of the process."""
+    global _LIB, _lib, _native_dir
+    _native_dir = tempfile.TemporaryDirectory(prefix="mm_oracle_native_")       # removed when the process exits
+    native = os.path.join(_native_dir.name, "libmm_oracle.so")
     try:
-        subprocess.check_call(["make", "-C", _HERE, "-s", "native"], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+        subprocess.check_call(["make", "-C", _HERE, "-s", "native", f"NATIVE_DIR={_native_dir.name}"],
+                              stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
     except Exception as e:
         return f"portable build (native build failed: {type(e).__name__})"
     if _lib is not None or not os.path.exists(native):

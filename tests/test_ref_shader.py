@@ -138,11 +138,14 @@ def test_quat_mult_matches_reference_source(ref, oracle):
 
 
 @pytest.mark.parametrize("name", REF_SHADER_CASES)
-def test_oracle_image_equals_reference_shader_image(ref, oracle, mm, noise, scenes, name):
-    """Whole dispatches: every written pixel of the reference shader's fp32 image, bit for bit."""
+def test_oracle_image_equals_reference_shader_image(oracle, mm, noise, scenes, name):
+    """Whole dispatches: every written pixel of the reference shader's fp32 image, bit for bit.  Where the _ref library
+    is absent, the oracle's image stands in for it and the digest of the reference shader's image, committed with the
+    fixtures, is the comparison."""
+    from oracle import ref_shader
     sc, u, p, ch = build_case(mm, name, scenes)
-    want = ref.render(sc, noise, u, p, ch)
     got, cnt, _ = oracle.render(sc, noise, u, p, ch)
+    want = ref_shader.render(sc, noise, u, p, ch) if ref_shader.available() else got
     assert (want[..., 3] == 1).sum() == cnt["paths"] // p.spp            # every pixel of every chunk was written
     assert got.tobytes() == want.tobytes()
     assert hashlib.sha256(want.tobytes()).hexdigest() == GOLDEN[name]["ref_shader_image"]
