@@ -101,6 +101,9 @@ typedef struct mm_params {
                                       the block's live paths are re-formed into warps through shared memory, sorted by ray steepness
                                       |dir.y|, ended paths dropped.  Same bits; fewer instructions (-14 % interior-body executions) but
                                       measured slower on B200 (profiles/r2_experiments.md), kept as the evidence for that design    */
+#define MM_FLAG_NO_TAIL     4096u   /* trace every path to its end in the one-thread-per-path kernel (for comparisons; same bits).  By
+                                      default a warp that is past bounce_limit segments with at most 8 live lanes hands those paths to
+                                      a second kernel that runs them densely, one thread per path (render_kernel.cu, DESIGN.md §4)  */
 
 /* Exact event counts of one render call; identical on CPU oracle and GPU (SURVEY §8 d). */
 typedef struct mm_counters {
@@ -246,8 +249,12 @@ int mm_sync(mm_ctx *ctx);
 int mm_set_stream(mm_ctx *ctx, void *stream);
 /* Counters of the most recent render launch; waits for that launch's (asynchronous) counter copy, not for the stream. */
 int mm_last_counters(mm_ctx *ctx, mm_counters *out);
-/* Device time of the most recent render kernel in milliseconds (CUDA events on the context's stream). */
+/* Device time of the most recent render launch in milliseconds (CUDA events on the context's stream, around the trace kernel
+ * and, unless MM_FLAG_NO_TAIL, the straggler kernel after it). */
 int mm_last_ms(mm_ctx *ctx, float *ms);
+/* Straggler tail of the most recent render launch: paths the trace kernel queued for the second kernel, and pixels whose delivery
+ * was deferred to it.  Both 0 under MM_FLAG_NO_TAIL.  Waits like mm_last_counters. */
+int mm_last_tail(mm_ctx *ctx, uint64_t *queued_paths, uint64_t *deferred_pixels);
 /* The context's cudaStream_t, for callers that order their own work (NCCL, torch) after the kernel. */
 int mm_stream(mm_ctx *ctx, void **stream);
 /* Static facts of the loaded scene / selected kernel (for reports). */

@@ -19,6 +19,7 @@ FLAG_POOL_KERNEL = 256
 FLAG_SCREEN_RGBA8 = 512
 FLAG_REGROUP = 1024
 FLAG_GENERAL_RECTS = 2048
+FLAG_NO_TAIL = 4096
 EXCHANGE_PEER, EXCHANGE_NCCL, EXCHANGE_NONE = 0, 1, 2
 MAX_PEERS = 8
 
@@ -134,6 +135,7 @@ PROTOTYPES = {
     "mm_set_stream": (C.c_int, [_vp, _vp]),
     "mm_last_counters": (C.c_int, [_vp, _P(Counters)]),
     "mm_last_ms": (C.c_int, [_vp, _P(C.c_float)]),
+    "mm_last_tail": (C.c_int, [_vp, _P(C.c_uint64), _P(C.c_uint64)]),
     "mm_stream": (C.c_int, [_vp, _P(_vp)]),
     "mm_get_scene_info": (C.c_int, [_vp, _P(SceneInfo)]),
     "mm_selftest_quotient": (C.c_int, [_vp, C.c_uint64, C.c_uint64, _P(C.c_uint64)]),

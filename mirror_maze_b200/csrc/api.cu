@@ -10,6 +10,7 @@
 
 using namespace mmk;
 
+#include <algorithm>
 #include <mutex>
 #include <vector>
 #include "ctx.h"
@@ -98,6 +99,7 @@ int mm_destroy(mm_ctx *ctx) {
     cudaFree(ctx->d_pairs); cudaFree(ctx->d_rects); cudaFree(ctx->d_rects_axis); cudaFree(ctx->d_shade); cudaFree(ctx->d_noise); cudaFree(ctx->d_chunks);
     cudaFree(ctx->d_counters); cudaFree(ctx->d_screen); cudaFree(ctx->d_screen2); cudaFree(ctx->d_dbg_rad);
     for (auto p : ctx->d_dbg_u32) cudaFree(p);
+    cudaFree(ctx->d_tail_q); cudaFree(ctx->d_tail_pix);
     if (ctx->h_counters) cudaFreeHost(ctx->h_counters);
     if (ctx->ev0) cudaEventDestroy(ctx->ev0);
     if (ctx->ev1) cudaEventDestroy(ctx->ev1);
@@ -304,6 +306,31 @@ int build_launch(mm_ctx *ctx, const mm_uniform *uni, const mm_params *par, bool 
         p.rg_mask = m && *m ? (uint32_t)strtoul(m, nullptr, 0) : 0xFFFFFFFFu;
     }
     L.choice.block_threads = bt;
+    // Straggler tail (render_kernel.cu): the default kernel queues the paths of warps past bounce_limit segments with at most
+    // kTailK live lanes, and trace_tail_kernel runs them densely.  The queue holds an eighth of the frame's paths (a replay
+    // of the 1080p 16-spp frame queues 6 %, profiles/r3_tail_replay.txt) within kTailBudget; paths past it stay in their
+    // warp.  MM_TAIL_K / MM_TAIL_CAP are developer overrides for tuning runs and tests.
+    if (!L.choice.regroup && !(par->flags & MM_FLAG_NO_TAIL) && (p.total_paths >> p.log2_spp) < (1ull << 32)) {
+        constexpr uint32_t kTailK = 8;
+        constexpr size_t kTailBudget = size_t(1) << 30;
+        const size_t pix_bytes = (4 + 3 * (size_t)spp) * sizeof(float);
+        uint64_t cap = p.total_paths / 8 + 1024;
+        if (cap > kTailBudget / (sizeof(TailPath) + pix_bytes)) cap = kTailBudget / (sizeof(TailPath) + pix_bytes);
+        cap = std::min<uint64_t>(cap, env_u32("MM_TAIL_CAP", 0xFFFFFFFFu, 0, 0xFFFFFFFFu));
+        const uint64_t pixels = std::min<uint64_t>(cap, p.total_paths >> p.log2_spp);   // a deferred pixel has a queued path
+        if (cap && (ctx->tail_q_cap < cap || ctx->tail_pix_bytes < pixels * pix_bytes)) {
+            CK(cudaStreamSynchronize(ctx->stream));
+            cudaFree(ctx->d_tail_q); cudaFree(ctx->d_tail_pix);
+            ctx->d_tail_q = nullptr; ctx->d_tail_pix = nullptr; ctx->tail_q_cap = 0; ctx->tail_pix_bytes = 0;
+            CK(cudaMalloc(&ctx->d_tail_q, cap * sizeof(TailPath)));
+            CK(cudaMalloc(&ctx->d_tail_pix, pixels * pix_bytes));
+            ctx->tail_q_cap = cap; ctx->tail_pix_bytes = pixels * pix_bytes;
+        }
+        p.tail_k = cap ? env_u32("MM_TAIL_K", kTailK, 0, 32) : 0u;
+        p.tail_cap = (uint32_t)cap;
+        p.tail_q = ctx->d_tail_q;
+        p.tail_pix = ctx->d_tail_pix;
+    }
     L.smem = 3 * (size_t)bt * sizeof(float);                             // reduction scratch
     if (L.choice.regroup) L.smem += 4 * (size_t)bt * sizeof(float4) + 64 * sizeof(uint32_t);   // path state in flight + bin counters
     const uint64_t blocks = (p.total_paths + (uint64_t)bt - 1) / (uint64_t)bt;
@@ -322,6 +349,7 @@ int do_launch(mm_ctx *ctx, Launch &L) {
         ctx->cfg_fn = fn; ctx->cfg_smem = L.smem;
     }
     ctx->last_smem = (uint32_t)L.smem; ctx->last_block_threads = (uint32_t)L.choice.block_threads;
+    ctx->last_tail_cap = L.p.tail_k ? L.p.tail_cap : 0u;
     CK(cudaMemsetAsync(ctx->d_counters, 0, sizeof(Counters), ctx->stream));
     CK(cudaEventRecord(ctx->ev0, ctx->stream));
     if (L.choice.pool) {
@@ -335,6 +363,10 @@ int do_launch(mm_ctx *ctx, Launch &L) {
         CK(launch_pool(L.p, L.choice, (unsigned)blocks, (unsigned)L.choice.block_threads, L.smem, ctx->stream));
     } else {
         CK(launch_trace(L.p, L.choice, L.blocks, L.smem, ctx->stream));
+        if (L.p.tail_k) {                 // one thread per queued path; the grid strides over whatever the queue holds
+            const uint64_t want = ((uint64_t)L.p.tail_cap + kTailBlock - 1) / kTailBlock, full = (uint64_t)ctx->n_sms * (1024 / kTailBlock);
+            CK(launch_tail(L.p, L.choice, (unsigned)(want < full ? want : full), ctx->stream));
+        }
     }
     CK(cudaEventRecord(ctx->ev1, ctx->stream));
     CK(cudaMemcpyAsync(ctx->h_counters, ctx->d_counters, sizeof(Counters), cudaMemcpyDeviceToHost, ctx->stream));
@@ -783,6 +815,17 @@ int mm_last_ms(mm_ctx *ctx, float *ms) {
     if (!ctx->timed) return fail(ctx, MM_ERR_INVALID, "mm_last_ms: nothing rendered yet");
     CK(cudaEventSynchronize(ctx->ev1));
     CK(cudaEventElapsedTime(ms, ctx->ev0, ctx->ev1));
+    return MM_OK;
+}
+
+int mm_last_tail(mm_ctx *ctx, uint64_t *queued_paths, uint64_t *deferred_pixels) {
+    if (!ctx || !queued_paths || !deferred_pixels) return MM_ERR_INVALID;
+    ctx->err.clear();
+    if (!ctx->timed) return fail(ctx, MM_ERR_INVALID, "mm_last_tail: nothing rendered yet");
+    CK(cudaEventSynchronize(ctx->ev2));
+    const uint64_t cap = ctx->last_tail_cap, head = ctx->h_counters->tail_paths;
+    *queued_paths = head < cap ? head : cap;
+    *deferred_pixels = ctx->h_counters->tail_pixels;
     return MM_OK;
 }
 

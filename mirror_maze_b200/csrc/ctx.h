@@ -34,6 +34,9 @@ struct mm_ctx {
     uint32_t *d_dbg_u32[3] = {nullptr, nullptr, nullptr};
     float *d_dbg_rad = nullptr;
     size_t dbg_cap = 0;
+    mmk::TailPath *d_tail_q = nullptr;  // straggler queue and deferred-pixel slots (trace_kernel -> trace_tail_kernel)
+    float *d_tail_pix = nullptr;
+    size_t tail_q_cap = 0, tail_pix_bytes = 0;
     // asynchronous host-buffer frames (mm_render_async / mm_wait)
     float *h_stage = nullptr;         // pinned staging for callers whose buffer the library does not know to be pinned
     size_t stage_bytes = 0;
@@ -47,7 +50,7 @@ struct mm_ctx {
     float *d_snap = nullptr;
     bool present_in_flight = false;
     // last launch facts
-    uint32_t last_smem = 0, last_blocks_per_sm = 0, last_block_threads = 0;
+    uint32_t last_smem = 0, last_blocks_per_sm = 0, last_block_threads = 0, last_tail_cap = 0;
     const void *cfg_fn = nullptr;     // kernel variant whose attributes / occupancy were last set up
     size_t cfg_smem = 0;
 };

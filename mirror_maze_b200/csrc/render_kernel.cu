@@ -24,15 +24,104 @@
 namespace mmk {
 namespace {
 
+// Stores one finished pixel, from the sums of its spp tone-mapped samples in the reference's order (shaders.metal:343-366),
+// into every output of the dispatch: the frame, the tiles, the zero-copy host frame and the frames of the fused exchange.
+__device__ __forceinline__ void deliver_pixel(const KParams &P, float sx, float sy, float sz, uint32_t pxx, uint32_t pxy, size_t tile) {
+    const float d = (float)(int)P.spp;
+    float4 px = make_float4(fdiv(sx, d), fdiv(sy, d), fdiv(sz, d), 1.0f);
+    if (P.quant8) px = quant8(px);
+    if (P.image && pxx < P.W && pxy < P.H) reinterpret_cast<float4 *>(P.image)[(size_t)pxy * P.W + pxx] = px;
+    if (P.tiles) reinterpret_cast<float4 *>(P.tiles)[tile] = px;
+    if ((P.n_peers || P.host_out) && pxx < P.W && pxy < P.H) {
+        const size_t at = (size_t)pxy * P.W + pxx;
+        if (P.host_out) reinterpret_cast<float4 *>(P.host_out)[at] = px;        // zero-copy output: mapped pinned host frame, over PCIe
+        if (P.peers_multicast) {                                    // fused exchange, NVSwitch multicast: one store, replicated by the switch
+            float4 *mc = reinterpret_cast<float4 *>(P.peers[0]) + at;
+            asm volatile("multimem.st.weak.global.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(mc), "f"(px.x), "f"(px.y), "f"(px.z), "f"(px.w) : "memory");
+        } else {                                                    // fused exchange, NVLink peer mappings: one store per rank's frame
+            for (uint32_t i = 0; i < P.n_peers; i++) reinterpret_cast<float4 *>(P.peers[i])[at] = px;
+        }
+    }
+}
+
+// Event counts: warp-reduce, one atomic per warp and counter.
+template <bool CNT>
+__device__ __forceinline__ void add_counters(const KParams &P, uint32_t seg, uint32_t nhits, uint32_t nliteral, uint32_t paths, Tally tl) {
+    unsigned long long v_rays = seg, v_hits = nhits, v_lit = nliteral, v_paths = paths;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        v_rays += __shfl_xor_sync(0xFFFFFFFFu, v_rays, o);
+        v_hits += __shfl_xor_sync(0xFFFFFFFFu, v_hits, o);
+        v_lit += __shfl_xor_sync(0xFFFFFFFFu, v_lit, o);
+        v_paths += __shfl_xor_sync(0xFFFFFFFFu, v_paths, o);
+    }
+    unsigned long long v_inner = tl.inner, v_leaf = tl.leaf, v_rect = tl.rect;
+    uint32_t v_ms = tl.max_stack;
+    if (CNT) {
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            v_inner += __shfl_xor_sync(0xFFFFFFFFu, v_inner, o);
+            v_leaf += __shfl_xor_sync(0xFFFFFFFFu, v_leaf, o);
+            v_rect += __shfl_xor_sync(0xFFFFFFFFu, v_rect, o);
+            v_ms = max(v_ms, __shfl_xor_sync(0xFFFFFFFFu, v_ms, o));
+        }
+    }
+    if ((threadIdx.x & 31u) == 0u) {
+        if (v_rays) atomicAdd(&P.counters->rays, v_rays);
+        if (v_hits) atomicAdd(&P.counters->hits, v_hits);
+        if (v_paths) atomicAdd(&P.counters->paths, v_paths);
+        if (v_lit) atomicAdd(&P.counters->literal_rays, v_lit);
+        if (CNT) {
+            atomicAdd(&P.counters->inner_visits, v_inner);
+            atomicAdd(&P.counters->leaf_visits, v_leaf);
+            atomicAdd(&P.counters->rect_tests, v_rect);
+            atomicMax(&P.counters->max_stack, (unsigned long long)v_ms);
+        }
+    }
+}
+
 // Block epilogue shared by the trace kernels.  On entry red[] holds every thread's tone-mapped sample (3 planes of
 // kBlockThreads floats, indexed by the thread the path started on) and the block has synchronised.
-template <bool CNT, int kBlockThreads>
+// TAIL: qi is the straggler-queue entry of the thread's path when trace_kernel queued it (0xFFFFFFFF otherwise).  A pixel with
+// a queued sample is not stored here: its other samples go to a deferred-pixel slot, and trace_tail_kernel delivers the pixel
+// when its last sample arrives.
+template <bool CNT, bool TAIL, int kBlockThreads>
 __device__ __forceinline__ void block_epilogue(const KParams &P, float *red, bool active, uint32_t flat, uint32_t pxx, uint32_t pxy, uint32_t k,
-                                               uint32_t seg, uint32_t nhits, uint32_t nliteral, Tally tl) {
-    // Per-pixel reduction in the reference's order (shaders.metal:343-366): pairs, quads, octets (the phases whose
-    // stride is < spp), then the pixel's first thread adds the octets serially and divides by spp.
+                                               uint32_t seg, uint32_t nhits, uint32_t nliteral, Tally tl, uint32_t qi) {
     const uint32_t tid = threadIdx.x;
     float *rx = red, *ry = red + kBlockThreads, *rz = red + 2 * kBlockThreads;
+    bool deferred = false;
+    if (TAIL && __syncthreads_or(qi != 0xFFFFFFFFu)) {
+        __shared__ uint32_t pslot[kBlockThreads];                          // per pixel of the block: queued samples, then its slot
+        const uint32_t pix = tid >> P.log2_spp, si = tid & (P.spp - 1);    // blocks hold whole pixels (block_threads_for)
+        if (tid < (kBlockThreads >> P.log2_spp)) pslot[tid] = 0u;
+        __syncthreads();
+        if (qi != 0xFFFFFFFFu) atomicAdd(&pslot[pix], 1u);
+        __syncthreads();
+        if (si == 0u) {
+            const uint32_t missing = pslot[pix];
+            uint32_t s = 0xFFFFFFFFu;
+            if (missing) {
+                s = (uint32_t)atomicAdd(&P.counters->tail_pixels, 1ull);
+                uint32_t *h = reinterpret_cast<uint32_t *>(P.tail_pix) + (size_t)s * (4u + 3u * P.spp);
+                h[0] = missing; h[1] = pxx; h[2] = pxy; h[3] = k * P.ppc + (flat >> P.log2_spp);
+            }
+            pslot[pix] = s;
+        }
+        __syncthreads();
+        const uint32_t s = pslot[pix];
+        if (s != 0xFFFFFFFFu) {
+            deferred = true;
+            if (qi != 0xFFFFFFFFu) {
+                P.tail_q[qi].e.y = __uint_as_float(s);
+            } else {
+                float *v = P.tail_pix + (size_t)s * (4u + 3u * P.spp) + 4u;
+                v[si] = rx[tid]; v[P.spp + si] = ry[tid]; v[2u * P.spp + si] = rz[tid];
+            }
+        }
+    }
+    // Per-pixel reduction in the reference's order (shaders.metal:343-366): pairs, quads, octets (the phases whose
+    // stride is < spp), then the pixel's first thread adds the octets serially and divides by spp.
 #pragma unroll
     for (uint32_t stride = 1; stride <= 4; stride *= 2) {
         if (stride < P.spp && (tid & (2 * stride - 1)) == 0) {
@@ -42,64 +131,63 @@ __device__ __forceinline__ void block_epilogue(const KParams &P, float *red, boo
         }
         __syncthreads();
     }
-    if (active && (flat & (P.spp - 1)) == 0) {
+    if (active && !deferred && (flat & (P.spp - 1)) == 0) {
         float sx = rx[tid], sy = ry[tid], sz = rz[tid];
         for (uint32_t i = 1; i < P.spp / 8; i++) {
             sx = fadd(sx, rx[tid + 8 * i]); sy = fadd(sy, ry[tid + 8 * i]); sz = fadd(sz, rz[tid + 8 * i]);
         }
-        const float d = (float)(int)P.spp;
-        float4 px = make_float4(fdiv(sx, d), fdiv(sy, d), fdiv(sz, d), 1.0f);
-        if (P.quant8) px = quant8(px);
-        if (P.image && pxx < P.W && pxy < P.H) reinterpret_cast<float4 *>(P.image)[(size_t)pxy * P.W + pxx] = px;
-        if (P.tiles) reinterpret_cast<float4 *>(P.tiles)[(size_t)k * P.ppc + (flat >> P.log2_spp)] = px;
-        if ((P.n_peers || P.host_out) && pxx < P.W && pxy < P.H) {
-            const size_t at = (size_t)pxy * P.W + pxx;
-            if (P.host_out) reinterpret_cast<float4 *>(P.host_out)[at] = px;        // zero-copy output: mapped pinned host frame, over PCIe
-            if (P.peers_multicast) {                                    // fused exchange, NVSwitch multicast: one store, replicated by the switch
-                float4 *mc = reinterpret_cast<float4 *>(P.peers[0]) + at;
-                asm volatile("multimem.st.weak.global.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(mc), "f"(px.x), "f"(px.y), "f"(px.z), "f"(px.w) : "memory");
-            } else {                                                    // fused exchange, NVLink peer mappings: one store per rank's frame
-                for (uint32_t i = 0; i < P.n_peers; i++) reinterpret_cast<float4 *>(P.peers[i])[at] = px;
-            }
-        }
+        deliver_pixel(P, sx, sy, sz, pxx, pxy, (size_t)k * P.ppc + (flat >> P.log2_spp));
     }
+    add_counters<CNT>(P, seg, nhits, nliteral, active ? 1u : 0u, tl);
+}
 
-    // Event counts: warp-reduce, one atomic per warp and counter.
-    {
-        unsigned long long v_rays = seg, v_hits = nhits, v_lit = nliteral, v_paths = active ? 1u : 0u;
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            v_rays += __shfl_xor_sync(0xFFFFFFFFu, v_rays, o);
-            v_hits += __shfl_xor_sync(0xFFFFFFFFu, v_hits, o);
-            v_lit += __shfl_xor_sync(0xFFFFFFFFu, v_lit, o);
-            v_paths += __shfl_xor_sync(0xFFFFFFFFu, v_paths, o);
-        }
-        unsigned long long v_inner = tl.inner, v_leaf = tl.leaf, v_rect = tl.rect;
-        uint32_t v_ms = tl.max_stack;
-        if (CNT) {
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) {
-                v_inner += __shfl_xor_sync(0xFFFFFFFFu, v_inner, o);
-                v_leaf += __shfl_xor_sync(0xFFFFFFFFu, v_leaf, o);
-                v_rect += __shfl_xor_sync(0xFFFFFFFFu, v_rect, o);
-                v_ms = max(v_ms, __shfl_xor_sync(0xFFFFFFFFu, v_ms, o));
-            }
-        }
-        if ((tid & 31u) == 0u) {
-            atomicAdd(&P.counters->rays, v_rays);
-            atomicAdd(&P.counters->hits, v_hits);
-            atomicAdd(&P.counters->paths, v_paths);
-            if (v_lit) atomicAdd(&P.counters->literal_rays, v_lit);
-            if (CNT) {
-                atomicAdd(&P.counters->inner_visits, v_inner);
-                atomicAdd(&P.counters->leaf_visits, v_leaf);
-                atomicAdd(&P.counters->rect_tests, v_rect);
-                atomicMax(&P.counters->max_stack, (unsigned long long)v_ms);
-            }
+// One segment of the bounce loop (shaders.metal:306-340) for the lanes of a warp together: traverse, then shade the hit of
+// every live lane.  A lane whose path has ended (or that has no path) idles with alive = false.
+template <bool CNT, bool DBG>
+__device__ __forceinline__ void bounce_segment(const KParams &P, uint32_t root, bool &alive, V3 &ori, V3 &dir, V3 &color, V3 &light, float &t,
+                                               uint32_t &slot, uint32_t &state, int &n, int &mirror_hits, uint32_t &first_hit,
+                                               uint32_t &seg, uint32_t &nhits, uint32_t &nliteral, Tally &tl) {
+    const bool lit = ray_is_literal(P, ori, dir);
+    const bool any_lit = __any_sync(0xFFFFFFFFu, alive && lit) || !P.rect_fast_ok;   // MIXED also means literal rect tests
+    Hit h;
+    if (P.rcp_mode) {
+        if (!any_lit) h = traverse<false, CNT, true>(P.pairs, P.rects, root, alive, false, ori, dir, t, slot, &tl);
+        else h = traverse<true, CNT, true>(P.pairs, P.rects, root, alive, lit, ori, dir, t, slot, &tl);
+    } else {
+        if (!any_lit && P.rects_axis) h = traverse<false, CNT, false, true>(P.pairs, P.rects_axis, root, alive, false, ori, dir, t, slot, &tl);
+        else if (!any_lit) h = traverse<false, CNT, false>(P.pairs, P.rects, root, alive, false, ori, dir, t, slot, &tl);
+        else h = traverse<true, CNT, false>(P.pairs, P.rects, root, alive, lit, ori, dir, t, slot, &tl);
+    }
+    t = h.t; slot = h.slot;
+    if (alive) {
+        if (lit) nliteral++;
+        seg++;
+        if (!(t < 1e30f)) {                                        // :308, :336-339 (sky term is * 0.0)
+            alive = false;
+        } else {
+            nhits++;
+            uint32_t orig = 0xFFFFFFFFu;
+            if (!shade_hit(P, slot, t, ori, dir, color, light, state, mirror_hits, (DBG && n == 0) ? &orig : nullptr)) alive = false;
+            if (DBG && n == 0) first_hit = orig;
+            t = 1e30f;                                             // :323, :330
+            n++;
+            alive = alive && (n < P.bounce_limit + mirror_hits);   // :306
         }
     }
 }
 
+__device__ __forceinline__ void write_dbg(const KParams &P, uint64_t path, uint32_t first_hit, uint32_t seg, int mirror_hits, V3 light) {
+    if (P.dbg_first_hit) P.dbg_first_hit[path] = first_hit;
+    if (P.dbg_segments) P.dbg_segments[path] = seg;
+    if (P.dbg_mirror_hits) P.dbg_mirror_hits[path] = (uint32_t)mirror_hits;
+    if (P.dbg_radiance) { P.dbg_radiance[3 * path] = light.x; P.dbg_radiance[3 * path + 1] = light.y; P.dbg_radiance[3 * path + 2] = light.z; }
+}
+
+// The straggler tail.  Almost every path ends after exactly bounce_limit segments; a mirror hit adds one (:306), so past
+// bounce_limit a warp typically runs a whole traversal and shading for 1-3 live lanes at the price of 32.  At a segment
+// boundary past bounce_limit, a warp with 1..tail_k live lanes instead writes those paths' complete state to a global queue
+// (one atomic per warp; entries past tail_cap stay with the warp, which is the one-kernel behaviour) and leaves the bounce loop.
+// trace_tail_kernel then runs the queued paths densely, one thread per path, with the same traversal and shading code.
 template <bool CNT, bool DBG, int kBlockThreads>
 __global__ void __launch_bounds__(kBlockThreads, 1024 / kBlockThreads)
 trace_kernel(const __grid_constant__ KParams P) {
@@ -115,7 +203,7 @@ trace_kernel(const __grid_constant__ KParams P) {
     const uint32_t root = P.root_count ? (kLeafBit | P.root_link | (P.root_count << 24)) : P.root_link;   // pair 0 is at byte offset 0
     V3 st_ori = mk(0.0f, 0.0f, 0.0f), st_dir = mk(1.0f, 1.0f, 1.0f), st_color = mk(1.0f, 1.0f, 1.0f), st_light = mk(0.0f, 0.0f, 0.0f);
     float st_t = 1e30f;
-    uint32_t st_slot = 0xFFFFFFFFu, st_state = 0u, first_hit = 0xFFFFFFFFu;
+    uint32_t st_slot = 0xFFFFFFFFu, st_state = 0u, first_hit = 0xFFFFFFFFu, qi = 0xFFFFFFFFu;
     int mirror_hits = 0;
     bool n_alive = false;
 
@@ -133,48 +221,91 @@ trace_kernel(const __grid_constant__ KParams P) {
         float t = st_t;
         uint32_t slot = st_slot, state = st_state;
         int n = 0;
-        bool alive = active && n_alive;
-        while (__any_sync(0xFFFFFFFFu, alive)) {
-            const bool lit = ray_is_literal(P, ori, dir);
-            const bool any_lit = __any_sync(0xFFFFFFFFu, alive && lit) || !P.rect_fast_ok;   // MIXED also means literal rect tests
-            Hit h;
-            if (P.rcp_mode) {
-                if (!any_lit) h = traverse<false, CNT, true>(P.pairs, P.rects, root, alive, false, ori, dir, t, slot, &tl);
-                else h = traverse<true, CNT, true>(P.pairs, P.rects, root, alive, lit, ori, dir, t, slot, &tl);
-            } else {
-                if (!any_lit && P.rects_axis) h = traverse<false, CNT, false, true>(P.pairs, P.rects_axis, root, alive, false, ori, dir, t, slot, &tl);
-                else if (!any_lit) h = traverse<false, CNT, false>(P.pairs, P.rects, root, alive, false, ori, dir, t, slot, &tl);
-                else h = traverse<true, CNT, false>(P.pairs, P.rects, root, alive, lit, ori, dir, t, slot, &tl);
+        bool alive = active && n_alive, may_queue = P.tail_k != 0u;
+        while (true) {
+            unsigned live;
+            while ((live = __ballot_sync(0xFFFFFFFFu, alive)) != 0u) {
+                // Every live lane has hit on every segment so far, so all of them have the same n (= their segment count).
+                if (may_queue && (uint32_t)__popc(live) <= P.tail_k && __ballot_sync(0xFFFFFFFFu, alive && n >= P.bounce_limit)) break;
+                bounce_segment<CNT, DBG>(P, root, alive, ori, dir, color, light, t, slot, state, n, mirror_hits, first_hit, seg, nhits, nliteral, tl);
             }
-            t = h.t; slot = h.slot;
-            if (alive) {
-                if (lit) nliteral++;
-                seg++;
-                if (!(t < 1e30f)) {                                        // :308, :336-339 (sky term is * 0.0)
-                    alive = false;
-                } else {
-                    nhits++;
-                    uint32_t orig = 0xFFFFFFFFu;
-                    if (!shade_hit(P, slot, t, ori, dir, color, light, state, mirror_hits, (DBG && n == 0) ? &orig : nullptr)) alive = false;
-                    if (DBG && n == 0) first_hit = orig;
-                    t = 1e30f;                                             // :323, :330
-                    n++;
-                    alive = alive && (n < P.bounce_limit + mirror_hits);   // :306
-                }
+            if (live == 0u) break;
+            // Queue the live paths: one reservation per warp.  Lanes that find the queue full keep their paths and trace on.
+            may_queue = false;
+            const uint32_t lead = (uint32_t)__ffs(live) - 1u, lane = threadIdx.x & 31u;
+            unsigned long long base = 0;
+            if (lane == lead) base = atomicAdd(&P.counters->tail_paths, (unsigned long long)__popc(live));
+            base = __shfl_sync(0xFFFFFFFFu, base, lead) + (unsigned long long)__popc(live & ((1u << lane) - 1u));
+            if (alive && base < P.tail_cap) {
+                qi = (uint32_t)base;
+                TailPath *q = P.tail_q + qi;
+                q->a = make_float4(ori.x, ori.y, ori.z, dir.x);
+                q->b = make_float4(dir.y, dir.z, color.x, color.y);
+                q->c = make_float4(color.z, light.x, light.y, light.z);
+                q->d = make_float4(__uint_as_float(state), __uint_as_float((uint32_t)n | ((uint32_t)mirror_hits << 16)),
+                                   __uint_as_float((uint32_t)path), __uint_as_float((uint32_t)(path >> 32)));
+                q->e = make_float4(__uint_as_float(DBG ? first_hit : 0xFFFFFFFFu), 0.0f, 0.0f, 0.0f);   // .y: deferred-pixel slot, set in the epilogue
+                alive = false;
             }
         }
         sample = mk(fsqrt(fmaxf(light.x, 0.0f)), fsqrt(fmaxf(light.y, 0.0f)), fsqrt(fmaxf(light.z, 0.0f)));   // :344
-        if (DBG && active) {
-            if (P.dbg_first_hit) P.dbg_first_hit[path] = first_hit;
-            if (P.dbg_segments) P.dbg_segments[path] = seg;
-            if (P.dbg_mirror_hits) P.dbg_mirror_hits[path] = (uint32_t)mirror_hits;
-            if (P.dbg_radiance) { P.dbg_radiance[3 * path] = light.x; P.dbg_radiance[3 * path + 1] = light.y; P.dbg_radiance[3 * path + 2] = light.z; }
-        }
+        if (DBG && active && qi == 0xFFFFFFFFu) write_dbg(P, path, first_hit, seg, mirror_hits, light);
     }
 
     red[threadIdx.x] = sample.x; red[kBlockThreads + threadIdx.x] = sample.y; red[2 * kBlockThreads + threadIdx.x] = sample.z;
     __syncthreads();
-    block_epilogue<CNT, kBlockThreads>(P, red, active, flat, pxx, pxy, k, seg, nhits, nliteral, tl);
+    block_epilogue<CNT, true, kBlockThreads>(P, red, active, flat, pxx, pxy, k, seg, nhits, nliteral, tl, qi);
+}
+
+// The paths trace_kernel queued, one thread per path in queue order (dense warps), from where they stopped to their end.  The
+// thread that stores a pixel's last missing sample reduces the pixel's samples in the reference's order and delivers it.
+template <bool CNT, bool DBG>
+__global__ void __launch_bounds__(kTailBlock, 1024 / kTailBlock)
+trace_tail_kernel(const __grid_constant__ KParams P) {
+    const unsigned long long head = P.counters->tail_paths;                // written by trace_kernel, the launch before
+    const uint32_t nq = head < P.tail_cap ? (uint32_t)head : P.tail_cap;
+    const uint32_t root = P.root_count ? (kLeafBit | P.root_link | (P.root_count << 24)) : P.root_link;
+    const uint32_t words = 4u + 3u * P.spp;
+    Tally tl = {0u, 0u, 0u, 0u};
+    uint32_t seg = 0, nhits = 0, nliteral = 0;
+    for (uint32_t i0 = blockIdx.x * kTailBlock; i0 < nq; i0 += gridDim.x * kTailBlock) {
+        const uint32_t i = i0 + threadIdx.x;
+        const bool has = i < nq;
+        V3 ori = mk(0.0f, 0.0f, 0.0f), dir = mk(1.0f, 1.0f, 1.0f), color = mk(1.0f, 1.0f, 1.0f), light = mk(0.0f, 0.0f, 0.0f);
+        uint32_t state = 0u, first_hit = 0xFFFFFFFFu, pix = 0u, slot = 0xFFFFFFFFu;
+        uint64_t path = 0;
+        int n = 0, mirror_hits = 0;
+        if (has) {
+            const TailPath *q = P.tail_q + i;
+            const float4 a = q->a, b = q->b, c = q->c, d = q->d, e = q->e;
+            ori = mk(a.x, a.y, a.z); dir = mk(a.w, b.x, b.y); color = mk(b.z, b.w, c.x); light = mk(c.y, c.z, c.w);
+            state = __float_as_uint(d.x);
+            const uint32_t nm = __float_as_uint(d.y);
+            n = (int)(nm & 0xFFFFu); mirror_hits = (int)(nm >> 16);
+            path = (uint64_t)__float_as_uint(d.z) | ((uint64_t)__float_as_uint(d.w) << 32);
+            first_hit = __float_as_uint(e.x); pix = __float_as_uint(e.y);
+        }
+        const uint32_t pseg = (uint32_t)n - seg;                          // segments this path ran in trace_kernel, less ours so far
+        float t = 1e30f;
+        bool alive = has;
+        while (__any_sync(0xFFFFFFFFu, alive))
+            bounce_segment<CNT, DBG>(P, root, alive, ori, dir, color, light, t, slot, state, n, mirror_hits, first_hit, seg, nhits, nliteral, tl);
+        if (has) {
+            if (DBG) write_dbg(P, path, first_hit, pseg + seg, mirror_hits, light);
+            const uint32_t si = (uint32_t)path & (P.spp - 1u);           // sample within the pixel (T and group starts are multiples of spp)
+            float *v = P.tail_pix + (size_t)pix * words;
+            v[4u + si] = fsqrt(fmaxf(light.x, 0.0f)); v[4u + P.spp + si] = fsqrt(fmaxf(light.y, 0.0f));   // :344
+            v[4u + 2u * P.spp + si] = fsqrt(fmaxf(light.z, 0.0f));
+            __threadfence();                                               // the sample is visible before the count drops
+            if (atomicSub(reinterpret_cast<uint32_t *>(v), 1u) == 1u) {    // the pixel's last missing sample
+                __threadfence();
+                const uint32_t *h = reinterpret_cast<const uint32_t *>(v);
+                deliver_pixel(P, reduce_samples(v + 4, P.spp, 1), reduce_samples(v + 4 + P.spp, P.spp, 1),
+                              reduce_samples(v + 4 + 2 * P.spp, P.spp, 1), h[1], h[2], h[3]);
+            }
+        }
+    }
+    add_counters<CNT>(P, seg, nhits, nliteral, 0u, tl);
 }
 
 // ---- trace_kernel_rg: the same kernel with the block's paths RE-FORMED INTO WARPS at every segment boundary ---------------------
@@ -310,7 +441,7 @@ trace_kernel_rg(const __grid_constant__ KParams P) {
         round++;
     }
     __syncthreads();
-    block_epilogue<CNT, kBlockThreads>(P, red, active, flat, pxx, pxy, k, seg, nhits, nliteral, tl);
+    block_epilogue<CNT, false, kBlockThreads>(P, red, active, flat, pxx, pxy, k, seg, nhits, nliteral, tl, 0xFFFFFFFFu);
 }
 
 // De-interleave gathered tiles into the frame (consumer side of the multi-GPU tile gather).
@@ -490,6 +621,14 @@ cudaError_t launch_trace(const KParams &p, KernelChoice c, unsigned blocks, size
     const void *fn = kernel_ptr(c);
     void *args[] = {const_cast<KParams *>(&p)};
     return cudaLaunchKernel(fn, dim3(blocks), dim3(c.block_threads), args, smem_bytes, stream);
+}
+
+cudaError_t launch_tail(const KParams &p, KernelChoice c, unsigned blocks, cudaStream_t stream) {
+    const void *fn = c.debug ? reinterpret_cast<const void *>(&trace_tail_kernel<true, true>)
+                             : (c.counters ? reinterpret_cast<const void *>(&trace_tail_kernel<true, false>)
+                                           : reinterpret_cast<const void *>(&trace_tail_kernel<false, false>));
+    void *args[] = {const_cast<KParams *>(&p)};
+    return cudaLaunchKernel(fn, dim3(blocks), dim3(kTailBlock), args, 0, stream);
 }
 
 cudaError_t launch_mb_gather(const void *table, uint32_t n_records, uint32_t iters, unsigned blocks, float *sink, cudaStream_t stream) {

@@ -65,7 +65,18 @@ struct __align__(16) RectS {
 struct Counters {   // device-side mirror of mm_counters
     unsigned long long paths, rays, inner_visits, leaf_visits, rect_tests, hits, literal_rays, max_stack;
     unsigned long long next_unit;   // pool kernel: work-distribution ticket (zeroed with the counters before every launch)
+    unsigned long long tail_paths;  // straggler queue head: paths trace_kernel handed to trace_tail_kernel (may pass tail_cap)
+    unsigned long long tail_pixels; // deferred-pixel slots handed out
 };
+
+// One straggler path in the queue trace_kernel fills and trace_tail_kernel drains, 80 B:
+//   a = (ori.xyz, dir.x)  b = (dir.yz, color.xy)  c = (color.z, light.xyz)
+//   d = (RNG state, n | mirror_hits << 16, path index low, high word)   e = (first_hit, deferred-pixel slot, -, -)
+// A path is only queued while alive, so every segment it ran was a hit: its segment count so far is n.
+struct __align__(16) TailPath { float4 a, b, c, d, e; };
+static_assert(sizeof(TailPath) == 80, "straggler record is 80 B");
+// A deferred-pixel slot is 4 + 3 spp words: (samples still missing, pixel x, pixel y, tile index), then the pixel's tone-mapped
+// samples as three planes of spp floats.
 
 struct KParams {
     mm_uniform uni;            // the reference's 56-byte uniform, by value like set_bytes (main.rs:875-879)
@@ -105,6 +116,11 @@ struct KParams {
     uint32_t pool_R;            // pixel records per warp
     uint32_t pool_region_words; // words of shared memory per warp
     uint32_t pool_th_leaf, pool_th_shade;   // a body below 32 ready paths runs once this many wait for it
+    // straggler tail (trace_kernel -> trace_tail_kernel)
+    uint32_t tail_k;            // a warp past bounce_limit segments with 1..tail_k live lanes queues them and stops; 0 = off
+    uint32_t tail_cap;          // queue entries; deferred-pixel slots are never more than queued paths
+    TailPath *tail_q;
+    float *tail_pix;            // deferred-pixel slots of 4 + 3 spp words
     Counters *counters;
     uint32_t *dbg_first_hit, *dbg_segments, *dbg_mirror_hits;
     float *dbg_radiance;
@@ -126,6 +142,8 @@ const void *kernel_ptr(KernelChoice c);
 const void *pool_kernel_ptr(KernelChoice c);
 cudaError_t launch_pool(const KParams &p, KernelChoice c, unsigned blocks, unsigned threads, size_t smem_bytes, cudaStream_t stream);
 cudaError_t launch_trace(const KParams &p, KernelChoice c, unsigned blocks, size_t smem_bytes, cudaStream_t stream);
+cudaError_t launch_tail(const KParams &p, KernelChoice c, unsigned blocks, cudaStream_t stream);
+constexpr int kTailBlock = 256;
 cudaError_t launch_mb_gather(const void *table, uint32_t n_records, uint32_t iters, unsigned blocks, float *sink, cudaStream_t stream);
 cudaError_t launch_mb_ffma(uint32_t iters, unsigned blocks, float *sink, cudaStream_t stream);
 cudaError_t launch_scatter_all(const float *gathered, float *image, const mm_chunk *chunks, uint32_t world, uint32_t max_count,

@@ -242,6 +242,12 @@ class Renderer:
         self._ck(self._lib.mm_last_ms(self._ctx, C.byref(ms)))
         return float(ms.value)
 
+    def last_tail(self):
+        """mm_last_tail: (paths queued for the straggler kernel, pixels deferred to it) in the most recent render."""
+        q, px = C.c_uint64(), C.c_uint64()
+        self._ck(self._lib.mm_last_tail(self._ctx, C.byref(q), C.byref(px)))
+        return int(q.value), int(px.value)
+
 
 class MultiRenderer:
     """mm_multi: one process, several GPUs behind the C-ABI (no torch involved): scene replicated, the frame's groups
