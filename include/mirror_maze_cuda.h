@@ -104,6 +104,10 @@ typedef struct mm_params {
 #define MM_FLAG_NO_TAIL     4096u   /* trace every path to its end in the one-thread-per-path kernel (for comparisons; same bits).  By
                                       default a warp that is past bounce_limit segments with at most 8 live lanes hands those paths to
                                       a second kernel that runs them densely, one thread per path (render_kernel.cu, DESIGN.md §4)  */
+#define MM_FLAG_NO_Y_TABLE  8192u   /* trace with trace_kernel even when the scene has the y-table (for comparisons; same bits).  By default
+                                      a scene with at most 8 distinct child y-intervals (every maze has 5) is traced by
+                                      trace_ytab_kernel, which computes a ray's y slab quotients once per traversal instead of in
+                                      every interior visit (DESIGN.md §3-4)                                                       */
 
 /* Exact event counts of one render call; identical on CPU oracle and GPU (SURVEY §8 d). */
 typedef struct mm_counters {
@@ -264,6 +268,7 @@ typedef struct mm_scene_info {
     uint32_t fast_slab_ok;      /* 1 when scene bounds allow the shared-reciprocal exact slab test    */
     uint32_t smem_bytes, block_threads, blocks_per_sm, n_sms;
     uint32_t axis_rects;        /* 1 when every rect is axis-aligned: the collapsed 32-byte rect test is in use */
+    uint32_t y_table;           /* y-table entries the last render launch used (trace_ytab_kernel), 0 when it ran without one */
 } mm_scene_info;
 int mm_get_scene_info(mm_ctx *ctx, mm_scene_info *out);
 

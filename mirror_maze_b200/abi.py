@@ -20,6 +20,7 @@ FLAG_SCREEN_RGBA8 = 512
 FLAG_REGROUP = 1024
 FLAG_GENERAL_RECTS = 2048
 FLAG_NO_TAIL = 4096
+FLAG_NO_Y_TABLE = 8192
 EXCHANGE_PEER, EXCHANGE_NCCL, EXCHANGE_NONE = 0, 1, 2
 MAX_PEERS = 8
 
@@ -89,7 +90,8 @@ class Debug(C.Structure):
 
 class SceneInfo(C.Structure):
     _fields_ = [(n, C.c_uint32) for n in ("n_planes", "n_nodes", "bvh_depth", "max_leaf", "fast_rect_ok", "fast_slab_ok",
-                                          "smem_bytes", "block_threads", "blocks_per_sm", "n_sms", "axis_rects")]
+                                          "smem_bytes", "block_threads", "blocks_per_sm", "n_sms", "axis_rects",
+                                          "y_table")]
 
     def as_dict(self):
         return {n: int(getattr(self, n)) for n, _ in self._fields_}

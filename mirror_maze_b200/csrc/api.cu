@@ -96,7 +96,8 @@ int mm_destroy(mm_ctx *ctx) {
     if (!ctx) return MM_OK;
     cudaSetDevice(ctx->device);
     if (ctx->stream) cudaStreamSynchronize(ctx->stream);
-    cudaFree(ctx->d_pairs); cudaFree(ctx->d_rects); cudaFree(ctx->d_rects_axis); cudaFree(ctx->d_shade); cudaFree(ctx->d_noise); cudaFree(ctx->d_chunks);
+    cudaFree(ctx->d_pairs); cudaFree(ctx->d_pairs_y); cudaFree(ctx->d_rects); cudaFree(ctx->d_rects_axis); cudaFree(ctx->d_shade); cudaFree(ctx->d_noise);
+    cudaFree(ctx->d_chunks);
     cudaFree(ctx->d_counters); cudaFree(ctx->d_screen); cudaFree(ctx->d_screen2); cudaFree(ctx->d_dbg_rad);
     for (auto p : ctx->d_dbg_u32) cudaFree(p);
     cudaFree(ctx->d_tail_q); cudaFree(ctx->d_tail_pix);
@@ -137,28 +138,42 @@ int mm_upload_scene(mm_ctx *ctx, const mm_plane *planes, uint32_t n_planes, cons
     CK(cudaSetDevice(ctx->device));
     CK(cudaStreamSynchronize(ctx->stream));
     ctx->have_scene = false;
-    cudaFree(ctx->d_pairs); cudaFree(ctx->d_rects); cudaFree(ctx->d_rects_axis); cudaFree(ctx->d_shade); cudaFree(ctx->d_noise);
-    ctx->d_pairs = nullptr; ctx->d_rects = nullptr; ctx->d_rects_axis = nullptr; ctx->d_shade = nullptr; ctx->d_noise = nullptr;
+    cudaFree(ctx->d_pairs); cudaFree(ctx->d_pairs_y); cudaFree(ctx->d_rects); cudaFree(ctx->d_rects_axis); cudaFree(ctx->d_shade); cudaFree(ctx->d_noise);
+    ctx->d_pairs = nullptr; ctx->d_pairs_y = nullptr; ctx->d_rects = nullptr; ctx->d_rects_axis = nullptr; ctx->d_shade = nullptr; ctx->d_noise = nullptr;
+    ctx->n_yiv = 0;
     const size_t noise_bytes = (size_t)noise_w * noise_h * 4;
-    {
-        // The kernel forms record addresses as {high word, low word + offset} (one 32-bit add, render_kernel.cu), so the
-        // pair table must not straddle a 4-GB boundary.  An allocation that does is kept until a second one — which then
-        // cannot cover the same boundary — has been made.
-        const size_t pair_bytes = prep.pairs.size() * sizeof(PairRec);
+    // The kernel forms record addresses as {high word, low word + offset} (one 32-bit add, render_kernel.cu), so a pair
+    // table must not straddle a 4-GB boundary.  An allocation that does is kept until a second one — which then cannot
+    // cover the same boundary — has been made.
+    auto alloc_window = [&](size_t bytes, void **out) -> int {
         void *first = nullptr, *second = nullptr;
-        CK(cudaMalloc(&first, pair_bytes));
+        CK(cudaMalloc(&first, bytes));
         auto straddles = [&](void *p) {
             const uintptr_t a = reinterpret_cast<uintptr_t>(p);
-            return (a >> 32) != ((a + pair_bytes - 1) >> 32);
+            return (a >> 32) != ((a + bytes - 1) >> 32);
         };
         if (straddles(first)) {
-            cudaError_t e = cudaMalloc(&second, pair_bytes);
+            cudaError_t e = cudaMalloc(&second, bytes);
             cudaFree(first);
             if (e != cudaSuccess) return fail(ctx, MM_ERR_NOMEM, std::string("mm_upload_scene: ") + cudaGetErrorString(e));
             if (straddles(second)) { cudaFree(second); return fail(ctx, MM_ERR_CUDA, "mm_upload_scene: pair table straddles a 4-GB boundary"); }
             first = second;
         }
-        ctx->d_pairs = static_cast<PairRec *>(first);
+        *out = first;
+        return MM_OK;
+    };
+    {
+        void *p = nullptr;
+        if ((rc = alloc_window(prep.pairs.size() * sizeof(PairRec), &p)) != MM_OK) return rc;
+        ctx->d_pairs = static_cast<PairRec *>(p);
+    }
+    if (!prep.pairs_y.empty()) {
+        const size_t rec_bytes = prep.pairs_y.size() * sizeof(PairRecY), iv_bytes = prep.y_ivals.size() * sizeof(float4);
+        void *p = nullptr;
+        if ((rc = alloc_window(rec_bytes + iv_bytes, &p)) != MM_OK) return rc;
+        ctx->d_pairs_y = static_cast<PairRecY *>(p);
+        CK(cudaMemcpyAsync(ctx->d_pairs_y, prep.pairs_y.data(), rec_bytes, cudaMemcpyHostToDevice, ctx->stream));
+        CK(cudaMemcpyAsync(static_cast<char *>(p) + rec_bytes, prep.y_ivals.data(), iv_bytes, cudaMemcpyHostToDevice, ctx->stream));
     }
     CK(cudaMalloc(&ctx->d_rects, prep.rects.size() * sizeof(RectI)));
     CK(cudaMalloc(&ctx->d_shade, prep.shade.size() * sizeof(RectS)));
@@ -176,6 +191,8 @@ int mm_upload_scene(mm_ctx *ctx, const mm_plane *planes, uint32_t n_planes, cons
     ctx->root_link = prep.root_link; ctx->root_count = prep.root_count;
     ctx->depth = prep.depth; ctx->max_leaf = prep.max_leaf; ctx->fast_ok = prep.fast_ok; ctx->rect_fast_ok = prep.rect_fast_ok;
     ctx->noise_w = noise_w; ctx->noise_h = noise_h;
+    ctx->n_pairs_y = (uint32_t)prep.pairs_y.size();
+    ctx->n_yiv = ctx->d_pairs_y ? (uint32_t)prep.y_ivals.size() : 0u;
     ctx->have_scene = true;
     return MM_OK;
 }
@@ -293,6 +310,7 @@ int build_launch(mm_ctx *ctx, const mm_uniform *uni, const mm_params *par, bool 
     L.choice.counters = debug || (par->flags & MM_FLAG_COUNTERS);
     L.choice.pool = false;
     L.choice.regroup = false;
+    L.choice.ytab = false;
     if (configure_pool(ctx, par, L)) return MM_OK;
     // opt-in (MM_FLAG_REGROUP, or MM_KERNEL=regroup for tuning runs): the kernel that re-forms the block's warps at segment boundaries
     const char *env_kernel = getenv("MM_KERNEL");
@@ -331,7 +349,16 @@ int build_launch(mm_ctx *ctx, const mm_uniform *uni, const mm_params *par, bool 
         p.tail_q = ctx->d_tail_q;
         p.tail_pix = ctx->d_tail_pix;
     }
+    // The y-table traversal (trace_ytab_kernel, DESIGN.md §3-4) covers the exact slab arithmetic of scenes that have the table;
+    // MM_FLAG_NO_Y_TABLE keeps trace_kernel for comparisons.
+    L.choice.ytab = !L.choice.regroup && ctx->n_yiv && !p.force_literal && !p.rcp_mode && p.scene_fast_ok && !(par->flags & MM_FLAG_NO_Y_TABLE);
+    if (L.choice.ytab) {
+        p.pairs_y = ctx->d_pairs_y;
+        p.y_ivals = reinterpret_cast<const float4 *>(ctx->d_pairs_y + ctx->n_pairs_y);
+        p.n_yiv = ctx->n_yiv;
+    }
     L.smem = 3 * (size_t)bt * sizeof(float);                             // reduction scratch
+    if (L.choice.ytab) L.smem += (size_t)(bt / 32) * p.n_yiv * kYEntryStride;                 // y-table: [warp][interval][lane]
     if (L.choice.regroup) L.smem += 4 * (size_t)bt * sizeof(float4) + 64 * sizeof(uint32_t);   // path state in flight + bin counters
     const uint64_t blocks = (p.total_paths + (uint64_t)bt - 1) / (uint64_t)bt;
     if (blocks > 0x7FFFFFFFull) return fail(ctx, MM_ERR_UNSUPPORTED, "too many paths for one launch");
@@ -350,6 +377,7 @@ int do_launch(mm_ctx *ctx, Launch &L) {
     }
     ctx->last_smem = (uint32_t)L.smem; ctx->last_block_threads = (uint32_t)L.choice.block_threads;
     ctx->last_tail_cap = L.p.tail_k ? L.p.tail_cap : 0u;
+    ctx->last_y_table = L.choice.ytab ? L.p.n_yiv : 0u;
     CK(cudaMemsetAsync(ctx->d_counters, 0, sizeof(Counters), ctx->stream));
     CK(cudaEventRecord(ctx->ev0, ctx->stream));
     if (L.choice.pool) {
@@ -365,7 +393,8 @@ int do_launch(mm_ctx *ctx, Launch &L) {
         CK(launch_trace(L.p, L.choice, L.blocks, L.smem, ctx->stream));
         if (L.p.tail_k) {                 // one thread per queued path; the grid strides over whatever the queue holds
             const uint64_t want = ((uint64_t)L.p.tail_cap + kTailBlock - 1) / kTailBlock, full = (uint64_t)ctx->n_sms * (1024 / kTailBlock);
-            CK(launch_tail(L.p, L.choice, (unsigned)(want < full ? want : full), ctx->stream));
+            const size_t tail_smem = L.choice.ytab ? (size_t)(kTailBlock / 32) * L.p.n_yiv * kYEntryStride : 0;
+            CK(launch_tail(L.p, L.choice, (unsigned)(want < full ? want : full), tail_smem, ctx->stream));
         }
     }
     CK(cudaEventRecord(ctx->ev1, ctx->stream));
@@ -844,6 +873,7 @@ int mm_get_scene_info(mm_ctx *ctx, mm_scene_info *out) {
     out->fast_slab_ok = ctx->fast_ok ? 1u : 0u;
     out->smem_bytes = ctx->last_smem; out->block_threads = ctx->last_block_threads; out->blocks_per_sm = ctx->last_blocks_per_sm;
     out->n_sms = (uint32_t)ctx->n_sms;
+    out->y_table = ctx->last_y_table;
     return MM_OK;
 }
 

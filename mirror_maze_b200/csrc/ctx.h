@@ -16,6 +16,8 @@ struct mm_ctx {
     // scene
     bool have_scene = false;
     mmk::PairRec *d_pairs = nullptr;
+    mmk::PairRecY *d_pairs_y = nullptr;   // n_pairs_y y-table records followed by n_yiv y-intervals; present when n_yiv > 0
+    uint32_t n_pairs_y = 0, n_yiv = 0;
     mmk::RectI *d_rects = nullptr;
     mmk::RectS *d_shade = nullptr;
     mmk::RectA *d_rects_axis = nullptr;   // present when every rect is axis-aligned
@@ -51,6 +53,7 @@ struct mm_ctx {
     bool present_in_flight = false;
     // last launch facts
     uint32_t last_smem = 0, last_blocks_per_sm = 0, last_block_threads = 0, last_tail_cap = 0;
+    uint32_t last_y_table = 0;        // y-table entries of the last launch, 0 when it ran without the table
     const void *cfg_fn = nullptr;     // kernel variant whose attributes / occupancy were last set up
     size_t cfg_smem = 0;
 };

@@ -143,14 +143,22 @@ __device__ __forceinline__ void block_epilogue(const KParams &P, float *red, boo
 
 // One segment of the bounce loop (shaders.metal:306-340) for the lanes of a warp together: traverse, then shade the hit of
 // every live lane.  A lane whose path has ended (or that has no path) idles with alive = false.
-template <bool CNT, bool DBG>
+// YT: warps without literal lanes take the y-table traversal (the host selects YT only without MM_FLAG_RCP_SLAB); ytab is the
+// lane's column of the y-table in dynamic shared memory.
+template <bool CNT, bool DBG, bool YT>
 __device__ __forceinline__ void bounce_segment(const KParams &P, uint32_t root, bool &alive, V3 &ori, V3 &dir, V3 &color, V3 &light, float &t,
                                                uint32_t &slot, uint32_t &state, int &n, int &mirror_hits, uint32_t &first_hit,
-                                               uint32_t &seg, uint32_t &nhits, uint32_t &nliteral, Tally &tl) {
+                                               uint32_t &seg, uint32_t &nhits, uint32_t &nliteral, Tally &tl, uint32_t ytab) {
     const bool lit = ray_is_literal(P, ori, dir);
     const bool any_lit = __any_sync(0xFFFFFFFFu, alive && lit) || !P.rect_fast_ok;   // MIXED also means literal rect tests
     Hit h;
-    if (P.rcp_mode) {
+    if (YT) {
+        if (!any_lit && P.rects_axis)
+            h = traverse<false, CNT, false, true, true>(P.pairs_y, P.rects_axis, root, alive, false, ori, dir, t, slot, &tl, ytab, P.y_ivals, P.n_yiv);
+        else if (!any_lit)
+            h = traverse<false, CNT, false, false, true>(P.pairs_y, P.rects, root, alive, false, ori, dir, t, slot, &tl, ytab, P.y_ivals, P.n_yiv);
+        else h = traverse<true, CNT, false>(P.pairs, P.rects, root, alive, lit, ori, dir, t, slot, &tl);
+    } else if (P.rcp_mode) {
         if (!any_lit) h = traverse<false, CNT, true>(P.pairs, P.rects, root, alive, false, ori, dir, t, slot, &tl);
         else h = traverse<true, CNT, true>(P.pairs, P.rects, root, alive, lit, ori, dir, t, slot, &tl);
     } else {
@@ -188,11 +196,13 @@ __device__ __forceinline__ void write_dbg(const KParams &P, uint64_t path, uint3
 // boundary past bounce_limit, a warp with 1..tail_k live lanes instead writes those paths' complete state to a global queue
 // (one atomic per warp; entries past tail_cap stay with the warp, which is the one-kernel behaviour) and leaves the bounce loop.
 // trace_tail_kernel then runs the queued paths densely, one thread per path, with the same traversal and shading code.
-template <bool CNT, bool DBG, int kBlockThreads>
-__global__ void __launch_bounds__(kBlockThreads, 1024 / kBlockThreads)
-trace_kernel(const __grid_constant__ KParams P) {
+// The body of trace_kernel (YT = false) and trace_ytab_kernel (YT = true: the y-table traversal, whose table follows red[] in
+// dynamic shared memory, n_yiv entries of kYEntryStride bytes per warp).
+template <bool CNT, bool DBG, bool YT, int kBlockThreads>
+__device__ __forceinline__ void trace_body(const KParams &P) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     float *red = reinterpret_cast<float *>(smem_raw);                      // 3 * kBlockThreads floats
+    const uint32_t ytab = YT ? 3u * kBlockThreads * sizeof(float) + (threadIdx.x >> 5) * P.n_yiv * kYEntryStride + (threadIdx.x & 31u) * 8u : 0u;
 
     const uint64_t path = (uint64_t)blockIdx.x * kBlockThreads + threadIdx.x;
     const bool active = path < P.total_paths;
@@ -227,7 +237,7 @@ trace_kernel(const __grid_constant__ KParams P) {
             while ((live = __ballot_sync(0xFFFFFFFFu, alive)) != 0u) {
                 // Every live lane has hit on every segment so far, so all of them have the same n (= their segment count).
                 if (may_queue && (uint32_t)__popc(live) <= P.tail_k && __ballot_sync(0xFFFFFFFFu, alive && n >= P.bounce_limit)) break;
-                bounce_segment<CNT, DBG>(P, root, alive, ori, dir, color, light, t, slot, state, n, mirror_hits, first_hit, seg, nhits, nliteral, tl);
+                bounce_segment<CNT, DBG, YT>(P, root, alive, ori, dir, color, light, t, slot, state, n, mirror_hits, first_hit, seg, nhits, nliteral, tl, ytab);
             }
             if (live == 0u) break;
             // Queue the live paths: one reservation per warp.  Lanes that find the queue full keep their paths and trace on.
@@ -257,14 +267,24 @@ trace_kernel(const __grid_constant__ KParams P) {
     block_epilogue<CNT, true, kBlockThreads>(P, red, active, flat, pxx, pxy, k, seg, nhits, nliteral, tl, qi);
 }
 
+template <bool CNT, bool DBG, int kBlockThreads>
+__global__ void __launch_bounds__(kBlockThreads, 1024 / kBlockThreads)
+trace_kernel(const __grid_constant__ KParams P) { trace_body<CNT, DBG, false, kBlockThreads>(P); }
+
+template <bool CNT, bool DBG, int kBlockThreads>
+__global__ void __launch_bounds__(kBlockThreads, 1024 / kBlockThreads)
+trace_ytab_kernel(const __grid_constant__ KParams P) { trace_body<CNT, DBG, true, kBlockThreads>(P); }
+
 // The paths trace_kernel queued, one thread per path in queue order (dense warps), from where they stopped to their end.  The
 // thread that stores a pixel's last missing sample reduces the pixel's samples in the reference's order and delivers it.
-template <bool CNT, bool DBG>
+// YT: the y-table traversal, as in trace_ytab_kernel; the table is the whole dynamic shared memory.
+template <bool CNT, bool DBG, bool YT>
 __global__ void __launch_bounds__(kTailBlock, 1024 / kTailBlock)
 trace_tail_kernel(const __grid_constant__ KParams P) {
     const unsigned long long head = P.counters->tail_paths;                // written by trace_kernel, the launch before
     const uint32_t nq = head < P.tail_cap ? (uint32_t)head : P.tail_cap;
     const uint32_t root = P.root_count ? (kLeafBit | P.root_link | (P.root_count << 24)) : P.root_link;
+    const uint32_t ytab = YT ? (threadIdx.x >> 5) * P.n_yiv * kYEntryStride + (threadIdx.x & 31u) * 8u : 0u;
     const uint32_t words = 4u + 3u * P.spp;
     Tally tl = {0u, 0u, 0u, 0u};
     uint32_t seg = 0, nhits = 0, nliteral = 0;
@@ -289,7 +309,7 @@ trace_tail_kernel(const __grid_constant__ KParams P) {
         float t = 1e30f;
         bool alive = has;
         while (__any_sync(0xFFFFFFFFu, alive))
-            bounce_segment<CNT, DBG>(P, root, alive, ori, dir, color, light, t, slot, state, n, mirror_hits, first_hit, seg, nhits, nliteral, tl);
+            bounce_segment<CNT, DBG, YT>(P, root, alive, ori, dir, color, light, t, slot, state, n, mirror_hits, first_hit, seg, nhits, nliteral, tl, ytab);
         if (has) {
             if (DBG) write_dbg(P, path, first_hit, pseg + seg, mirror_hits, light);
             const uint32_t si = (uint32_t)path & (P.spp - 1u);           // sample within the pixel (T and group starts are multiples of spp)
@@ -606,12 +626,27 @@ const void *kptr(int bt) {
                              : reinterpret_cast<const void *>(&trace_kernel<C, D, kLargeBlock>);
 }
 
+template <bool C, bool D>
+const void *kptr_yt(int bt) {
+    return bt == kSmallBlock ? reinterpret_cast<const void *>(&trace_ytab_kernel<C, D, kSmallBlock>)
+                             : reinterpret_cast<const void *>(&trace_ytab_kernel<C, D, kLargeBlock>);
+}
+
+template <bool C, bool D>
+const void *tail_ptr(bool yt) {
+    return yt ? reinterpret_cast<const void *>(&trace_tail_kernel<C, D, true>) : reinterpret_cast<const void *>(&trace_tail_kernel<C, D, false>);
+}
+
 }  // namespace
 
 const void *kernel_ptr(KernelChoice c) {
     if (c.regroup) {
         if (c.debug) return kptr_rg<true, true>(c.block_threads);
         return c.counters ? kptr_rg<true, false>(c.block_threads) : kptr_rg<false, false>(c.block_threads);
+    }
+    if (c.ytab) {
+        if (c.debug) return kptr_yt<true, true>(c.block_threads);
+        return c.counters ? kptr_yt<true, false>(c.block_threads) : kptr_yt<false, false>(c.block_threads);
     }
     if (c.debug) return kptr<true, true>(c.block_threads);
     return c.counters ? kptr<true, false>(c.block_threads) : kptr<false, false>(c.block_threads);
@@ -623,12 +658,10 @@ cudaError_t launch_trace(const KParams &p, KernelChoice c, unsigned blocks, size
     return cudaLaunchKernel(fn, dim3(blocks), dim3(c.block_threads), args, smem_bytes, stream);
 }
 
-cudaError_t launch_tail(const KParams &p, KernelChoice c, unsigned blocks, cudaStream_t stream) {
-    const void *fn = c.debug ? reinterpret_cast<const void *>(&trace_tail_kernel<true, true>)
-                             : (c.counters ? reinterpret_cast<const void *>(&trace_tail_kernel<true, false>)
-                                           : reinterpret_cast<const void *>(&trace_tail_kernel<false, false>));
+cudaError_t launch_tail(const KParams &p, KernelChoice c, unsigned blocks, size_t smem_bytes, cudaStream_t stream) {
+    const void *fn = c.debug ? tail_ptr<true, true>(c.ytab) : (c.counters ? tail_ptr<true, false>(c.ytab) : tail_ptr<false, false>(c.ytab));
     void *args[] = {const_cast<KParams *>(&p)};
-    return cudaLaunchKernel(fn, dim3(blocks), dim3(kTailBlock), args, 0, stream);
+    return cudaLaunchKernel(fn, dim3(blocks), dim3(kTailBlock), args, smem_bytes, stream);
 }
 
 cudaError_t launch_mb_gather(const void *table, uint32_t n_records, uint32_t iters, unsigned blocks, float *sink, cudaStream_t stream) {

@@ -22,6 +22,25 @@ struct __align__(32) PairRec {
     struct { float4 z; uint4 link; } zl[2];
 };
 static_assert(sizeof(PairRec) == 192, "pair record is 192 B");
+
+// The same pair for the y-table traversal (traverse<..., YT = true>), 160 B.  Every maze has only a handful of distinct
+// (min.y, max.y) child intervals (floor, roof, walls, light panels, outer walls: 5), so the ray's y quotients of all of them
+// are computed once per traversal call into a per-lane table in shared memory, and a visit reads its two children's
+// (near.y, far.y) from there instead of recomputing four quotients.  x and z are laid out like PairRec::zl's z:
+//   xz[sx + 2*sz] = (c0.near.x, c1.near.x, c0.far.x, c1.far.x,  c0.near.z, c1.near.z, c0.far.z, c1.far.z)
+//   link          = (c0.desc, c1.desc, c0.yoff, c1.yoff)     yoff = y-interval index * kYEntryStride (shared-memory byte offset)
+//   desc: as in PairRec, with interior children at pair index * 160.
+// A visit reads xz[s] as one 32-B load and link as one 16-B load; the record is padded to 160 B so that every xz stays
+// 32-B aligned.  The intervals themselves follow the last record as float4 (min.y, max.y, max.y, min.y): the ray's travel
+// order picks .xy (dir.y >= 0) or .zw.
+struct __align__(32) PairRecY {
+    float4 xz[4][2];
+    uint4 link;
+    uint4 pad;
+};
+static_assert(sizeof(PairRecY) == 160, "y-table pair record is 160 B");
+constexpr uint32_t kMaxYIntervals = 8;         // scenes with more distinct child y-intervals use PairRec only
+constexpr uint32_t kYEntryStride = 32 * 8;     // table layout [warp][interval][lane], 8 B per entry (near, far)
 constexpr uint32_t kLeafBit = 0x80000000u;
 constexpr uint32_t kMaxLeafCount = 126;
 
@@ -99,6 +118,9 @@ struct KParams {
     uint32_t quant8;           // MM_FLAG_SCREEN_RGBA8: stored pixels are quantised to k/255 (round to nearest even)
     uint64_t total_paths;
     const PairRec *pairs;
+    const PairRecY *pairs_y;          // y-table pair records (trace_ytab_kernel; null otherwise)
+    const float4 *y_ivals;            // their n_yiv y-intervals, right after the last PairRecY
+    uint32_t n_yiv;
     const RectI *rects;
     const RectA *rects_axis;          // non-null when every rect of the scene is axis-aligned (and MM_FLAG_FORCE_LITERAL is off)
     const RectS *shade;
@@ -137,12 +159,13 @@ constexpr int kLargeBlock = 256;
 inline int block_threads_for(uint32_t spp) { return spp <= (uint32_t)kSmallBlock ? kSmallBlock : kLargeBlock; }
 
 // Returns the kernel's static properties for the occupancy query and launch.
-struct KernelChoice { bool counters, debug; int block_threads; bool pool; bool regroup; };
+// ytab: trace_ytab_kernel / trace_tail_kernel<..., true> (the y-table traversal) instead of trace_kernel.
+struct KernelChoice { bool counters, debug; int block_threads; bool pool; bool regroup; bool ytab; };
 const void *kernel_ptr(KernelChoice c);
 const void *pool_kernel_ptr(KernelChoice c);
 cudaError_t launch_pool(const KParams &p, KernelChoice c, unsigned blocks, unsigned threads, size_t smem_bytes, cudaStream_t stream);
 cudaError_t launch_trace(const KParams &p, KernelChoice c, unsigned blocks, size_t smem_bytes, cudaStream_t stream);
-cudaError_t launch_tail(const KParams &p, KernelChoice c, unsigned blocks, cudaStream_t stream);
+cudaError_t launch_tail(const KParams &p, KernelChoice c, unsigned blocks, size_t smem_bytes, cudaStream_t stream);
 constexpr int kTailBlock = 256;
 cudaError_t launch_mb_gather(const void *table, uint32_t n_records, uint32_t iters, unsigned blocks, float *sink, cudaStream_t stream);
 cudaError_t launch_mb_ffma(uint32_t iters, unsigned blocks, float *sink, cudaStream_t stream);

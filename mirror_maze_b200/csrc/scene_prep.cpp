@@ -190,6 +190,39 @@ int prepare_scene(const mm_plane *planes, uint32_t n_planes, const mm_bvh_node *
         for (int k = 0; k < 3; k++) fast_ok = fast_ok && c[k] <= c[k + 3] && c[k + 6] <= c[k + 9];
     }
     out.n_pairs = n_pairs;
+    // y-table records (render_kernel.cuh, PairRecY): only for the exact fast form, and only while the children's distinct
+    // (min.y, max.y) intervals fit the table.  Intervals are told apart by their bits, so an entry's operands are exactly the
+    // bounds a PairRec of the same child holds.  A scene whose root is a leaf has no interior visit and keeps PairRec only.
+    if (fast_ok) {
+        out.pairs_y.assign(n_pairs ? n_pairs : 1, PairRecY());
+        std::memset(out.pairs_y.data(), 0, out.pairs_y.size() * sizeof(PairRecY));
+        auto y_index = [&](const mm_bvh_node &c) -> uint32_t {
+            const float4 iv = make_float4(c.aabb_min.y, c.aabb_max.y, c.aabb_max.y, c.aabb_min.y);
+            for (uint32_t j = 0; j < out.y_ivals.size(); j++)
+                if (std::memcmp(&out.y_ivals[j], &iv, sizeof(iv)) == 0) return j;
+            out.y_ivals.push_back(iv);
+            return (uint32_t)out.y_ivals.size() - 1u;
+        };
+        auto desc_y = [&](uint32_t c) -> uint32_t {
+            const mm_bvh_node &nd = nodes[c];
+            return nd.tri_count > 0 ? (kLeafBit | nd.left_first | (nd.tri_count << 24)) : pair_id[c] * (uint32_t)sizeof(PairRecY);
+        };
+        for (uint32_t i = 0; i < n_nodes && out.y_ivals.size() <= kMaxYIntervals; i++) {
+            if (!reachable[i] || nodes[i].tri_count != 0) continue;
+            const mm_bvh_node &a = nodes[nodes[i].left_first], &b = nodes[nodes[i].left_first + 1];
+            PairRecY &p = out.pairs_y[pair_id[i]];
+            for (int sz = 0; sz < 2; sz++)
+                for (int sx = 0; sx < 2; sx++) {
+                    p.xz[sx + 2 * sz][0] = make_float4(sx ? a.aabb_max.x : a.aabb_min.x, sx ? b.aabb_max.x : b.aabb_min.x,
+                                                       sx ? a.aabb_min.x : a.aabb_max.x, sx ? b.aabb_min.x : b.aabb_max.x);
+                    p.xz[sx + 2 * sz][1] = make_float4(sz ? a.aabb_max.z : a.aabb_min.z, sz ? b.aabb_max.z : b.aabb_min.z,
+                                                       sz ? a.aabb_min.z : a.aabb_max.z, sz ? b.aabb_min.z : b.aabb_max.z);
+                }
+            const uint32_t ya = y_index(a), yb = y_index(b);
+            p.link = make_uint4(desc_y(nodes[i].left_first), desc_y(nodes[i].left_first + 1), ya * kYEntryStride, yb * kYEntryStride);
+        }
+        if (out.y_ivals.empty() || out.y_ivals.size() > kMaxYIntervals) { out.pairs_y.clear(); out.y_ivals.clear(); }
+    }
     out.root_link = nodes[0].tri_count > 0 ? nodes[0].left_first : 0u;
     out.root_count = nodes[0].tri_count;
     out.depth = depth;

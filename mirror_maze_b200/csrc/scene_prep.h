@@ -12,6 +12,8 @@ struct Prepared {
     std::vector<RectI> rects;
     std::vector<RectS> shade;
     std::vector<RectA> rects_axis;   // filled when axis_ok
+    std::vector<PairRecY> pairs_y;   // filled when fast_ok and the children have at most kMaxYIntervals distinct y-intervals
+    std::vector<float4> y_ivals;     // those intervals as (min.y, max.y, max.y, min.y), in first-use order
     uint32_t n_pairs = 0, root_link = 0, root_count = 0, depth = 0, max_leaf = 0;
     bool fast_ok = false;        // box coordinates inside the guarded ranges of the shared-reciprocal slab quotient
     bool rect_fast_ok = false;   // edge lengths inside the guarded range of edge_thresholds

@@ -175,6 +175,21 @@ __device__ __forceinline__ void inner_step_packed(const ulonglong2 &A, const ulo
     descend<CNT>(lo1, hi1, lo2, hi2, lk, t, cur, sp, stack, tl);
 }
 
+// One interior visit of the y-table traversal (PairRecY): the same quotients, with the two children's y pairs read from the
+// per-lane table (y0 = child 0's (near.y, far.y), y1 = child 1's) instead of recomputed.  k holds x in both halves of its
+// first four pairs.  XZ = (c0.near.x, c1.near.x | c0.far.x, c1.far.x | c0.near.z, c1.near.z | c0.far.z, c1.far.z).
+template <bool CNT>
+__device__ __forceinline__ void inner_step_ytab(const Line32 &XZ, f2 y0, f2 y1, const uint2 &lk, const RayK &k, float t, uint32_t &cur,
+                                                uint32_t *&sp, const uint32_t *stack, Tally &tl) {
+    const f2 xn = quot2<false>(XZ.x, k.no_xy, k.nd_xy, k.r_xy, k.rl_xy), xf = quot2<false>(XZ.y, k.no_xy, k.nd_xy, k.r_xy, k.rl_xy);
+    const f2 zn = quot2<false>(XZ.z, k.no_zz, k.nd_zz, k.r_zz, k.rl_zz), zf = quot2<false>(XZ.w, k.no_zz, k.nd_zz, k.r_zz, k.rl_zz);
+    const float lo1 = fmaxf(fmaxf(lo2f(xn), lo2f(y0)), lo2f(zn));
+    const float hi1 = fminf(fminf(lo2f(xf), hi2f(y0)), lo2f(zf));
+    const float lo2 = fmaxf(fmaxf(hi2f(xn), lo2f(y1)), hi2f(zn));
+    const float hi2 = fminf(fminf(hi2f(xf), hi2f(y1)), hi2f(zf));
+    descend<CNT>(lo1, hi1, lo2, hi2, lk, t, cur, sp, stack, tl);
+}
+
 // One interior visit, general form: the literal min/max of shaders.metal:88-93 with NaN-dropping fmin/fmax, for rays whose
 // operands are outside the guarded ranges (zero / subnormal / huge / NaN components) or under MM_FLAG_FORCE_LITERAL.
 // Reads the record in its "up" order: a = (c0.min.x, c0.min.y, c0.max.x, c0.max.y), zu = (c0.min.z, c1.min.z, c0.max.z, c1.max.z).
@@ -285,21 +300,42 @@ constexpr int kRepUnroll = 2;                      // visits per loop trip: 2 me
 // budget for its per-ray constants.
 struct Hit { float t; uint32_t slot; };
 // AX = true: the scene's rects are all axis-aligned and `rects` points at RectA records (leaf_step_axis).
-template <bool MIXED, bool CNT, bool RCP, bool AX = false>
-__device__ __noinline__ Hit traverse(const PairRec *__restrict__ pairs, const void *__restrict__ rects, uint32_t root, bool alive,
-                                     bool lit, V3 ori, V3 dir, float beam_t, uint32_t beam_slot, Tally *tlp) {
+// YT = true (only with MIXED = false, RCP = false): `pairs` points at PairRecY records, and the ray's y quotients of the scene's
+// n_yiv y-intervals y_ivals are first written to the lane's column of the y-table, at byte `ytab` of the dynamic shared memory
+// (entry i at ytab + i * kYEntryStride), with the same operations a visit of the other form performs on them.
+extern __shared__ __align__(16) unsigned char mm_dyn_smem[];
+template <bool MIXED, bool CNT, bool RCP, bool AX = false, bool YT = false>
+__device__ __noinline__ Hit traverse(const void *__restrict__ pairs, const void *__restrict__ rects, uint32_t root, bool alive,
+                                     bool lit, V3 ori, V3 dir, float beam_t, uint32_t beam_slot, Tally *tlp,
+                                     uint32_t ytab = 0u, const float4 *__restrict__ y_ivals = nullptr, uint32_t n_yiv = 0u) {
+    static_assert(!YT || (!MIXED && !RCP), "the y-table traversal is the exact fast form only");
     Tally tl = {0u, 0u, 0u, 0u};
     uint32_t stack[MM_MAX_STACK];              // local memory (L1); BVH depth is validated against it at upload
     const float rx = __frcp_rn(dir.x), ry = __frcp_rn(dir.y), rz = __frcp_rn(dir.z);
     const float rlx = fmul(__fmaf_rn(-dir.x, rx, 1.0f), rx), rly = fmul(__fmaf_rn(-dir.y, ry, 1.0f), ry),
                 rlz = fmul(__fmaf_rn(-dir.z, rz, 1.0f), rz);
     RayK k;
-    k.no_xy = pack2(-ori.x, -ori.y); k.nd_xy = pack2(-dir.x, -dir.y); k.r_xy = pack2(rx, ry); k.rl_xy = pack2(rlx, rly);
+    if (YT) {
+        const f2 no_yy = pack2(-ori.y, -ori.y), nd_yy = pack2(-dir.y, -dir.y), r_yy = pack2(ry, ry), rl_yy = pack2(rly, rly);
+        const uint32_t sy = dir.y < 0.0f ? 8u : 0u;
+#pragma unroll
+        for (uint32_t i = 0; i < kMaxYIntervals; i++) {
+            if (i < n_yiv) {
+                const f2 b = __ldg(reinterpret_cast<const f2 *>(reinterpret_cast<const char *>(y_ivals + i) + sy));   // (near.y, far.y)
+                *reinterpret_cast<f2 *>(mm_dyn_smem + ytab + i * kYEntryStride) = quot2<false>(b, no_yy, nd_yy, r_yy, rl_yy);
+            }
+        }
+        k.no_xy = pack2(-ori.x, -ori.x); k.nd_xy = pack2(-dir.x, -dir.x); k.r_xy = pack2(rx, rx); k.rl_xy = pack2(rlx, rlx);
+    } else {
+        k.no_xy = pack2(-ori.x, -ori.y); k.nd_xy = pack2(-dir.x, -dir.y); k.r_xy = pack2(rx, ry); k.rl_xy = pack2(rlx, rly);
+    }
     k.no_zz = pack2(-ori.z, -ori.z); k.nd_zz = pack2(-dir.z, -dir.z); k.r_zz = pack2(rz, rz); k.rl_zz = pack2(rlz, rlz);
-    // per-ray record pointers with the travel order folded in: ab[sx + 2 sy] at +32 (sx + 2 sy), z|link[sz] at +128 + 32 sz
+    // per-ray record pointers with the travel order folded in: ab[sx + 2 sy] at +32 (sx + 2 sy), z|link[sz] at +128 + 32 sz;
+    // YT: xz[sx + 2 sz] at +32 (sx + 2 sz), link at +128
     const char *base = reinterpret_cast<const char *>(pairs);
-    const char *pAB = base + (lit ? 0 : (dir.x < 0.0f ? 32 : 0) + (dir.y < 0.0f ? 64 : 0));
-    const char *pZ = base + 128 + ((!lit && dir.z < 0.0f) ? 32 : 0);
+    const char *pAB = YT ? base + (dir.x < 0.0f ? 32 : 0) + (dir.z < 0.0f ? 64 : 0)
+                         : base + (lit ? 0 : (dir.x < 0.0f ? 32 : 0) + (dir.y < 0.0f ? 64 : 0));
+    const char *pZ = YT ? base + 128 : base + 128 + ((!lit && dir.z < 0.0f) ? 32 : 0);
     asm("" : "+l"(pAB)); asm("" : "+l"(pZ));      // keep them live: ptxas otherwise re-derives them from sign(dir) at every node
     // The pair table lies inside one 4-GB-aligned window (checked at upload), so a record address is {hi, lo + offset} with
     // no carry: one 32-bit add per pointer instead of a 64-bit add (two instructions).
@@ -321,7 +357,16 @@ __device__ __noinline__ Hit traverse(const PairRec *__restrict__ pairs, const vo
                 if ((cur & kLeafBit) == 0u) {
                     const size_t off = cur;                      // interior descriptors are byte offsets
                     if (CNT) tl.inner++;
-                    if (!MIXED || !lit) {
+                    if (YT) {
+                        uint64_t aXZ, aL;
+                        asm("mov.b64 %0, {%1, %2};" : "=l"(aXZ) : "r"(ab_lo + cur), "r"(hi_a));
+                        asm("mov.b64 %0, {%1, %2};" : "=l"(aL) : "r"(z_lo + cur), "r"(hi_z));
+                        const Line32 xz = ldg256(reinterpret_cast<const void *>(aXZ));
+                        const uint4 lk = __ldg(reinterpret_cast<const uint4 *>(aL));
+                        const f2 y0 = *reinterpret_cast<const f2 *>(mm_dyn_smem + ytab + lk.z);
+                        const f2 y1 = *reinterpret_cast<const f2 *>(mm_dyn_smem + ytab + lk.w);
+                        inner_step_ytab<CNT>(xz, y0, y1, make_uint2(lk.x, lk.y), k, t, cur, sp, stack, tl);
+                    } else if (!MIXED || !lit) {
                         // 32-B load for (A, B): measured 1.5 % faster than two 16-B loads; folding (Z, link) into a second
                         // 32-B load gave nothing (profiles/r1_block_shape.txt)
                         uint64_t aAB, aZ;
