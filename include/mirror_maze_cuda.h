@@ -313,7 +313,8 @@ int mm_microbench(mm_ctx *ctx, int kind, uint64_t table_bytes, double *result);
 /*
  * Self-test of the kernel's shared-reciprocal slab quotient (see render_kernel.cu header): evaluates n_pairs
  * pseudo-random (x, d) pairs inside the guarded ranges, half of them adjacent to rounding midpoints, with both
- * the fast sequence and __fdiv_rn, and returns how many differ (must be 0).
+ * the fast sequence (scalar, and packed with non-zero origins as the traversal runs it) and __fdiv_rn, then a fixed
+ * set of edge operands (docs/exact_quotient.md, Evidence), and returns how many differ (must be 0).
  */
 int mm_selftest_quotient(mm_ctx *ctx, uint64_t n_pairs, uint64_t seed, uint64_t *mismatches);
 /* The present blur divides by 3 (shaders.metal:222) with a three-operation exact sequence instead of the IEEE divide; this
@@ -337,6 +338,19 @@ int mm_rect_edge_thresholds(float length, float *lo, float *up);
  * when the rect is not axis-aligned (a scene with such a rect uses the general test throughout).  Host-only.
  */
 int mm_axis_rect(const mm_plane *plane, float out[5], uint32_t *k);
+/*
+ * Verification hook for the traversal (intersect_bvh_iterative, shaders.metal:115-156) ray by ray, on the uploaded scene.
+ * rays: n x 8 floats (ori.xyz, dir.xyz, starting t, alive: non-zero = traced); slots: n starting slots in leaf order (the
+ * beam's index before the call), or NULL for none (0xFFFFFFFF).  Rays go 32 to a warp in the order given (a partial last warp
+ * has dead lanes), and each warp selects its traversal form exactly as the bounce loop of mm_render does under the same
+ * flags: MM_FLAG_FORCE_LITERAL, MM_FLAG_RCP_SLAB, MM_FLAG_GENERAL_RECTS and MM_FLAG_NO_Y_TABLE (any other flag is
+ * MM_ERR_INVALID).  Per ray: t_out = the returned t; index_out = the hit's plane index, as mm_debug.first_hit reports it
+ * (0xFFFFFFFF for none); tally_out = 6 words (interior visits, leaf visits, rect tests, deepest stack occupancy, lit = 1 when
+ * the ray needs the literal-divide slab form, form = the traversal its warp ran: bit 0 mixed literal, bit 1 reciprocal-
+ * multiply, bit 2 axis-aligned rect test, bit 3 y-table).  A dead ray returns its t and slot and counts nothing.  Synchronous.
+ */
+int mm_trace_rays(mm_ctx *ctx, uint32_t flags, const float *rays, const uint32_t *slots, uint32_t n,
+                  float *t_out, uint32_t *index_out, uint32_t *tally_out);
 
 /* ---- One process, several GPUs (SURVEY §8 b/e) ---------------------------------------------------------------------- */
 

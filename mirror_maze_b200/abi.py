@@ -145,6 +145,7 @@ PROTOTYPES = {
     "mm_render_peers_device": (C.c_int, [_vp, _P(Uniform), _P(Params), _P(C.c_void_p), C.c_uint32]),
     "mm_rect_edge_thresholds": (C.c_int, [C.c_float, _P(C.c_float), _P(C.c_float)]),
     "mm_axis_rect": (C.c_int, [_P(Plane), _P(C.c_float), _P(C.c_uint32)]),
+    "mm_trace_rays": (C.c_int, [_vp, C.c_uint32, _vp, _vp, C.c_uint32, _vp, _vp, _vp]),
     "mm_microbench": (C.c_int, [_vp, C.c_int, C.c_uint64, _P(C.c_double)]),
     "mm_present": (C.c_int, [_vp, _vp]),
     "mm_present_rgba8": (C.c_int, [_vp, _vp, _vp]),

@@ -259,6 +259,29 @@ static bool configure_pool(mm_ctx *ctx, const mm_params *par, Launch &L) {
     return true;
 }
 
+// The scene and flag part of a launch's parameters, shared by every render and by mm_trace_rays: the BVH root, the tables,
+// and the arithmetic and rect form the traversal uses under flags (MM_FLAG_FORCE_LITERAL, MM_FLAG_RCP_SLAB,
+// MM_FLAG_GENERAL_RECTS, MM_FLAG_NO_Y_TABLE).  Returns whether the y-table traversal applies (trace_ytab_kernel, DESIGN.md
+// §3-4): it covers the exact slab arithmetic of scenes that have the table; MM_FLAG_NO_Y_TABLE keeps trace_kernel for
+// comparisons.  The y-table fields are set only then.
+bool traversal_params(const mm_ctx *ctx, uint32_t flags, KParams &p) {
+    p.n_pairs = ctx->n_pairs; p.n_slots = ctx->n_slots;
+    p.root_link = ctx->root_link; p.root_count = ctx->root_count;
+    p.force_literal = (flags & MM_FLAG_FORCE_LITERAL) ? 1u : 0u;
+    p.rcp_mode = (flags & MM_FLAG_RCP_SLAB) ? 1u : 0u;
+    p.scene_fast_ok = ctx->fast_ok ? 1u : 0u;
+    p.rect_fast_ok = (ctx->rect_fast_ok && !(flags & MM_FLAG_FORCE_LITERAL)) ? 1u : 0u;
+    p.pairs = ctx->d_pairs; p.rects = ctx->d_rects; p.shade = ctx->d_shade;
+    p.rects_axis = (p.rect_fast_ok && !(flags & MM_FLAG_GENERAL_RECTS)) ? ctx->d_rects_axis : nullptr;
+    const bool ytab = ctx->n_yiv && !p.force_literal && !p.rcp_mode && p.scene_fast_ok && !(flags & MM_FLAG_NO_Y_TABLE);
+    if (ytab) {
+        p.pairs_y = ctx->d_pairs_y;
+        p.y_ivals = reinterpret_cast<const float4 *>(ctx->d_pairs_y + ctx->n_pairs_y);
+        p.n_yiv = ctx->n_yiv;
+    }
+    return ytab;
+}
+
 int build_launch(mm_ctx *ctx, const mm_uniform *uni, const mm_params *par, bool debug, Launch &L) {
     if (!uni || !par) return fail(ctx, MM_ERR_INVALID, "null uniform or params");
     if (!ctx->have_scene) return fail(ctx, MM_ERR_NO_SCENE, "no scene uploaded");
@@ -292,17 +315,10 @@ int build_launch(mm_ctx *ctx, const mm_uniform *uni, const mm_params *par, bool 
     p.dim_y = p.T / p.dim_x;
     p.ppc = chunk * chunk;
     p.W = (uint32_t)uni->view_width; p.H = (uint32_t)uni->view_height;
-    p.n_pairs = ctx->n_pairs; p.n_slots = ctx->n_slots;
-    p.root_link = ctx->root_link; p.root_count = ctx->root_count;
     p.noise_w = ctx->noise_w; p.noise_h = ctx->noise_h;
-    p.force_literal = (par->flags & MM_FLAG_FORCE_LITERAL) ? 1u : 0u;
-    p.rcp_mode = (par->flags & MM_FLAG_RCP_SLAB) ? 1u : 0u;
-    p.scene_fast_ok = ctx->fast_ok ? 1u : 0u;
+    const bool ytab = traversal_params(ctx, par->flags, p);
     p.quant8 = (par->flags & MM_FLAG_SCREEN_RGBA8) ? 1u : 0u;
-    p.rect_fast_ok = (ctx->rect_fast_ok && !(par->flags & MM_FLAG_FORCE_LITERAL)) ? 1u : 0u;
     p.total_paths = (uint64_t)count * T;
-    p.pairs = ctx->d_pairs; p.rects = ctx->d_rects; p.shade = ctx->d_shade;
-    p.rects_axis = (p.rect_fast_ok && !(par->flags & MM_FLAG_GENERAL_RECTS)) ? ctx->d_rects_axis : nullptr;
     p.chunks = ctx->d_chunks; p.noise = ctx->d_noise;
     p.counters = ctx->d_counters;
 
@@ -349,14 +365,7 @@ int build_launch(mm_ctx *ctx, const mm_uniform *uni, const mm_params *par, bool 
         p.tail_q = ctx->d_tail_q;
         p.tail_pix = ctx->d_tail_pix;
     }
-    // The y-table traversal (trace_ytab_kernel, DESIGN.md §3-4) covers the exact slab arithmetic of scenes that have the table;
-    // MM_FLAG_NO_Y_TABLE keeps trace_kernel for comparisons.
-    L.choice.ytab = !L.choice.regroup && ctx->n_yiv && !p.force_literal && !p.rcp_mode && p.scene_fast_ok && !(par->flags & MM_FLAG_NO_Y_TABLE);
-    if (L.choice.ytab) {
-        p.pairs_y = ctx->d_pairs_y;
-        p.y_ivals = reinterpret_cast<const float4 *>(ctx->d_pairs_y + ctx->n_pairs_y);
-        p.n_yiv = ctx->n_yiv;
-    }
+    L.choice.ytab = !L.choice.regroup && ytab;
     L.smem = 3 * (size_t)bt * sizeof(float);                             // reduction scratch
     if (L.choice.ytab) L.smem += (size_t)(bt / 32) * p.n_yiv * kYEntryStride;                 // y-table: [warp][interval][lane]
     if (L.choice.regroup) L.smem += 4 * (size_t)bt * sizeof(float4) + 64 * sizeof(uint32_t);   // path state in flight + bin counters
@@ -813,6 +822,41 @@ int mm_selftest_quotient(mm_ctx *ctx, uint64_t n_pairs, uint64_t seed, uint64_t 
     CK(cudaMemcpyAsync(ctx->h_counters, ctx->d_counters, sizeof(Counters), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     *mismatches = ctx->h_counters->paths;
+    return MM_OK;
+}
+
+int mm_trace_rays(mm_ctx *ctx, uint32_t flags, const float *rays, const uint32_t *slots, uint32_t n, float *t_out, uint32_t *index_out,
+                  uint32_t *tally_out) {
+    if (!ctx) return MM_ERR_INVALID;
+    ctx->err.clear();
+    if (!rays || !t_out || !index_out || !tally_out || n == 0) return fail(ctx, MM_ERR_INVALID, "mm_trace_rays: null pointer or zero size");
+    if (n > (1u << 30)) return fail(ctx, MM_ERR_UNSUPPORTED, "mm_trace_rays: more than 2^30 rays in one call");
+    if (flags & ~(MM_FLAG_FORCE_LITERAL | MM_FLAG_RCP_SLAB | MM_FLAG_GENERAL_RECTS | MM_FLAG_NO_Y_TABLE))
+        return fail(ctx, MM_ERR_INVALID, "mm_trace_rays: flags other than FORCE_LITERAL, RCP_SLAB, GENERAL_RECTS and NO_Y_TABLE");
+    if (!ctx->have_scene) return fail(ctx, MM_ERR_NO_SCENE, "no scene uploaded");
+    if (slots)
+        for (uint32_t i = 0; i < n; i++)
+            if (slots[i] != 0xFFFFFFFFu && slots[i] >= ctx->n_slots) return fail(ctx, MM_ERR_INVALID, "mm_trace_rays: slot out of range");
+    KParams p;
+    memset(&p, 0, sizeof(p));
+    const bool ytab = traversal_params(ctx, flags, p);
+    CK(cudaSetDevice(ctx->device));
+    // one allocation: rays (8 floats), slot, t, index, tallies (6 words) per ray
+    const size_t rays_b = (size_t)n * 8 * sizeof(float), word_b = (size_t)n * sizeof(uint32_t);
+    char *buf = nullptr;
+    CK(cudaMalloc(&buf, rays_b + 9 * word_b));
+    float *d_rays = reinterpret_cast<float *>(buf), *d_t = reinterpret_cast<float *>(buf + rays_b + word_b);
+    uint32_t *d_slots = reinterpret_cast<uint32_t *>(buf + rays_b), *d_index = reinterpret_cast<uint32_t *>(buf + rays_b + 2 * word_b);
+    uint32_t *d_tally = reinterpret_cast<uint32_t *>(buf + rays_b + 3 * word_b);
+    cudaError_t e = cudaMemcpyAsync(d_rays, rays, rays_b, cudaMemcpyHostToDevice, ctx->stream);
+    if (e == cudaSuccess && slots) e = cudaMemcpyAsync(d_slots, slots, word_b, cudaMemcpyHostToDevice, ctx->stream);
+    if (e == cudaSuccess) e = launch_probe(p, ytab, d_rays, slots ? d_slots : nullptr, n, d_t, d_index, d_tally, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(t_out, d_t, word_b, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(index_out, d_index, word_b, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(tally_out, d_tally, 6 * word_b, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    cudaFree(buf);
+    if (e != cudaSuccess) return fail(ctx, MM_ERR_CUDA, std::string("mm_trace_rays: ") + cudaGetErrorString(e));
     return MM_OK;
 }
 

@@ -68,6 +68,7 @@ struct Launch {
 };
 
 int fail(mm_ctx *ctx, int code, const std::string &msg);
+bool traversal_params(const mm_ctx *ctx, uint32_t flags, mmk::KParams &p);
 int build_launch(mm_ctx *ctx, const mm_uniform *uni, const mm_params *par, bool debug, Launch &L);
 int do_launch(mm_ctx *ctx, Launch &L);
 int ensure_screen(mm_ctx *ctx, uint32_t W, uint32_t H);

@@ -141,31 +141,51 @@ __device__ __forceinline__ void block_epilogue(const KParams &P, float *red, boo
     add_counters<CNT>(P, seg, nhits, nliteral, active ? 1u : 0u, tl);
 }
 
+// Which traverse<MIXED, CNT, RCP, AX, YT> instantiation a warp ran, as bits (reported by probe_rays_kernel).
+constexpr uint32_t kFormMixed = 1u, kFormRcp = 2u, kFormAxis = 4u, kFormYTable = 8u;
+
+// One traversal for the lanes of a warp together, in the form the warp selects: a warp with a live literal lane (or a scene
+// without the divide-free rect test) runs the mixed form, any other the y-table (YT), reciprocal-multiply or plain packed
+// form, with the axis-aligned rect test where the scene has it.  lit: this lane's ray is literal; form: the kForm* bits of
+// the instantiation that ran, written only when FORM (so that the bounce loop compiles exactly as without it).  YT: the host
+// selects it only without MM_FLAG_RCP_SLAB; ytab is the lane's column of the y-table in dynamic shared memory.
+template <bool CNT, bool YT, bool FORM = false>
+__device__ __forceinline__ Hit warp_traverse(const KParams &P, uint32_t root, const bool &alive, const V3 &ori, const V3 &dir, const float &t,
+                                             const uint32_t &slot, Tally &tl, uint32_t ytab, bool &lit, uint32_t &form) {
+    lit = ray_is_literal(P, ori, dir);
+    const bool any_lit = __any_sync(0xFFFFFFFFu, alive && lit) || !P.rect_fast_ok;   // MIXED also means literal rect tests
+    Hit h;
+    if (YT) {
+        if (!any_lit && P.rects_axis) {
+            h = traverse<false, CNT, false, true, true>(P.pairs_y, P.rects_axis, root, alive, false, ori, dir, t, slot, &tl, ytab, P.y_ivals, P.n_yiv);
+            if (FORM) form = kFormYTable | kFormAxis;
+        } else if (!any_lit) {
+            h = traverse<false, CNT, false, false, true>(P.pairs_y, P.rects, root, alive, false, ori, dir, t, slot, &tl, ytab, P.y_ivals, P.n_yiv);
+            if (FORM) form = kFormYTable;
+        } else {
+            h = traverse<true, CNT, false>(P.pairs, P.rects, root, alive, lit, ori, dir, t, slot, &tl);
+            if (FORM) form = kFormMixed;
+        }
+    } else if (P.rcp_mode) {
+        if (!any_lit) { h = traverse<false, CNT, true>(P.pairs, P.rects, root, alive, false, ori, dir, t, slot, &tl); if (FORM) form = kFormRcp; }
+        else { h = traverse<true, CNT, true>(P.pairs, P.rects, root, alive, lit, ori, dir, t, slot, &tl); if (FORM) form = kFormMixed | kFormRcp; }
+    } else {
+        if (!any_lit && P.rects_axis) { h = traverse<false, CNT, false, true>(P.pairs, P.rects_axis, root, alive, false, ori, dir, t, slot, &tl); if (FORM) form = kFormAxis; }
+        else if (!any_lit) { h = traverse<false, CNT, false>(P.pairs, P.rects, root, alive, false, ori, dir, t, slot, &tl); if (FORM) form = 0u; }
+        else { h = traverse<true, CNT, false>(P.pairs, P.rects, root, alive, lit, ori, dir, t, slot, &tl); if (FORM) form = kFormMixed; }
+    }
+    return h;
+}
+
 // One segment of the bounce loop (shaders.metal:306-340) for the lanes of a warp together: traverse, then shade the hit of
 // every live lane.  A lane whose path has ended (or that has no path) idles with alive = false.
-// YT: warps without literal lanes take the y-table traversal (the host selects YT only without MM_FLAG_RCP_SLAB); ytab is the
-// lane's column of the y-table in dynamic shared memory.
 template <bool CNT, bool DBG, bool YT>
 __device__ __forceinline__ void bounce_segment(const KParams &P, uint32_t root, bool &alive, V3 &ori, V3 &dir, V3 &color, V3 &light, float &t,
                                                uint32_t &slot, uint32_t &state, int &n, int &mirror_hits, uint32_t &first_hit,
                                                uint32_t &seg, uint32_t &nhits, uint32_t &nliteral, Tally &tl, uint32_t ytab) {
-    const bool lit = ray_is_literal(P, ori, dir);
-    const bool any_lit = __any_sync(0xFFFFFFFFu, alive && lit) || !P.rect_fast_ok;   // MIXED also means literal rect tests
-    Hit h;
-    if (YT) {
-        if (!any_lit && P.rects_axis)
-            h = traverse<false, CNT, false, true, true>(P.pairs_y, P.rects_axis, root, alive, false, ori, dir, t, slot, &tl, ytab, P.y_ivals, P.n_yiv);
-        else if (!any_lit)
-            h = traverse<false, CNT, false, false, true>(P.pairs_y, P.rects, root, alive, false, ori, dir, t, slot, &tl, ytab, P.y_ivals, P.n_yiv);
-        else h = traverse<true, CNT, false>(P.pairs, P.rects, root, alive, lit, ori, dir, t, slot, &tl);
-    } else if (P.rcp_mode) {
-        if (!any_lit) h = traverse<false, CNT, true>(P.pairs, P.rects, root, alive, false, ori, dir, t, slot, &tl);
-        else h = traverse<true, CNT, true>(P.pairs, P.rects, root, alive, lit, ori, dir, t, slot, &tl);
-    } else {
-        if (!any_lit && P.rects_axis) h = traverse<false, CNT, false, true>(P.pairs, P.rects_axis, root, alive, false, ori, dir, t, slot, &tl);
-        else if (!any_lit) h = traverse<false, CNT, false>(P.pairs, P.rects, root, alive, false, ori, dir, t, slot, &tl);
-        else h = traverse<true, CNT, false>(P.pairs, P.rects, root, alive, lit, ori, dir, t, slot, &tl);
-    }
+    bool lit;
+    uint32_t form;
+    const Hit h = warp_traverse<CNT, YT>(P, root, alive, ori, dir, t, slot, tl, ytab, lit, form);
     t = h.t; slot = h.slot;
     if (alive) {
         if (lit) nliteral++;
@@ -326,6 +346,41 @@ trace_tail_kernel(const __grid_constant__ KParams P) {
         }
     }
     add_counters<CNT>(P, seg, nhits, nliteral, 0u, tl);
+}
+
+// Verification hook (mm_trace_rays): one traversal per ray through the bounce loop's form selection, 32 consecutive rays to a
+// warp, so that the caller decides each warp's composition.  rays: n x 8 floats (ori.xyz, dir.xyz, t, alive != 0); slots: the
+// starting slots, or null for none.  Per ray: the returned t, the hit's plane index (the shading record's original index, as
+// shade_hit reports first_hit; 0xFFFFFFFF for no slot) and (inner, leaf, rect, max_stack, lit, form).  A dead ray keeps its
+// t and slot and counts nothing.  YT: the y-table traversal; the table is the whole dynamic shared memory, [warp][interval][lane].
+template <bool YT>
+__global__ void __launch_bounds__(kProbeBlock)
+probe_rays_kernel(const __grid_constant__ KParams P, const float *__restrict__ rays, const uint32_t *__restrict__ slots, uint32_t n,
+                  float *__restrict__ t_out, uint32_t *__restrict__ index_out, uint32_t *__restrict__ tally_out) {
+    const uint32_t i = blockIdx.x * kProbeBlock + threadIdx.x;
+    const bool has = i < n;
+    const uint32_t root = P.root_count ? (kLeafBit | P.root_link | (P.root_count << 24)) : P.root_link;
+    const uint32_t ytab = YT ? (threadIdx.x >> 5) * P.n_yiv * kYEntryStride + (threadIdx.x & 31u) * 8u : 0u;
+    V3 ori = mk(0.0f, 0.0f, 0.0f), dir = mk(1.0f, 1.0f, 1.0f);
+    float t = 1e30f;
+    uint32_t slot = 0xFFFFFFFFu;
+    bool alive = false;
+    if (has) {
+        const float *r = rays + 8 * (size_t)i;
+        ori = mk(r[0], r[1], r[2]); dir = mk(r[3], r[4], r[5]); t = r[6];
+        alive = r[7] != 0.0f;
+        if (slots) slot = slots[i];
+    }
+    Tally tl = {0u, 0u, 0u, 0u};
+    bool lit;
+    uint32_t form;
+    const Hit h = warp_traverse<true, YT, true>(P, root, alive, ori, dir, t, slot, tl, ytab, lit, form);
+    if (has) {
+        t_out[i] = h.t;
+        index_out[i] = h.slot == 0xFFFFFFFFu ? 0xFFFFFFFFu : __float_as_uint(__ldg(reinterpret_cast<const float4 *>(P.shade + h.slot) + 1).w);
+        uint32_t *o = tally_out + 6 * (size_t)i;
+        o[0] = tl.inner; o[1] = tl.leaf; o[2] = tl.rect; o[3] = tl.max_stack; o[4] = lit ? 1u : 0u; o[5] = form;
+    }
 }
 
 // ---- trace_kernel_rg: the same kernel with the block's paths RE-FORMED INTO WARPS at every segment boundary ---------------------
@@ -491,45 +546,103 @@ __global__ void scatter_all_kernel(const float4 *__restrict__ gathered, float4 *
     if (x < W && y < H) image[(size_t)y * W + x] = gathered[i];
 }
 
-// Self-test of the shared-reciprocal quotient against __fdiv_rn on pseudo-random operands inside the guarded ranges
-// (|d| in [2^-60, 2^60], x = 0 or |x| in [2^-40, 2^31]); half of the samples are built to land within a few
-// 2^-24 ulp of a rounding midpoint, the only place where a faithful-but-not-exact quotient could differ.
+// Self-test of the shared-reciprocal quotient against __fdiv_rn, through the scalar quot<true> and through quot2, the packed
+// sequence the traversal runs (b + (-o), then mul, fma, fma, fma).  Pseudo-random operands inside the guarded ranges
+// (|d| in [2^-60, 2^60], x = RN(b - o) = 0 or |x| in [2^-40, 2^31]); half of the samples are built to land within a few
+// 2^-24 ulp of a rounding midpoint, the only place where a faithful-but-not-exact quotient could differ, with quotient
+// exponents over the whole [-100, 91] the ranges allow.  A deterministic pass then covers the edge operands (below).
 __device__ __forceinline__ uint32_t mix32(uint64_t &s) {
     s = s * 6364136223846793005ull + 1442695040888963407ull;
     uint32_t x = (uint32_t)(((s >> 18) ^ s) >> 27), r = (uint32_t)(s >> 59);
     return (x >> r) | (x << ((32 - r) & 31));
 }
+__device__ __forceinline__ float with_exp(uint32_t bits, int e) { return __uint_as_float((bits & 0x807FFFFFu) | ((uint32_t)(e + 127) << 23)); }
+__device__ __forceinline__ bool d_guarded(float d) { return fabsf(d) >= 8.673617379884035e-19f /*2^-60*/ && fabsf(d) <= 1.152921504606847e18f /*2^60*/; }
+__device__ __forceinline__ bool x_guarded(float x) { return x == 0.0f || (fabsf(x) >= 9.094947017729282e-13f /*2^-40*/ && fabsf(x) <= 2147483648.0f /*2^31*/); }
+
+// One pseudo-random sample (x, d); false when it falls outside the guarded ranges.  keep_d: build x for the d given.
+__device__ __forceinline__ bool quot_sample(uint64_t &s, float &x, float &d, bool keep_d) {
+    const uint32_t a = mix32(s), b = mix32(s), c = mix32(s);
+    if (c & 1u) {
+        // adversarial: x ~ (q + half ulp(q)) * d for a random q, so x/d sits next to a rounding midpoint
+        const int eq = (int)(a % 192u) - 100;                              // quotient exponent in [-100, 91]
+        if (!keep_d) {                                                     // d's exponent such that |q d| can lie in [2^-40, 2^31]
+            const int lo = max(-60, -41 - eq), hi = min(60, 31 - eq);
+            d = with_exp(b, lo + (int)(mix32(s) % (uint32_t)(hi - lo + 1)));
+        }
+        const float q = with_exp(mix32(s), eq);
+        double mid = (double)q + 0.5 * (double)(__uint_as_float(__float_as_uint(fabsf(q)) + 1u) - fabsf(q)) * (q < 0 ? -1.0 : 1.0);
+        x = (float)(mid * (double)d);
+        if ((c >> 1) & 1u) x = __uint_as_float(__float_as_uint(x) + ((c >> 2) & 3u) - 1u);   // +-1 ulp neighbours
+    } else {
+        if (!keep_d) d = with_exp(b, (int)(a % 121u) - 60);
+        x = with_exp(mix32(s), (int)((c >> 1) % 72u) - 40);
+        if (((c >> 8) & 63u) == 0u) x = 0.0f;
+    }
+    return d_guarded(d) && x_guarded(x);
+}
+
+// An origin o for which b = RN(x + o) and RN(b - o) = x hold exactly: 0, or -sign(x) y with y = |x| with its low mantissa
+// bits masked and scaled by 2^-k, a multiple of ulp(x) not above |x|, so that |b| = |x| - y lies on x's grid.
+__device__ __forceinline__ float origin_for(float x, uint32_t salt) {
+    if ((salt & 3u) == 0u || x == 0.0f) return 0.0f;
+    const uint32_t k = (salt >> 2) & 7u;
+    const uint32_t keep = 0xFF800000u | ((salt >> 5) & 0x7FFFFFu & ~((1u << k) - 1u));
+    const float y = fmul(__uint_as_float(__float_as_uint(fabsf(x)) & keep), __uint_as_float((uint32_t)(127 - k) << 23));
+    return x > 0.0f ? -y : y;
+}
+
+__device__ __forceinline__ bool same_quot(float a, float b) { return __float_as_uint(a) == __float_as_uint(b) || (a == 0.0f && b == 0.0f); }
+
+// Mismatches of three samples against __fdiv_rn: (x0, d0) and (x1, d1) through the scalar form (o = 0) and as the two halves
+// of one packed quotient with their own origins (the interior visit's x|y pair); (x0, d0) and (x2, d0) as the halves of the
+// y-table fill's form, one origin and one direction duplicated (has2: x2 is a sample).
+__device__ uint32_t quot_check(float x0, float d0, float x1, float d1, float x2, bool has2, uint32_t salt) {
+    Axis a0, a1;
+    a0.o = 0.0f; a0.d = d0; a0.r = __frcp_rn(d0); a0.rl = fmul(__fmaf_rn(-d0, a0.r, 1.0f), a0.r);
+    a1.o = 0.0f; a1.d = d1; a1.r = __frcp_rn(d1); a1.rl = fmul(__fmaf_rn(-d1, a1.r, 1.0f), a1.r);
+    uint32_t bad = 0;
+    bad += !same_quot(quot<true>(x0, a0), quot<false>(x0, a0));
+    bad += !same_quot(quot<true>(x1, a1), quot<false>(x1, a1));
+    const float o0 = origin_for(x0, salt), o1 = origin_for(x1, salt >> 10);
+    const float b0 = fadd(x0, o0), b1 = fadd(x1, o1);
+    const f2 q = quot2<false>(pack2(b0, b1), pack2(-o0, -o1), pack2(-d0, -d1), pack2(a0.r, a1.r), pack2(a0.rl, a1.rl));
+    bad += !same_quot(lo2f(q), fdiv(fsub(b0, o0), d0));
+    bad += !same_quot(hi2f(q), fdiv(fsub(b1, o1), d1));
+    const float b2 = fadd(x2, o0);
+    if (has2 && x_guarded(fsub(b2, o0))) {
+        const f2 qy = quot2<false>(pack2(b0, b2), pack2(-o0, -o0), pack2(-d0, -d0), pack2(a0.r, a0.r), pack2(a0.rl, a0.rl));
+        bad += !same_quot(lo2f(qy), fdiv(fsub(b0, o0), d0));
+        bad += !same_quot(hi2f(qy), fdiv(fsub(b2, o0), d0));
+    }
+    return bad;
+}
+
+// Edge operands of the deterministic pass: d = +-m 2^k for k in [-60, 60] and x = +-m 2^k for k in [-40, 31], m = 1 (powers of
+// two: rho = rl = 0), 1 + 2^-23 or 2 - 2^-23 (all-ones mantissa), plus x = 0; those past 2^60 or 2^31 are skipped.  The
+// pairs include |d| = 2^-60 and 2^60 with their inside neighbours, |x| = 2^-40 and 2^31 with theirs, and the tiny-x, huge-d
+// combinations whose p = x rl and e r are subnormal.
+constexpr uint32_t kEdgeD = 2u * 3u * 121u, kEdgeX = 2u * 3u * 72u + 1u;
+__device__ __forceinline__ float edge_operand(uint32_t i, int k0) {
+    const uint32_t m = (i >> 1) % 3u, mant = m == 0u ? 0u : (m == 1u ? 1u : 0x7FFFFFu);
+    return __uint_as_float(((i & 1u) << 31) | ((uint32_t)((int)((i >> 1) / 3u) + k0 + 127) << 23) | mant);
+}
+
 __global__ void quot_selftest_kernel(uint64_t n, uint64_t seed, unsigned long long *mismatches) {
     const uint64_t tid = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x, stride = (uint64_t)gridDim.x * blockDim.x;
     uint64_t s = seed ^ (tid * 0x9E3779B97F4A7C15ull);
     unsigned long long bad = 0;
     for (uint64_t i = tid; i < n; i += stride) {
-        const uint32_t a = mix32(s), b = mix32(s), c = mix32(s);
-        // d: random sign/mantissa, exponent in [-60, 59]
-        const int ed = (int)(a % 120u) - 60;
-        float d = __uint_as_float((b & 0x807FFFFFu) | ((uint32_t)(ed + 127) << 23));
-        float x;
-        if (c & 1u) {
-            // adversarial: x ~ (q + half ulp(q)) * d for a random q, so x/d sits next to a rounding midpoint
-            const uint32_t qm = mix32(s);
-            const int eq = (int)(qm % 40u) - 20;
-            float q = __uint_as_float((mix32(s) & 0x807FFFFFu) | ((uint32_t)(eq + 127) << 23));
-            double mid = (double)q + 0.5 * (double)(__uint_as_float(__float_as_uint(fabsf(q)) + 1u) - fabsf(q)) * (q < 0 ? -1.0 : 1.0);
-            x = (float)(mid * (double)d);
-            if ((c >> 1) & 1u) x = __uint_as_float(__float_as_uint(x) + ((c >> 2) & 3u) - 1u);   // +-1 ulp neighbours
-        } else {
-            const int ex = (int)((c >> 1) % 71u) - 40;
-            x = __uint_as_float((mix32(s) & 0x807FFFFFu) | ((uint32_t)(ex + 127) << 23));
-            if (((c >> 8) & 63u) == 0u) x = 0.0f;
-        }
-        const float ax = fabsf(x);
-        if (!(ax == 0.0f || (ax >= 9.094947017729282e-13f && ax <= 2147483648.0f))) continue;
-        Axis ax_;
-        ax_.o = 0.0f; ax_.d = d;
-        ax_.r = __frcp_rn(d); ax_.rl = fmul(__fmaf_rn(-d, ax_.r, 1.0f), ax_.r);
-        const float qf = quot<true>(x, ax_), ql = quot<false>(x, ax_);
-        const bool same = (__float_as_uint(qf) == __float_as_uint(ql)) || (qf == 0.0f && ql == 0.0f);
-        if (!same) bad++;
+        float x0, d0, x1, d1, x2;
+        const bool ok0 = quot_sample(s, x0, d0, false), ok1 = quot_sample(s, x1, d1, false);
+        float d2 = d0;
+        const bool ok2 = quot_sample(s, x2, d2, true);
+        if (ok0 && ok1) bad += quot_check(x0, d0, x1, d1, x2, ok2, mix32(s));
+    }
+    for (uint64_t i = tid; i < (uint64_t)kEdgeD * kEdgeX; i += stride) {
+        const uint32_t id = (uint32_t)(i / kEdgeX), ix = (uint32_t)(i % kEdgeX);
+        const float d = edge_operand(id, -60), x = ix == kEdgeX - 1u ? 0.0f : edge_operand(ix, -40);
+        if (d_guarded(d) && x_guarded(x)) bad += quot_check(x, d, x, -d, -x, true, (uint32_t)i * 2654435761u);
     }
     if (bad) atomicAdd(mismatches, bad);
 }
@@ -662,6 +775,16 @@ cudaError_t launch_tail(const KParams &p, KernelChoice c, unsigned blocks, size_
     const void *fn = c.debug ? tail_ptr<true, true>(c.ytab) : (c.counters ? tail_ptr<true, false>(c.ytab) : tail_ptr<false, false>(c.ytab));
     void *args[] = {const_cast<KParams *>(&p)};
     return cudaLaunchKernel(fn, dim3(blocks), dim3(kTailBlock), args, smem_bytes, stream);
+}
+
+cudaError_t launch_probe(const KParams &p, bool ytab, const float *rays, const uint32_t *slots, uint32_t n, float *t_out, uint32_t *index_out,
+                         uint32_t *tally_out, cudaStream_t stream) {
+    const unsigned blocks = (n + kProbeBlock - 1) / kProbeBlock;
+    if (ytab)
+        probe_rays_kernel<true><<<blocks, kProbeBlock, (size_t)(kProbeBlock / 32) * p.n_yiv * kYEntryStride, stream>>>(p, rays, slots, n, t_out, index_out, tally_out);
+    else
+        probe_rays_kernel<false><<<blocks, kProbeBlock, 0, stream>>>(p, rays, slots, n, t_out, index_out, tally_out);
+    return cudaGetLastError();
 }
 
 cudaError_t launch_mb_gather(const void *table, uint32_t n_records, uint32_t iters, unsigned blocks, float *sink, cudaStream_t stream) {

@@ -167,6 +167,10 @@ cudaError_t launch_pool(const KParams &p, KernelChoice c, unsigned blocks, unsig
 cudaError_t launch_trace(const KParams &p, KernelChoice c, unsigned blocks, size_t smem_bytes, cudaStream_t stream);
 cudaError_t launch_tail(const KParams &p, KernelChoice c, unsigned blocks, size_t smem_bytes, cudaStream_t stream);
 constexpr int kTailBlock = 256;
+// mm_trace_rays: probe_rays_kernel over n rays (ytab: the y-table traversal; device buffers as in the header's prototype)
+constexpr uint32_t kProbeBlock = 64;
+cudaError_t launch_probe(const KParams &p, bool ytab, const float *rays, const uint32_t *slots, uint32_t n, float *t_out, uint32_t *index_out,
+                         uint32_t *tally_out, cudaStream_t stream);
 cudaError_t launch_mb_gather(const void *table, uint32_t n_records, uint32_t iters, unsigned blocks, float *sink, cudaStream_t stream);
 cudaError_t launch_mb_ffma(uint32_t iters, unsigned blocks, float *sink, cudaStream_t stream);
 cudaError_t launch_scatter_all(const float *gathered, float *image, const mm_chunk *chunks, uint32_t world, uint32_t max_count,

@@ -237,6 +237,22 @@ class Renderer:
         self._ck(self._lib.mm_selftest_div3(self._ctx, C.byref(bad)))
         return int(bad.value)
 
+    def trace_rays(self, rays, slots=None, flags=0):
+        """mm_trace_rays: one traversal per ray of the uploaded scene, 32 rays to a warp in the order given.  rays [n, 8] float32
+        (ori.xyz, dir.xyz, t, alive), slots [n] starting leaf-order slots or None.  Returns a dict of numpy arrays: t, index
+        (plane index of the hit), inner, leaf, rect, max_stack, lit and form (the traversal the ray's warp ran, bits
+        1 mixed literal, 2 reciprocal-multiply, 4 axis-aligned rects, 8 y-table)."""
+        rays = np.ascontiguousarray(rays, dtype=np.float32).reshape(-1, 8)
+        n = len(rays)
+        sl = None if slots is None else np.ascontiguousarray(slots, dtype=np.uint32)
+        t, index, tally = np.empty(n, np.float32), np.empty(n, np.uint32), np.empty((n, 6), np.uint32)
+        self._ck(self._lib.mm_trace_rays(self._ctx, flags, rays.ctypes.data, None if sl is None else sl.ctypes.data, n,
+                                         t.ctypes.data, index.ctypes.data, tally.ctypes.data))
+        out = {"t": t, "index": index}
+        for i, k in enumerate(("inner", "leaf", "rect", "max_stack", "lit", "form")):
+            out[k] = tally[:, i]
+        return out
+
     def last_ms(self):
         ms = C.c_float()
         self._ck(self._lib.mm_last_ms(self._ctx, C.byref(ms)))

@@ -449,6 +449,37 @@ uint64_t mmo_trace(const mm_plane *planes, uint32_t n_planes, const mm_bvh_node 
     return tr.size();
 }
 
+// intersect_bvh_iterative ray by ray, the reference for mm_trace_rays: rays n x 8 floats (ori.xyz, dir.xyz, starting t, alive),
+// index_in the starting beam.index (plane index; null: 0xFFFFFFFF), flags & MM_FLAG_RCP_SLAB selects the reciprocal-multiply
+// slab test.  Per ray: t, index and counts n x 5 (inner, leaf, rect, max_stack, stack overflow).  A dead ray (alive == 0)
+// keeps its t and index and counts nothing.  Returns MM_ERR_BVH when some ray overflowed the reference's 50-entry stack.
+int mmo_trace_rays(const mm_plane *planes, uint32_t n_planes, const mm_bvh_node *nodes, uint32_t n_nodes, const uint32_t *indices,
+                   uint32_t flags, const float *rays, const uint32_t *index_in, uint32_t n, float *t_out, uint32_t *index_out,
+                   uint64_t *counts_out, int n_threads) {
+    if (!planes || !nodes || !indices || !rays || !t_out || !index_out || !counts_out || n_planes == 0 || n_nodes == 0) return MM_ERR_INVALID;
+    const Scene sc = {planes, n_planes, nodes, n_nodes, indices, nullptr, nullptr};
+    int overflow = 0;
+#ifdef _OPENMP
+    if (n_threads > 0) omp_set_num_threads(n_threads);
+#endif
+#pragma omp parallel for schedule(dynamic, 256) reduction(| : overflow)
+    for (int64_t i = 0; i < (int64_t)n; i++) {
+        const float *r = rays + 8 * i;
+        Ray beam;
+        beam.ori = mk(r[0], r[1], r[2]); beam.dir = mk(r[3], r[4], r[5]); beam.t = r[6];
+        beam.index = index_in ? index_in[i] : 0xFFFFFFFFu;
+        Counts c;
+        c.rcp = (flags & MM_FLAG_RCP_SLAB) != 0;
+        if (r[7] != 0.0f) intersect_bvh_iterative(beam, sc, c);
+        t_out[i] = beam.t;
+        index_out[i] = beam.index;
+        uint64_t *o = counts_out + 5 * i;
+        o[0] = c.inner; o[1] = c.leaf; o[2] = c.rect; o[3] = c.max_stack; o[4] = c.overflow ? 1u : 0u;
+        overflow |= c.overflow ? 1 : 0;
+    }
+    return overflow ? MM_ERR_BVH : MM_OK;
+}
+
 // Unit-level entry points for known-answer tests.
 float mmo_random(uint32_t *state) { return random_f(*state); }
 uint32_t mmo_random_word(uint32_t *state) {   // the u32 `result` before the float conversion

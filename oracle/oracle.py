@@ -49,6 +49,9 @@ def lib():
         _lib.mmo_quat_mult.restype = None
         _lib.mmo_quat_mult.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
         _lib.mmo_num_threads.restype = C.c_int
+        _lib.mmo_trace_rays.restype = C.c_int
+        _lib.mmo_trace_rays.argtypes = [C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint32, C.c_void_p,
+                                        C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
     return _lib
 
 
@@ -105,6 +108,27 @@ def render(scene, noise, uniform, params, chunks, debug=False, threads=0, out=No
     if rc != 0:
         raise RuntimeError(f"mmo_render failed: {rc}")
     return out, {n: int(getattr(cnt, n)) for n, _ in cnt._fields_}, dbg
+
+
+def trace_rays(scene, rays, index=None, flags=0, threads=0):
+    """intersect_bvh_iterative per ray (mmo_trace_rays): rays [n, 8] float32 (ori.xyz, dir.xyz, t, alive), index [n] starting
+    plane indices or None.  Returns a dict of numpy arrays: t, index, inner, leaf, rect, max_stack, overflow."""
+    planes = np.ascontiguousarray(scene.planes)
+    nodes = np.ascontiguousarray(scene.nodes)
+    indices = np.ascontiguousarray(scene.indices, dtype=np.uint32)
+    rays = np.ascontiguousarray(rays, dtype=np.float32).reshape(-1, 8)
+    n = len(rays)
+    idx = None if index is None else np.ascontiguousarray(index, dtype=np.uint32)
+    t, out_idx, counts = np.empty(n, np.float32), np.empty(n, np.uint32), np.empty((n, 5), np.uint64)
+    rc = lib().mmo_trace_rays(planes.ctypes.data, len(planes), nodes.ctypes.data, len(nodes), indices.ctypes.data, flags,
+                              rays.ctypes.data, None if idx is None else idx.ctypes.data, n, t.ctypes.data, out_idx.ctypes.data,
+                              counts.ctypes.data, threads)
+    if rc not in (0, -4):
+        raise RuntimeError(f"mmo_trace_rays failed: {rc}")
+    out = {"t": t, "index": out_idx}
+    for i, k in enumerate(("inner", "leaf", "rect", "max_stack", "overflow")):
+        out[k] = counts[:, i]
+    return out
 
 
 def random_words(seed, n):
