@@ -201,6 +201,35 @@ int mm_render_async(mm_ctx *ctx, const mm_uniform *uni, const mm_params *params,
                     const mm_chunk *chunks, uint32_t n_chunks, float *out_rgba, const mm_debug *debug);
 int mm_wait(mm_ctx *ctx, mm_counters *counters);
 /*
+ * Several camera views of one scene in one launch (split screen, stereo pairs, cube-map probes, several fly-throughs on one
+ * GPU).  unis[n_views], 1 <= n_views <= MM_MAX_VIEWS: every view has its own camera and time; all share params (spp, limits,
+ * grid, flags, group range) and must have the same view_width / view_height / chunk_width (else MM_ERR_INVALID).
+ * chunks: n_views x (grid_x*grid_y) entries, view v's list at v*grid_x*grid_y; n_chunks must equal that count.  Every view
+ * renders exactly what mm_render gives for it alone, into its own persistent view screen owned by the context: created
+ * zero-filled at first use and again when n_views or the view size changes, kept across calls, separate from mm_render's
+ * screen (neither call touches the other's).  out_rgba: NULL, or n_views pointers, each NULL or a host frame of
+ * H*W*4 floats filled with mm_render's rules (mapped pinned memory: zero-copy stores by the kernel, unless
+ * MM_FLAG_NO_ZERO_COPY; otherwise a copy of the view's whole screen).  debug: per-path arrays of
+ * n_views*group_count*chunk_width^2*spp entries, view-major.  counters, mm_last_counters, mm_last_ms and mm_last_tail report
+ * the whole launch: sums over the views (max_stack: the maximum).  Flags as mm_render; MM_FLAG_POOL_KERNEL and
+ * MM_FLAG_REGROUP return MM_ERR_UNSUPPORTED.  mm_render_views_async returns once the launch is enqueued and is completed
+ * by mm_wait, as mm_render_async; mm_render_views == mm_render_views_async + mm_wait.
+ */
+#define MM_MAX_VIEWS 64
+int mm_render_views_async(mm_ctx *ctx, const mm_uniform *unis, uint32_t n_views, const mm_params *params,
+                          const mm_chunk *chunks, uint32_t n_chunks, float *const *out_rgba, const mm_debug *debug);
+int mm_render_views(mm_ctx *ctx, const mm_uniform *unis, uint32_t n_views, const mm_params *params,
+                    const mm_chunk *chunks, uint32_t n_chunks, float *const *out_rgba, mm_counters *counters,
+                    const mm_debug *debug);
+/*
+ * The present pass on all view screens in one launch, asynchronous like mm_present_async / mm_present_async_rgba8 and
+ * completed by mm_wait_present.  rgba8 = 0: the fp32 blur; out[v] receives view v's blurred screen (H*W*4 floats).
+ * rgba8 = 1: the quantising blur of MM_FLAG_SCREEN_RGBA8 screens; out[v] receives view v's texels (H*W*4 bytes).  out: NULL
+ * (blur only) or one pointer per view, each NULL or pinned host memory (mm_host_alloc / mm_host_register).  MM_ERR_INVALID
+ * before any mm_render_views.
+ */
+int mm_present_views(mm_ctx *ctx, uint32_t rgba8, void *const *out);
+/*
  * Pinned, device-mapped host memory for frames (the counterpart of the reference's StorageModeManaged buffers,
  * utils.rs:86-94): mm_host_alloc allocates it, mm_host_register pins and maps memory the caller already owns (a
  * Vec<f32>'s buffer; it must stay allocated until mm_host_unregister).  Process-wide, usable with every context and

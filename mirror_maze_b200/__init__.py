@@ -8,7 +8,7 @@ the CUDA library or a B200 is missing.
 """
 from .abi import (MMError, load_library, library_path, Float2, Float3, Float4, Plane, BVHNode, Camera, Uniform, Chunk,
                   Params, Counters, SceneInfo, FLAG_COUNTERS, FLAG_FORCE_LITERAL, FLAG_RCP_SLAB, FLAG_NO_ZERO_COPY, FLAG_POOL_KERNEL, FLAG_SCREEN_RGBA8, FLAG_REGROUP, FLAG_GENERAL_RECTS, FLAG_NO_TAIL, FLAG_NO_Y_TABLE, MAX_STACK, MAX_BVH_DEPTH,
-                  EXCHANGE_PEER, EXCHANGE_NCCL, EXCHANGE_NONE)
+                  EXCHANGE_PEER, EXCHANGE_NCCL, EXCHANGE_NONE, MAX_VIEWS)
 from .host import (MazeScene, StdRng, default_uniform, gen_chunks, calculate_quaternion, update_quat_angle, quat_mult,
                    load_noise, full_frame_params, check_collision, chacha_block, ChunkBag, move_camera, rect_edge_thresholds, axis_rect)
 from .renderer import Renderer, MultiRenderer, HostFrame, TiledFrameRenderer, tile_partition

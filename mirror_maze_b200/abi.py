@@ -23,6 +23,7 @@ FLAG_NO_TAIL = 4096
 FLAG_NO_Y_TABLE = 8192
 EXCHANGE_PEER, EXCHANGE_NCCL, EXCHANGE_NONE = 0, 1, 2
 MAX_PEERS = 8
+MAX_VIEWS = 64
 
 ERR_NAMES = {0: "MM_OK", -1: "MM_ERR_INVALID", -2: "MM_ERR_CUDA", -3: "MM_ERR_NO_SCENE", -4: "MM_ERR_BVH",
              -5: "MM_ERR_UNSUPPORTED", -6: "MM_ERR_NOMEM"}
@@ -113,6 +114,9 @@ PROTOTYPES = {
     "mm_render": (C.c_int, [_vp, _P(Uniform), _P(Params), _vp, C.c_uint32, _vp, _P(Counters), _P(Debug)]),
     "mm_render_async": (C.c_int, [_vp, _P(Uniform), _P(Params), _vp, C.c_uint32, _vp, _P(Debug)]),
     "mm_wait": (C.c_int, [_vp, _P(Counters)]),
+    "mm_render_views_async": (C.c_int, [_vp, _P(Uniform), C.c_uint32, _P(Params), _vp, C.c_uint32, _P(_vp), _P(Debug)]),
+    "mm_render_views": (C.c_int, [_vp, _P(Uniform), C.c_uint32, _P(Params), _vp, C.c_uint32, _P(_vp), _P(Counters), _P(Debug)]),
+    "mm_present_views": (C.c_int, [_vp, C.c_uint32, _P(_vp)]),
     "mm_host_alloc": (C.c_int, [C.c_size_t, _P(_vp)]),
     "mm_host_free": (C.c_int, [_vp]),
     "mm_host_register": (C.c_int, [_vp, C.c_size_t]),

@@ -108,6 +108,8 @@ int mm_destroy(mm_ctx *ctx) {
     if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
     cudaFree(ctx->d_screen8);
     cudaFree(ctx->d_snap);
+    cudaFree(ctx->d_view_chunks); cudaFree(ctx->d_views);
+    cudaFree(ctx->d_vscreen); cudaFree(ctx->d_vscreen2); cudaFree(ctx->d_vsnap); cudaFree(ctx->d_vscreen8);
     if (ctx->copy_stream) { cudaStreamSynchronize(ctx->copy_stream); cudaStreamDestroy(ctx->copy_stream); }
     if (ctx->ev_snap) cudaEventDestroy(ctx->ev_snap);
     if (ctx->ev_copy) cudaEventDestroy(ctx->ev_copy);
@@ -282,7 +284,7 @@ bool traversal_params(const mm_ctx *ctx, uint32_t flags, KParams &p) {
     return ytab;
 }
 
-int build_launch(mm_ctx *ctx, const mm_uniform *uni, const mm_params *par, bool debug, Launch &L) {
+int build_launch(mm_ctx *ctx, const mm_uniform *uni, const mm_params *par, bool debug, Launch &L, uint32_t n_views) {
     if (!uni || !par) return fail(ctx, MM_ERR_INVALID, "null uniform or params");
     if (!ctx->have_scene) return fail(ctx, MM_ERR_NO_SCENE, "no scene uploaded");
     const uint32_t spp = par->spp, chunk = uni->chunk_width;
@@ -293,7 +295,7 @@ int build_launch(mm_ctx *ctx, const mm_uniform *uni, const mm_params *par, bool 
     if (T > 32 && (T % 32) != 0) return fail(ctx, MM_ERR_UNSUPPORTED, "chunk_width^2 * spp must be <= 32 or a multiple of 32 (virtual threadgroup = 32 x T/32)");
     if (par->grid_x == 0 || par->grid_y == 0) return fail(ctx, MM_ERR_INVALID, "empty grid");
     const uint64_t n_groups = (uint64_t)par->grid_x * par->grid_y;
-    if (n_groups != ctx->n_chunks) return fail(ctx, MM_ERR_INVALID, "grid_x*grid_y must equal the chunk count");
+    if (!n_views && n_groups != ctx->n_chunks) return fail(ctx, MM_ERR_INVALID, "grid_x*grid_y must equal the chunk count");
     if (par->bounce_limit > 4096 || par->mirror_limit > 4096) return fail(ctx, MM_ERR_INVALID, "bounce/mirror limit too large");
     if (!(uni->view_width >= 1.0f) || !(uni->view_height >= 1.0f) || uni->view_width > 65536.0f || uni->view_height > 65536.0f)
         return fail(ctx, MM_ERR_INVALID, "bad view size");
@@ -318,8 +320,8 @@ int build_launch(mm_ctx *ctx, const mm_uniform *uni, const mm_params *par, bool 
     p.noise_w = ctx->noise_w; p.noise_h = ctx->noise_h;
     const bool ytab = traversal_params(ctx, par->flags, p);
     p.quant8 = (par->flags & MM_FLAG_SCREEN_RGBA8) ? 1u : 0u;
-    p.total_paths = (uint64_t)count * T;
-    p.chunks = ctx->d_chunks; p.noise = ctx->d_noise;
+    p.total_paths = (uint64_t)count * T * (n_views ? n_views : 1);
+    p.chunks = n_views ? ctx->d_view_chunks : ctx->d_chunks; p.noise = ctx->d_noise;
     p.counters = ctx->d_counters;
 
     L.choice.debug = debug;
@@ -327,10 +329,13 @@ int build_launch(mm_ctx *ctx, const mm_uniform *uni, const mm_params *par, bool 
     L.choice.pool = false;
     L.choice.regroup = false;
     L.choice.ytab = false;
-    if (configure_pool(ctx, par, L)) return MM_OK;
+    L.choice.views = n_views != 0;
+    L.views = n_views ? ctx->d_views : nullptr;
+    // the multi-view kernels exist for the default kernel only (mm_render_views refuses the flags of the other two)
+    if (!n_views && configure_pool(ctx, par, L)) return MM_OK;
     // opt-in (MM_FLAG_REGROUP, or MM_KERNEL=regroup for tuning runs): the kernel that re-forms the block's warps at segment boundaries
     const char *env_kernel = getenv("MM_KERNEL");
-    L.choice.regroup = (par->flags & MM_FLAG_REGROUP) || (env_kernel && !strcmp(env_kernel, "regroup"));
+    L.choice.regroup = !n_views && ((par->flags & MM_FLAG_REGROUP) || (env_kernel && !strcmp(env_kernel, "regroup")));
     int bt = block_threads_for(p.spp);
     if (L.choice.regroup) {
         const int want = (int)env_u32("MM_RG_BLOCK", kLargeBlock, 64, kLargeBlock);       // developer override: 64 / 128 / 256
@@ -399,11 +404,11 @@ int do_launch(mm_ctx *ctx, Launch &L) {
         if (blocks > want) blocks = want ? want : 1;                                 // tiny dispatches: no more warps than units
         CK(launch_pool(L.p, L.choice, (unsigned)blocks, (unsigned)L.choice.block_threads, L.smem, ctx->stream));
     } else {
-        CK(launch_trace(L.p, L.choice, L.blocks, L.smem, ctx->stream));
+        CK(launch_trace(L.p, L.choice, L.blocks, L.smem, ctx->stream, L.views));
         if (L.p.tail_k) {                 // one thread per queued path; the grid strides over whatever the queue holds
             const uint64_t want = ((uint64_t)L.p.tail_cap + kTailBlock - 1) / kTailBlock, full = (uint64_t)ctx->n_sms * (1024 / kTailBlock);
             const size_t tail_smem = L.choice.ytab ? (size_t)(kTailBlock / 32) * L.p.n_yiv * kYEntryStride : 0;
-            CK(launch_tail(L.p, L.choice, (unsigned)(want < full ? want : full), tail_smem, ctx->stream));
+            CK(launch_tail(L.p, L.choice, (unsigned)(want < full ? want : full), tail_smem, ctx->stream, L.views));
         }
     }
     CK(cudaEventRecord(ctx->ev1, ctx->stream));
@@ -425,6 +430,52 @@ int ensure_screen(mm_ctx *ctx, uint32_t W, uint32_t H) {
     CK(cudaMalloc(&ctx->d_screen, (size_t)W * H * 4 * sizeof(float)));
     CK(cudaMemsetAsync(ctx->d_screen, 0, (size_t)W * H * 4 * sizeof(float), ctx->stream));
     ctx->screen_w = W; ctx->screen_h = H;
+    return MM_OK;
+}
+
+// Device per-path debug arrays for n_paths paths, and the kernel's pointers to those the caller asked for.
+static int setup_debug(mm_ctx *ctx, const mm_debug *debug, size_t n_paths, KParams &p) {
+    if (n_paths > ctx->dbg_cap) {
+        CK(cudaStreamSynchronize(ctx->stream));
+        for (auto &q : ctx->d_dbg_u32) { cudaFree(q); q = nullptr; }
+        cudaFree(ctx->d_dbg_rad); ctx->d_dbg_rad = nullptr; ctx->dbg_cap = 0;
+        for (auto &q : ctx->d_dbg_u32) CK(cudaMalloc(&q, n_paths * sizeof(uint32_t)));
+        CK(cudaMalloc(&ctx->d_dbg_rad, n_paths * 3 * sizeof(float)));
+        ctx->dbg_cap = n_paths;
+    }
+    p.dbg_first_hit = debug->first_hit ? ctx->d_dbg_u32[0] : nullptr;
+    p.dbg_segments = debug->segments ? ctx->d_dbg_u32[1] : nullptr;
+    p.dbg_mirror_hits = debug->mirror_hits ? ctx->d_dbg_u32[2] : nullptr;
+    p.dbg_radiance = debug->radiance ? ctx->d_dbg_rad : nullptr;
+    return MM_OK;
+}
+
+// The read-back of the debug arrays into the caller's host arrays, on the context's stream.
+static int copy_debug(mm_ctx *ctx, const mm_debug *debug, size_t n_paths) {
+    if (debug->first_hit) CK(cudaMemcpyAsync(debug->first_hit, ctx->d_dbg_u32[0], n_paths * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    if (debug->segments) CK(cudaMemcpyAsync(debug->segments, ctx->d_dbg_u32[1], n_paths * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    if (debug->mirror_hits) CK(cudaMemcpyAsync(debug->mirror_hits, ctx->d_dbg_u32[2], n_paths * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    if (debug->radiance) CK(cudaMemcpyAsync(debug->radiance, ctx->d_dbg_rad, n_paths * 12, cudaMemcpyDeviceToHost, ctx->stream));
+    return MM_OK;
+}
+
+// The pinned staging buffer for callers whose frame memory is not known to be pinned, at least `bytes` long.
+static int ensure_stage(mm_ctx *ctx, size_t bytes) {
+    if (ctx->stage_bytes >= bytes) return MM_OK;
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
+    ctx->h_stage = nullptr; ctx->stage_bytes = 0;
+    CK(cudaMallocHost(&ctx->h_stage, bytes));
+    ctx->stage_bytes = bytes;
+    return MM_OK;
+}
+
+// The second stream and its events of the asynchronous present, created at first use.
+static int ensure_copy_stream(mm_ctx *ctx) {
+    if (ctx->copy_stream) return MM_OK;
+    CK(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
+    CK(cudaEventCreateWithFlags(&ctx->ev_snap, cudaEventDisableTiming));
+    CK(cudaEventCreateWithFlags(&ctx->ev_copy, cudaEventDisableTiming));
     return MM_OK;
 }
 
@@ -537,6 +588,11 @@ int mm_wait(mm_ctx *ctx, mm_counters *counters) {
         memcpy(ctx->pending_out, ctx->h_stage, ctx->pending_bytes);
         ctx->pending_out = nullptr;
     }
+    for (uint32_t v = 0; v < MM_MAX_VIEWS; v++) {          // staged views of mm_render_views_async
+        if (!ctx->pending_views[v]) continue;
+        memcpy(ctx->pending_views[v], reinterpret_cast<const char *>(ctx->h_stage) + v * ctx->pending_bytes, ctx->pending_bytes);
+        ctx->pending_views[v] = nullptr;
+    }
     ctx->in_flight = false;
     if (counters) {
         if (!ctx->timed) return fail(ctx, MM_ERR_INVALID, "mm_wait: nothing rendered yet");
@@ -572,28 +628,9 @@ int mm_render_async(mm_ctx *ctx, const mm_uniform *uni, const mm_params *params,
     L.p.host_out = static_cast<float *>(alias);
     ctx->last_zero_copy = alias ? 1u : 0u;
     const size_t n_paths = (size_t)L.p.total_paths;
-    if (dbg) {
-        if (n_paths > ctx->dbg_cap) {
-            CK(cudaStreamSynchronize(ctx->stream));
-            for (auto &p : ctx->d_dbg_u32) { cudaFree(p); p = nullptr; }
-            cudaFree(ctx->d_dbg_rad); ctx->d_dbg_rad = nullptr; ctx->dbg_cap = 0;
-            for (auto &p : ctx->d_dbg_u32) CK(cudaMalloc(&p, n_paths * sizeof(uint32_t)));
-            CK(cudaMalloc(&ctx->d_dbg_rad, n_paths * 3 * sizeof(float)));
-            ctx->dbg_cap = n_paths;
-        }
-        L.p.dbg_first_hit = debug->first_hit ? ctx->d_dbg_u32[0] : nullptr;
-        L.p.dbg_segments = debug->segments ? ctx->d_dbg_u32[1] : nullptr;
-        L.p.dbg_mirror_hits = debug->mirror_hits ? ctx->d_dbg_u32[2] : nullptr;
-        L.p.dbg_radiance = debug->radiance ? ctx->d_dbg_rad : nullptr;
-    }
+    if (dbg && (rc = setup_debug(ctx, debug, n_paths, L.p)) != MM_OK) return rc;
     const bool staged = out_rgba && !pinned;
-    if (staged && ctx->stage_bytes < frame_bytes) {
-        CK(cudaStreamSynchronize(ctx->stream));
-        if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
-        ctx->h_stage = nullptr; ctx->stage_bytes = 0;
-        CK(cudaMallocHost(&ctx->h_stage, frame_bytes));
-        ctx->stage_bytes = frame_bytes;
-    }
+    if (staged && (rc = ensure_stage(ctx, frame_bytes)) != MM_OK) return rc;
     rc = do_launch(ctx, L);
     if (rc != MM_OK) return rc;
     ctx->in_flight = true;
@@ -604,12 +641,7 @@ int mm_render_async(mm_ctx *ctx, const mm_uniform *uni, const mm_params *params,
         CK(cudaMemcpyAsync(dst, ctx->d_screen, frame_bytes, cudaMemcpyDeviceToHost, ctx->stream));
         if (staged) { ctx->pending_out = out_rgba; ctx->pending_bytes = frame_bytes; }
     }
-    if (dbg) {
-        if (debug->first_hit) CK(cudaMemcpyAsync(debug->first_hit, ctx->d_dbg_u32[0], n_paths * 4, cudaMemcpyDeviceToHost, ctx->stream));
-        if (debug->segments) CK(cudaMemcpyAsync(debug->segments, ctx->d_dbg_u32[1], n_paths * 4, cudaMemcpyDeviceToHost, ctx->stream));
-        if (debug->mirror_hits) CK(cudaMemcpyAsync(debug->mirror_hits, ctx->d_dbg_u32[2], n_paths * 4, cudaMemcpyDeviceToHost, ctx->stream));
-        if (debug->radiance) CK(cudaMemcpyAsync(debug->radiance, ctx->d_dbg_rad, n_paths * 12, cudaMemcpyDeviceToHost, ctx->stream));
-    }
+    if (dbg) return copy_debug(ctx, debug, n_paths);
     return MM_OK;
 }
 
@@ -618,6 +650,147 @@ int mm_render(mm_ctx *ctx, const mm_uniform *uni, const mm_params *params, const
     int rc = mm_render_async(ctx, uni, params, chunks, n_chunks, out_rgba, debug);
     if (rc != MM_OK) return rc;
     return mm_wait(ctx, counters);
+}
+
+/* ---- several views in one launch -------------------------------------------------------------------------------------- */
+
+namespace mmapi {
+// The persistent view screens: n screens of W x H, zero-filled whenever n or the size changes.
+static int ensure_view_screens(mm_ctx *ctx, uint32_t n, uint32_t W, uint32_t H) {
+    if (ctx->d_vscreen && ctx->vscreen_n == n && ctx->vscreen_w == W && ctx->vscreen_h == H) return MM_OK;
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (ctx->copy_stream) CK(cudaStreamSynchronize(ctx->copy_stream));
+    cudaFree(ctx->d_vscreen); cudaFree(ctx->d_vscreen2); cudaFree(ctx->d_vsnap); cudaFree(ctx->d_vscreen8);
+    ctx->d_vscreen = nullptr; ctx->d_vscreen2 = nullptr; ctx->d_vsnap = nullptr; ctx->d_vscreen8 = nullptr;
+    ctx->vscreen_n = 0;
+    const size_t bytes = (size_t)n * W * H * 4 * sizeof(float);
+    CK(cudaMalloc(&ctx->d_vscreen, bytes));
+    CK(cudaMemsetAsync(ctx->d_vscreen, 0, bytes, ctx->stream));
+    ctx->vscreen_n = n; ctx->vscreen_w = W; ctx->vscreen_h = H;
+    return MM_OK;
+}
+}  // namespace mmapi
+
+int mm_render_views_async(mm_ctx *ctx, const mm_uniform *unis, uint32_t n_views, const mm_params *params, const mm_chunk *chunks,
+                          uint32_t n_chunks, float *const *out_rgba, const mm_debug *debug) {
+    if (!ctx) return MM_ERR_INVALID;
+    ctx->err.clear();
+    if (!unis || !params || !chunks) return fail(ctx, MM_ERR_INVALID, "mm_render_views: null uniforms, params or chunk list");
+    if (n_views == 0 || n_views > MM_MAX_VIEWS) return fail(ctx, MM_ERR_INVALID, "mm_render_views: n_views must be in 1..MM_MAX_VIEWS");
+    if (params->flags & (MM_FLAG_POOL_KERNEL | MM_FLAG_REGROUP))
+        return fail(ctx, MM_ERR_UNSUPPORTED, "mm_render_views: MM_FLAG_POOL_KERNEL and MM_FLAG_REGROUP have no multi-view kernel");
+    for (uint32_t v = 1; v < n_views; v++)
+        if (unis[v].view_width != unis[0].view_width || unis[v].view_height != unis[0].view_height || unis[v].chunk_width != unis[0].chunk_width)
+            return fail(ctx, MM_ERR_INVALID, "mm_render_views: every view must have the same view size and chunk width");
+    const uint64_t n_groups = (uint64_t)params->grid_x * params->grid_y;
+    if (n_groups == 0 || (uint64_t)n_chunks != n_groups * n_views)
+        return fail(ctx, MM_ERR_INVALID, "mm_render_views: n_chunks must equal n_views*grid_x*grid_y");
+    int rc;
+    CK(cudaSetDevice(ctx->device));
+    if (ctx->in_flight && (rc = mm_wait(ctx, nullptr)) != MM_OK) return rc;     // one host-buffer frame in flight per context
+    if (!ctx->d_views) CK(cudaMalloc(&ctx->d_views, MM_MAX_VIEWS * sizeof(ViewRec)));
+    if (n_chunks > ctx->view_chunks_cap) {
+        CK(cudaStreamSynchronize(ctx->stream));
+        cudaFree(ctx->d_view_chunks);
+        ctx->d_view_chunks = nullptr; ctx->view_chunks_cap = 0;
+        CK(cudaMalloc(&ctx->d_view_chunks, (size_t)n_chunks * sizeof(mm_chunk)));
+        ctx->view_chunks_cap = n_chunks;
+    }
+    const bool dbg = debug && (debug->first_hit || debug->segments || debug->mirror_hits || debug->radiance);
+    Launch L;
+    rc = build_launch(ctx, unis, params, dbg, L, n_views);
+    if (rc != MM_OK) return rc;
+    const uint32_t W = L.p.W, H = L.p.H;
+    rc = ensure_view_screens(ctx, n_views, W, H);
+    if (rc != MM_OK) return rc;
+    const size_t frame_floats = (size_t)W * H * 4, frame_bytes = frame_floats * sizeof(float);
+    // Per view: zero-copy into a mapped pinned host frame (the kernel stores the view's pixels), a DMA copy of the view's
+    // screen into other pinned memory, or one through the pinned staging buffer for pageable memory (as mm_render_async).
+    ViewRec rec[MM_MAX_VIEWS];
+    bool copy[MM_MAX_VIEWS] = {}, staged[MM_MAX_VIEWS] = {}, any_staged = false;
+    uint32_t zero_copy = 0;
+    for (uint32_t v = 0; v < n_views; v++) {
+        float *out = out_rgba ? out_rgba[v] : nullptr;
+        void *pinned = out ? host_device_alias(out, frame_bytes) : nullptr;
+        void *alias = (params->flags & MM_FLAG_NO_ZERO_COPY) ? nullptr : pinned;
+        memset(&rec[v], 0, sizeof(ViewRec));
+        rec[v].uni = unis[v];
+        rec[v].chunk_off = (uint32_t)(v * n_groups);
+        rec[v].screen = ctx->d_vscreen + v * frame_floats;
+        rec[v].host_out = static_cast<float *>(alias);
+        copy[v] = out && !alias;
+        staged[v] = out && !pinned;
+        any_staged = any_staged || staged[v];
+        zero_copy |= alias ? 1u : 0u;
+    }
+    const size_t n_paths = (size_t)L.p.total_paths;
+    if (dbg && (rc = setup_debug(ctx, debug, n_paths, L.p)) != MM_OK) return rc;
+    if (any_staged && (rc = ensure_stage(ctx, n_views * frame_bytes)) != MM_OK) return rc;
+    CK(cudaMemcpyAsync(ctx->d_view_chunks, chunks, (size_t)n_chunks * sizeof(mm_chunk), cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(ctx->d_views, rec, n_views * sizeof(ViewRec), cudaMemcpyHostToDevice, ctx->stream));
+    ctx->last_zero_copy = zero_copy;
+    rc = do_launch(ctx, L);
+    if (rc != MM_OK) return rc;
+    ctx->in_flight = true;
+    for (uint32_t v = 0; v < n_views; v++) {
+        if (!copy[v]) continue;
+        float *dst = staged[v] ? ctx->h_stage + v * frame_floats : out_rgba[v];
+        CK(cudaMemcpyAsync(dst, rec[v].screen, frame_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+        if (staged[v]) { ctx->pending_views[v] = out_rgba[v]; ctx->pending_bytes = frame_bytes; }
+    }
+    if (dbg) return copy_debug(ctx, debug, n_paths);
+    return MM_OK;
+}
+
+int mm_render_views(mm_ctx *ctx, const mm_uniform *unis, uint32_t n_views, const mm_params *params, const mm_chunk *chunks,
+                    uint32_t n_chunks, float *const *out_rgba, mm_counters *counters, const mm_debug *debug) {
+    int rc = mm_render_views_async(ctx, unis, n_views, params, chunks, n_chunks, out_rgba, debug);
+    if (rc != MM_OK) return rc;
+    return mm_wait(ctx, counters);
+}
+
+int mm_present_views(mm_ctx *ctx, uint32_t rgba8, void *const *out) {
+    if (!ctx) return MM_ERR_INVALID;
+    ctx->err.clear();
+    if (!ctx->d_vscreen) return fail(ctx, MM_ERR_INVALID, "mm_present_views: no views rendered yet");
+    if (rgba8 > 1) return fail(ctx, MM_ERR_INVALID, "mm_present_views: rgba8 must be 0 or 1");
+    const uint32_t n = ctx->vscreen_n;
+    const size_t n_px = (size_t)ctx->vscreen_w * ctx->vscreen_h, screen_bytes = n_px * 4 * sizeof(float);
+    const size_t out_bytes = rgba8 ? n_px * 4 : screen_bytes;
+    bool any_out = false;
+    for (uint32_t v = 0; out && v < n; v++) {
+        if (!out[v]) continue;
+        if (!host_device_alias(out[v], out_bytes))
+            return fail(ctx, MM_ERR_INVALID, "mm_present_views: out[v] must be pinned host memory (mm_host_alloc / mm_host_register)");
+        any_out = true;
+    }
+    CK(cudaSetDevice(ctx->device));
+    int rc = ensure_copy_stream(ctx);
+    if (rc != MM_OK) return rc;
+    if (!ctx->d_vscreen2) CK(cudaMalloc(&ctx->d_vscreen2, n * screen_bytes));
+    if (rgba8 && !ctx->d_vscreen8) CK(cudaMalloc(&ctx->d_vscreen8, n * n_px * 4));
+    if (!rgba8 && any_out && !ctx->d_vsnap) CK(cudaMalloc(&ctx->d_vsnap, n * screen_bytes));
+    if (rgba8 && ctx->present_in_flight) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_copy, 0));   // the previous texels have left the device
+    CK(launch_blur_views(ctx->d_vscreen, ctx->d_vscreen2, ctx->vscreen_w, ctx->vscreen_h, n, ctx->stream, rgba8 != 0,
+                         rgba8 ? ctx->d_vscreen8 : nullptr));
+    float *t = ctx->d_vscreen; ctx->d_vscreen = ctx->d_vscreen2; ctx->d_vscreen2 = t;   // the blurred images are the screens now
+    if (!any_out) return MM_OK;
+    if (!rgba8) {
+        // snapshot for the read-back: the next dispatch may write into the screens while the copies are still on the wire
+        if (ctx->present_in_flight) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_copy, 0));   // the previous snapshot has left the device
+        for (uint32_t v = 0; v < n; v++)
+            if (out[v]) CK(cudaMemcpyAsync(ctx->d_vsnap + v * n_px * 4, ctx->d_vscreen + v * n_px * 4, screen_bytes, cudaMemcpyDeviceToDevice, ctx->stream));
+    }
+    CK(cudaEventRecord(ctx->ev_snap, ctx->stream));
+    CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_snap, 0));
+    for (uint32_t v = 0; v < n; v++) {
+        if (!out[v]) continue;
+        const void *src = rgba8 ? static_cast<const void *>(ctx->d_vscreen8 + v * n_px * 4) : static_cast<const void *>(ctx->d_vsnap + v * n_px * 4);
+        CK(cudaMemcpyAsync(out[v], src, out_bytes, cudaMemcpyDeviceToHost, ctx->copy_stream));
+    }
+    CK(cudaEventRecord(ctx->ev_copy, ctx->copy_stream));
+    ctx->present_in_flight = true;
+    return MM_OK;
 }
 
 int mm_scatter_tiles_device(mm_ctx *ctx, const mm_uniform *uni, const mm_params *params, const float *d_tiles, float *d_image) {
@@ -713,11 +886,8 @@ int mm_present_async_rgba8(mm_ctx *ctx, uint8_t *out_rgba8) {
     if (!out_rgba8 || !host_device_alias(out_rgba8, n_px * 4))
         return fail(ctx, MM_ERR_INVALID, "mm_present_async_rgba8: out_rgba8 must be pinned host memory (mm_host_alloc / mm_host_register)");
     CK(cudaSetDevice(ctx->device));
-    if (!ctx->copy_stream) {
-        CK(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
-        CK(cudaEventCreateWithFlags(&ctx->ev_snap, cudaEventDisableTiming));
-        CK(cudaEventCreateWithFlags(&ctx->ev_copy, cudaEventDisableTiming));
-    }
+    int rc = ensure_copy_stream(ctx);
+    if (rc != MM_OK) return rc;
     if (!ctx->d_screen2) CK(cudaMalloc(&ctx->d_screen2, bytes));
     if (!ctx->d_screen8) CK(cudaMalloc(&ctx->d_screen8, n_px * 4));
     if (ctx->present_in_flight) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_copy, 0));       // the previous texels have left the device
@@ -739,11 +909,8 @@ int mm_present_async(mm_ctx *ctx, float *out_rgba) {
     if (!out_rgba || !host_device_alias(out_rgba, bytes))
         return fail(ctx, MM_ERR_INVALID, "mm_present_async: out_rgba must be pinned host memory (mm_host_alloc / mm_host_register); use mm_present otherwise");
     CK(cudaSetDevice(ctx->device));
-    if (!ctx->copy_stream) {
-        CK(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
-        CK(cudaEventCreateWithFlags(&ctx->ev_snap, cudaEventDisableTiming));
-        CK(cudaEventCreateWithFlags(&ctx->ev_copy, cudaEventDisableTiming));
-    }
+    int rc = ensure_copy_stream(ctx);
+    if (rc != MM_OK) return rc;
     if (!ctx->d_screen2) CK(cudaMalloc(&ctx->d_screen2, bytes));
     if (!ctx->d_snap) CK(cudaMalloc(&ctx->d_snap, bytes));
     CK(launch_blur(ctx->d_screen, ctx->d_screen2, ctx->screen_w, ctx->screen_h, ctx->stream));

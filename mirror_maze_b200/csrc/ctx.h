@@ -51,6 +51,16 @@ struct mm_ctx {
     cudaEvent_t ev_snap = nullptr, ev_copy = nullptr;
     float *d_snap = nullptr;
     bool present_in_flight = false;
+    // multi-view launches (mm_render_views / mm_present_views): their own chunk list, view records and persistent screens
+    mm_chunk *d_view_chunks = nullptr;
+    uint32_t view_chunks_cap = 0;
+    mmk::ViewRec *d_views = nullptr;     // MM_MAX_VIEWS records, rewritten by every call
+    float *d_vscreen = nullptr;          // vscreen_n screens of vscreen_h x vscreen_w, back to back ([K][H][W])
+    float *d_vscreen2 = nullptr;         // ping-pong partner for the present blur
+    float *d_vsnap = nullptr;            // snapshot for the asynchronous fp32 read-back
+    uint8_t *d_vscreen8 = nullptr;       // RGBA8Unorm texels of the screens (mm_present_views with rgba8)
+    uint32_t vscreen_n = 0, vscreen_w = 0, vscreen_h = 0;
+    float *pending_views[MM_MAX_VIEWS] = {};   // caller buffers that receive h_stage + v * frame at mm_wait (staged views)
     // last launch facts
     uint32_t last_smem = 0, last_blocks_per_sm = 0, last_block_threads = 0, last_tail_cap = 0;
     uint32_t last_y_table = 0;        // y-table entries of the last launch, 0 when it ran without the table
@@ -65,11 +75,13 @@ struct Launch {
     mmk::KernelChoice choice;
     unsigned blocks;
     size_t smem;
+    const mmk::ViewRec *views;   // multi-view launch (choice.views): the device view records
 };
 
 int fail(mm_ctx *ctx, int code, const std::string &msg);
 bool traversal_params(const mm_ctx *ctx, uint32_t flags, mmk::KParams &p);
-int build_launch(mm_ctx *ctx, const mm_uniform *uni, const mm_params *par, bool debug, Launch &L);
+// n_views > 0: a multi-view launch of n_views views over the chunk list of mm_render_views (uni: the first view).
+int build_launch(mm_ctx *ctx, const mm_uniform *uni, const mm_params *par, bool debug, Launch &L, uint32_t n_views = 0);
 int do_launch(mm_ctx *ctx, Launch &L);
 int ensure_screen(mm_ctx *ctx, uint32_t W, uint32_t H);
 void counters_out(const mmk::Counters *h, mm_counters *o);

@@ -24,12 +24,17 @@
 namespace mmk {
 namespace {
 
-// Stores one finished pixel, from the sums of its spp tone-mapped samples in the reference's order (shaders.metal:343-366),
-// into every output of the dispatch: the frame, the tiles, the zero-copy host frame and the frames of the fused exchange.
-__device__ __forceinline__ void deliver_pixel(const KParams &P, float sx, float sy, float sz, uint32_t pxx, uint32_t pxy, size_t tile) {
+// A finished pixel from the sums of its spp tone-mapped samples in the reference's order (shaders.metal:343-366).
+__device__ __forceinline__ float4 pixel_value(const KParams &P, float sx, float sy, float sz) {
     const float d = (float)(int)P.spp;
     float4 px = make_float4(fdiv(sx, d), fdiv(sy, d), fdiv(sz, d), 1.0f);
     if (P.quant8) px = quant8(px);
+    return px;
+}
+// Stores one finished pixel into every output of the dispatch: the frame, the tiles, the zero-copy host frame and the frames of
+// the fused exchange.
+__device__ __forceinline__ void deliver_pixel(const KParams &P, float sx, float sy, float sz, uint32_t pxx, uint32_t pxy, size_t tile) {
+    const float4 px = pixel_value(P, sx, sy, sz);
     if (P.image && pxx < P.W && pxy < P.H) reinterpret_cast<float4 *>(P.image)[(size_t)pxy * P.W + pxx] = px;
     if (P.tiles) reinterpret_cast<float4 *>(P.tiles)[tile] = px;
     if ((P.n_peers || P.host_out) && pxx < P.W && pxy < P.H) {
@@ -41,6 +46,18 @@ __device__ __forceinline__ void deliver_pixel(const KParams &P, float sx, float 
         } else {                                                    // fused exchange, NVLink peer mappings: one store per rank's frame
             for (uint32_t i = 0; i < P.n_peers; i++) reinterpret_cast<float4 *>(P.peers[i])[at] = px;
         }
+    }
+}
+
+// The same for view v of a multi-view launch: its screen and its zero-copy host frame.
+__device__ __forceinline__ void deliver_view_pixel(const KParams &P, const ViewRec *views, uint32_t v, float sx, float sy, float sz, uint32_t pxx,
+                                                   uint32_t pxy) {
+    const float4 px = pixel_value(P, sx, sy, sz);
+    if (pxx < P.W && pxy < P.H) {
+        const ViewRec &V = views[v];
+        const size_t at = (size_t)pxy * P.W + pxx;
+        reinterpret_cast<float4 *>(V.screen)[at] = px;
+        if (V.host_out) reinterpret_cast<float4 *>(V.host_out)[at] = px;   // zero-copy output, over PCIe
     }
 }
 
@@ -85,9 +102,10 @@ __device__ __forceinline__ void add_counters(const KParams &P, uint32_t seg, uin
 // TAIL: qi is the straggler-queue entry of the thread's path when trace_kernel queued it (0xFFFFFFFF otherwise).  A pixel with
 // a queued sample is not stored here: its other samples go to a deferred-pixel slot, and trace_tail_kernel delivers the pixel
 // when its last sample arrives.
-template <bool CNT, bool TAIL, int kBlockThreads>
+// MV: a multi-view launch (views: its view records), where k is the launch's group index and the pixel goes to view k / group_count.
+template <bool CNT, bool TAIL, int kBlockThreads, bool MV = false>
 __device__ __forceinline__ void block_epilogue(const KParams &P, float *red, bool active, uint32_t flat, uint32_t pxx, uint32_t pxy, uint32_t k,
-                                               uint32_t seg, uint32_t nhits, uint32_t nliteral, Tally tl, uint32_t qi) {
+                                               uint32_t seg, uint32_t nhits, uint32_t nliteral, Tally tl, uint32_t qi, const ViewRec *views = nullptr) {
     const uint32_t tid = threadIdx.x;
     float *rx = red, *ry = red + kBlockThreads, *rz = red + 2 * kBlockThreads;
     bool deferred = false;
@@ -136,7 +154,8 @@ __device__ __forceinline__ void block_epilogue(const KParams &P, float *red, boo
         for (uint32_t i = 1; i < P.spp / 8; i++) {
             sx = fadd(sx, rx[tid + 8 * i]); sy = fadd(sy, ry[tid + 8 * i]); sz = fadd(sz, rz[tid + 8 * i]);
         }
-        deliver_pixel(P, sx, sy, sz, pxx, pxy, (size_t)k * P.ppc + (flat >> P.log2_spp));
+        if (MV) deliver_view_pixel(P, views, k / P.group_count, sx, sy, sz, pxx, pxy);
+        else deliver_pixel(P, sx, sy, sz, pxx, pxy, (size_t)k * P.ppc + (flat >> P.log2_spp));
     }
     add_counters<CNT>(P, seg, nhits, nliteral, active ? 1u : 0u, tl);
 }
@@ -217,9 +236,10 @@ __device__ __forceinline__ void write_dbg(const KParams &P, uint64_t path, uint3
 // (one atomic per warp; entries past tail_cap stay with the warp, which is the one-kernel behaviour) and leaves the bounce loop.
 // trace_tail_kernel then runs the queued paths densely, one thread per path, with the same traversal and shading code.
 // The body of trace_kernel (YT = false) and trace_ytab_kernel (YT = true: the y-table traversal, whose table follows red[] in
-// dynamic shared memory, n_yiv entries of kYEntryStride bytes per warp).
-template <bool CNT, bool DBG, bool YT, int kBlockThreads>
-__device__ __forceinline__ void trace_body(const KParams &P) {
+// dynamic shared memory, n_yiv entries of kYEntryStride bytes per warp).  MV: the multi-view launch of views_kernel /
+// views_ytab_kernel (start_view_path, deliver_view_pixel); path indices, and with them the debug arrays, are view-major.
+template <bool CNT, bool DBG, bool YT, int kBlockThreads, bool MV = false>
+__device__ __forceinline__ void trace_body(const KParams &P, const ViewRec *views = nullptr) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     float *red = reinterpret_cast<float *>(smem_raw);                      // 3 * kBlockThreads floats
     const uint32_t ytab = YT ? 3u * kBlockThreads * sizeof(float) + (threadIdx.x >> 5) * P.n_yiv * kYEntryStride + (threadIdx.x & 31u) * 8u : 0u;
@@ -238,7 +258,7 @@ __device__ __forceinline__ void trace_body(const KParams &P) {
     bool n_alive = false;
 
     if (active) {
-        const PathStart ps = start_path(P, path);
+        const PathStart ps = MV ? start_view_path(P, views, path) : start_path(P, path);
         k = ps.k; flat = ps.flat; pxx = ps.pxx; pxy = ps.pxy;
         n_alive = 0 < P.bounce_limit;                                      // :306, n = 0
         st_ori = ps.ori; st_dir = ps.dir; st_state = ps.state;
@@ -284,7 +304,7 @@ __device__ __forceinline__ void trace_body(const KParams &P) {
 
     red[threadIdx.x] = sample.x; red[kBlockThreads + threadIdx.x] = sample.y; red[2 * kBlockThreads + threadIdx.x] = sample.z;
     __syncthreads();
-    block_epilogue<CNT, true, kBlockThreads>(P, red, active, flat, pxx, pxy, k, seg, nhits, nliteral, tl, qi);
+    block_epilogue<CNT, true, kBlockThreads, MV>(P, red, active, flat, pxx, pxy, k, seg, nhits, nliteral, tl, qi, views);
 }
 
 template <bool CNT, bool DBG, int kBlockThreads>
@@ -295,12 +315,21 @@ template <bool CNT, bool DBG, int kBlockThreads>
 __global__ void __launch_bounds__(kBlockThreads, 1024 / kBlockThreads)
 trace_ytab_kernel(const __grid_constant__ KParams P) { trace_body<CNT, DBG, true, kBlockThreads>(P); }
 
+// mm_render_views: K views of group_count groups each in one launch (K * group_count * T paths, view-major).
+template <bool CNT, bool DBG, int kBlockThreads>
+__global__ void __launch_bounds__(kBlockThreads, 1024 / kBlockThreads)
+views_kernel(const __grid_constant__ KParams P, const ViewRec *__restrict__ views) { trace_body<CNT, DBG, false, kBlockThreads, true>(P, views); }
+
+template <bool CNT, bool DBG, int kBlockThreads>
+__global__ void __launch_bounds__(kBlockThreads, 1024 / kBlockThreads)
+views_ytab_kernel(const __grid_constant__ KParams P, const ViewRec *__restrict__ views) { trace_body<CNT, DBG, true, kBlockThreads, true>(P, views); }
+
 // The paths trace_kernel queued, one thread per path in queue order (dense warps), from where they stopped to their end.  The
 // thread that stores a pixel's last missing sample reduces the pixel's samples in the reference's order and delivers it.
-// YT: the y-table traversal, as in trace_ytab_kernel; the table is the whole dynamic shared memory.
-template <bool CNT, bool DBG, bool YT>
-__global__ void __launch_bounds__(kTailBlock, 1024 / kTailBlock)
-trace_tail_kernel(const __grid_constant__ KParams P) {
+// YT: the y-table traversal, as in trace_ytab_kernel; the table is the whole dynamic shared memory.  MV: the paths of a
+// multi-view launch (views_tail_kernel); a deferred pixel's tile index k * ppc + pixel names its view, k / group_count.
+template <bool CNT, bool DBG, bool YT, bool MV>
+__device__ __forceinline__ void tail_body(const KParams &P, const ViewRec *views) {
     const unsigned long long head = P.counters->tail_paths;                // written by trace_kernel, the launch before
     const uint32_t nq = head < P.tail_cap ? (uint32_t)head : P.tail_cap;
     const uint32_t root = P.root_count ? (kLeafBit | P.root_link | (P.root_count << 24)) : P.root_link;
@@ -340,13 +369,25 @@ trace_tail_kernel(const __grid_constant__ KParams P) {
             if (atomicSub(reinterpret_cast<uint32_t *>(v), 1u) == 1u) {    // the pixel's last missing sample
                 __threadfence();
                 const uint32_t *h = reinterpret_cast<const uint32_t *>(v);
-                deliver_pixel(P, reduce_samples(v + 4, P.spp, 1), reduce_samples(v + 4 + P.spp, P.spp, 1),
-                              reduce_samples(v + 4 + 2 * P.spp, P.spp, 1), h[1], h[2], h[3]);
+                if (MV)
+                    deliver_view_pixel(P, views, h[3] / (P.group_count * P.ppc), reduce_samples(v + 4, P.spp, 1), reduce_samples(v + 4 + P.spp, P.spp, 1),
+                                       reduce_samples(v + 4 + 2 * P.spp, P.spp, 1), h[1], h[2]);
+                else
+                    deliver_pixel(P, reduce_samples(v + 4, P.spp, 1), reduce_samples(v + 4 + P.spp, P.spp, 1),
+                                  reduce_samples(v + 4 + 2 * P.spp, P.spp, 1), h[1], h[2], h[3]);
             }
         }
     }
     add_counters<CNT>(P, seg, nhits, nliteral, 0u, tl);
 }
+
+template <bool CNT, bool DBG, bool YT>
+__global__ void __launch_bounds__(kTailBlock, 1024 / kTailBlock)
+trace_tail_kernel(const __grid_constant__ KParams P) { tail_body<CNT, DBG, YT, false>(P, nullptr); }
+
+template <bool CNT, bool DBG, bool YT>
+__global__ void __launch_bounds__(kTailBlock, 1024 / kTailBlock)
+views_tail_kernel(const __grid_constant__ KParams P, const ViewRec *__restrict__ views) { tail_body<CNT, DBG, YT, true>(P, views); }
 
 // Verification hook (mm_trace_rays): one traversal per ray through the bounce loop's form selection, 32 consecutive rays to a
 // warp, so that the caller decides each warp's composition.  rays: n x 8 floats (ori.xyz, dir.xyz, t, alive != 0); slots: the
@@ -672,8 +713,8 @@ __global__ void div3_selftest_kernel(unsigned long long *mismatches) {
 
 // fragment_shader's 5-tap blur (shaders.metal:214-225), ping-pong.  HBM-bound: 16 B read + 16 B written per pixel (the four
 // neighbour taps hit L1/L2).  One thread handles two horizontally adjacent pixels (8 loads for 2 pixels instead of 10).
-__global__ void __launch_bounds__(256) blur_kernel(const float4 *__restrict__ src, float4 *__restrict__ dst, uint32_t W, uint32_t H, bool q8,
-                                                   uchar4 *__restrict__ bytes) {
+__device__ __forceinline__ void blur_body(const float4 *__restrict__ src, float4 *__restrict__ dst, uint32_t W, uint32_t H, bool q8,
+                                          uchar4 *__restrict__ bytes) {
     const uint32_t x0 = 2u * (blockIdx.x * blockDim.x + threadIdx.x), y = blockIdx.y;
     if (x0 >= W || y >= H) return;
     const float4 zero = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
@@ -695,6 +736,17 @@ __global__ void __launch_bounds__(256) blur_kernel(const float4 *__restrict__ sr
         bytes[row + x0] = make_uchar4((unsigned char)unorm8(o0.x), (unsigned char)unorm8(o0.y), (unsigned char)unorm8(o0.z), (unsigned char)unorm8(o0.w));
         if (two) bytes[row + x0 + 1] = make_uchar4((unsigned char)unorm8(o1.x), (unsigned char)unorm8(o1.y), (unsigned char)unorm8(o1.z), (unsigned char)unorm8(o1.w));
     }
+}
+__global__ void __launch_bounds__(256) blur_kernel(const float4 *__restrict__ src, float4 *__restrict__ dst, uint32_t W, uint32_t H, bool q8,
+                                                   uchar4 *__restrict__ bytes) {
+    blur_body(src, dst, W, H, q8, bytes);
+}
+// The blur of mm_present_views: screen blockIdx.z of [n][H][W] screens stored back to back, each blurred as blur_kernel blurs one
+// (the bounds checks keep every tap inside its own screen).
+__global__ void __launch_bounds__(256) blur_views_kernel(const float4 *__restrict__ src, float4 *__restrict__ dst, uint32_t W, uint32_t H, bool q8,
+                                                         uchar4 *__restrict__ bytes) {
+    const size_t at = (size_t)blockIdx.z * W * H;
+    blur_body(src + at, dst + at, W, H, q8, bytes ? bytes + at : nullptr);
 }
 
 // Micro-benchmarks for the two rooflines the path is measured against (SURVEY §8 d): how fast can this GPU fetch 56 useful
@@ -750,9 +802,27 @@ const void *tail_ptr(bool yt) {
     return yt ? reinterpret_cast<const void *>(&trace_tail_kernel<C, D, true>) : reinterpret_cast<const void *>(&trace_tail_kernel<C, D, false>);
 }
 
+template <bool C, bool D>
+const void *kptr_views(int bt, bool yt) {
+    if (yt)
+        return bt == kSmallBlock ? reinterpret_cast<const void *>(&views_ytab_kernel<C, D, kSmallBlock>)
+                                 : reinterpret_cast<const void *>(&views_ytab_kernel<C, D, kLargeBlock>);
+    return bt == kSmallBlock ? reinterpret_cast<const void *>(&views_kernel<C, D, kSmallBlock>)
+                             : reinterpret_cast<const void *>(&views_kernel<C, D, kLargeBlock>);
+}
+
+template <bool C, bool D>
+const void *views_tail_ptr(bool yt) {
+    return yt ? reinterpret_cast<const void *>(&views_tail_kernel<C, D, true>) : reinterpret_cast<const void *>(&views_tail_kernel<C, D, false>);
+}
+
 }  // namespace
 
 const void *kernel_ptr(KernelChoice c) {
+    if (c.views) {
+        if (c.debug) return kptr_views<true, true>(c.block_threads, c.ytab);
+        return c.counters ? kptr_views<true, false>(c.block_threads, c.ytab) : kptr_views<false, false>(c.block_threads, c.ytab);
+    }
     if (c.regroup) {
         if (c.debug) return kptr_rg<true, true>(c.block_threads);
         return c.counters ? kptr_rg<true, false>(c.block_threads) : kptr_rg<false, false>(c.block_threads);
@@ -765,15 +835,16 @@ const void *kernel_ptr(KernelChoice c) {
     return c.counters ? kptr<true, false>(c.block_threads) : kptr<false, false>(c.block_threads);
 }
 
-cudaError_t launch_trace(const KParams &p, KernelChoice c, unsigned blocks, size_t smem_bytes, cudaStream_t stream) {
+cudaError_t launch_trace(const KParams &p, KernelChoice c, unsigned blocks, size_t smem_bytes, cudaStream_t stream, const ViewRec *views) {
     const void *fn = kernel_ptr(c);
-    void *args[] = {const_cast<KParams *>(&p)};
+    void *args[] = {const_cast<KParams *>(&p), &views};                      // the single-view kernels take KParams alone
     return cudaLaunchKernel(fn, dim3(blocks), dim3(c.block_threads), args, smem_bytes, stream);
 }
 
-cudaError_t launch_tail(const KParams &p, KernelChoice c, unsigned blocks, size_t smem_bytes, cudaStream_t stream) {
-    const void *fn = c.debug ? tail_ptr<true, true>(c.ytab) : (c.counters ? tail_ptr<true, false>(c.ytab) : tail_ptr<false, false>(c.ytab));
-    void *args[] = {const_cast<KParams *>(&p)};
+cudaError_t launch_tail(const KParams &p, KernelChoice c, unsigned blocks, size_t smem_bytes, cudaStream_t stream, const ViewRec *views) {
+    const void *fn = c.views ? (c.debug ? views_tail_ptr<true, true>(c.ytab) : (c.counters ? views_tail_ptr<true, false>(c.ytab) : views_tail_ptr<false, false>(c.ytab)))
+                             : (c.debug ? tail_ptr<true, true>(c.ytab) : (c.counters ? tail_ptr<true, false>(c.ytab) : tail_ptr<false, false>(c.ytab)));
+    void *args[] = {const_cast<KParams *>(&p), &views};
     return cudaLaunchKernel(fn, dim3(blocks), dim3(kTailBlock), args, smem_bytes, stream);
 }
 
@@ -812,6 +883,14 @@ cudaError_t launch_blur(const float *src, float *dst, uint32_t W, uint32_t H, cu
     dim3 grid((W + 511) / 512, H);                                            // two pixels per thread
     blur_kernel<<<grid, 256, 0, stream>>>(reinterpret_cast<const float4 *>(src), reinterpret_cast<float4 *>(dst), W, H, quant8,
                                           reinterpret_cast<uchar4 *>(bytes));
+    return cudaGetLastError();
+}
+
+cudaError_t launch_blur_views(const float *src, float *dst, uint32_t W, uint32_t H, uint32_t n, cudaStream_t stream, bool quant8, uint8_t *bytes) {
+    if (W == 0 || H == 0 || n == 0) return cudaSuccess;
+    dim3 grid((W + 511) / 512, H, n);                                         // two pixels per thread, one z slice per screen
+    blur_views_kernel<<<grid, 256, 0, stream>>>(reinterpret_cast<const float4 *>(src), reinterpret_cast<float4 *>(dst), W, H, quant8,
+                                                reinterpret_cast<uchar4 *>(bytes));
     return cudaGetLastError();
 }
 

@@ -97,8 +97,21 @@ static_assert(sizeof(TailPath) == 80, "straggler record is 80 B");
 // A deferred-pixel slot is 4 + 3 spp words: (samples still missing, pixel x, pixel y, tile index), then the pixel's tone-mapped
 // samples as three planes of spp floats.
 
+// One view of a multi-view launch (mm_render_views), 80 B, uploaded with every call.  The multi-view kernels take the array
+// as a second parameter after KParams, which keeps KParams, and with it every single-view kernel, as it is.  The views share
+// everything of KParams but its camera and time (uni carries their common view size and chunk width); of its outputs,
+// image, tiles, peers and host_out are unused.
+struct __align__(16) ViewRec {
+    mm_uniform uni;            // the view's camera and time
+    uint32_t chunk_off;        // the view's chunk list starts at KParams::chunks + chunk_off
+    uint32_t pad;
+    float *screen;             // the view's persistent screen, H*W*4 floats
+    float *host_out;           // zero-copy output: the device alias of the view's mapped pinned host frame, or null
+};
+static_assert(sizeof(ViewRec) == 80, "view record is 80 B");
+
 struct KParams {
-    mm_uniform uni;            // the reference's 56-byte uniform, by value like set_bytes (main.rs:875-879)
+    mm_uniform uni;           // the reference's 56-byte uniform, by value like set_bytes (main.rs:875-879)
     uint32_t spp, log2_spp;
     int32_t bounce_limit, mirror_limit;
     uint32_t grid_x, grid_y;
@@ -160,12 +173,14 @@ inline int block_threads_for(uint32_t spp) { return spp <= (uint32_t)kSmallBlock
 
 // Returns the kernel's static properties for the occupancy query and launch.
 // ytab: trace_ytab_kernel / trace_tail_kernel<..., true> (the y-table traversal) instead of trace_kernel.
-struct KernelChoice { bool counters, debug; int block_threads; bool pool; bool regroup; bool ytab; };
+// views: the multi-view kernels (views_kernel / views_ytab_kernel, views_tail_kernel) of mm_render_views.
+struct KernelChoice { bool counters, debug; int block_threads; bool pool; bool regroup; bool ytab; bool views; };
 const void *kernel_ptr(KernelChoice c);
 const void *pool_kernel_ptr(KernelChoice c);
 cudaError_t launch_pool(const KParams &p, KernelChoice c, unsigned blocks, unsigned threads, size_t smem_bytes, cudaStream_t stream);
-cudaError_t launch_trace(const KParams &p, KernelChoice c, unsigned blocks, size_t smem_bytes, cudaStream_t stream);
-cudaError_t launch_tail(const KParams &p, KernelChoice c, unsigned blocks, size_t smem_bytes, cudaStream_t stream);
+// views: the view records of a multi-view launch (c.views), device memory.
+cudaError_t launch_trace(const KParams &p, KernelChoice c, unsigned blocks, size_t smem_bytes, cudaStream_t stream, const ViewRec *views = nullptr);
+cudaError_t launch_tail(const KParams &p, KernelChoice c, unsigned blocks, size_t smem_bytes, cudaStream_t stream, const ViewRec *views = nullptr);
 constexpr int kTailBlock = 256;
 // mm_trace_rays: probe_rays_kernel over n rays (ytab: the y-table traversal; device buffers as in the header's prototype)
 constexpr uint32_t kProbeBlock = 64;
@@ -176,6 +191,8 @@ cudaError_t launch_mb_ffma(uint32_t iters, unsigned blocks, float *sink, cudaStr
 cudaError_t launch_scatter_all(const float *gathered, float *image, const mm_chunk *chunks, uint32_t world, uint32_t max_count,
                                uint32_t n_groups, uint32_t chunk, uint32_t W, uint32_t H, cudaStream_t stream);
 cudaError_t launch_blur(const float *src, float *dst, uint32_t W, uint32_t H, cudaStream_t stream, bool quant8 = false, uint8_t *bytes = nullptr);
+// The same over n screens stored back to back ([n][H][W]) in one launch; no tap crosses a screen's border.
+cudaError_t launch_blur_views(const float *src, float *dst, uint32_t W, uint32_t H, uint32_t n, cudaStream_t stream, bool quant8, uint8_t *bytes);
 cudaError_t launch_div3_selftest(unsigned long long *d_mismatches, cudaStream_t stream);
 cudaError_t launch_quot_selftest(uint64_t n, uint64_t seed, unsigned long long *d_mismatches, cudaStream_t stream);
 cudaError_t launch_scatter(const float *tiles, float *image, const mm_chunk *chunks, uint32_t grid_groups, uint32_t group_first,

@@ -424,13 +424,10 @@ struct PathStart {
     uint32_t pxx, pxy;         // pixel
     uint32_t k, flat;          // group index within the launch, thread index within the group
 };
-__device__ __forceinline__ PathStart start_path(const KParams &P, uint64_t path) {
-    PathStart s;
-    s.k = (uint32_t)(path / P.T);
-    s.flat = (uint32_t)(path - (uint64_t)s.k * P.T);
-    const uint32_t g = P.group_first + s.k * P.group_step;
+// Thread s.flat of grid group g under camera cam at frame `time`, chunk list `chunks` (s.k and s.flat set by the caller).
+__device__ __forceinline__ void start_at(const KParams &P, PathStart &s, uint32_t g, const mm_chunk *chunks, const mm_camera &cam, uint32_t time) {
     const uint32_t tgx = g % P.grid_x, tgy = g / P.grid_x;
-    const mm_chunk ch = P.chunks[g];                                   // :266-267
+    const mm_chunk ch = chunks[g];                                     // :266-267
     const uint32_t gx = s.flat % P.dim_x, gy = s.flat / P.dim_x;       // inverse of :271
     const uint32_t chunk = P.uni.chunk_width;
     const uint32_t pixel_number = s.flat >> P.log2_spp;                // :272
@@ -438,7 +435,6 @@ __device__ __forceinline__ PathStart start_path(const KParams &P, uint64_t path)
     s.pxy = ch.y + pixel_number % chunk;                               // :273,275
     const uint32_t texid_x = tgx * P.dim_x + gx, texid_y = tgy * P.dim_y + gy;
 
-    const mm_camera &cam = P.uni.cam;
     const V3 center = mk(cam.camera_center.x, cam.camera_center.y, cam.camera_center.z);
     const float pnx = fdiv(__uint2float_rn(s.pxx), P.uni.view_width), pny = fdiv(__uint2float_rn(s.pxy), P.uni.view_height);   // :281
     const V3 corner = sub3(center, mk(fdiv(cam.viewport.x, 2.0f), fdiv(cam.viewport.y, 2.0f), -cam.focal_length));        // :282
@@ -450,12 +446,30 @@ __device__ __forceinline__ PathStart start_path(const KParams &P, uint64_t path)
     sample_noise_xy(P.noise, P.noise_w, P.noise_h, __uint2float_rn(gx), __uint2float_rn(gy), nx, ny);   // :291
     // :298 — float + uint promotes to float, products wrap in u32, left to right; float->uint saturates.
     const float seed_f = fadd(fadd(fadd(fadd(nx, ny), __uint2float_rn(texid_x * 15823u)), __uint2float_rn(texid_y * 9737333u)),
-                              __uint2float_rn(P.uni.time));
+                              __uint2float_rn(time));
     uint32_t state = __float2uint_rz(seed_f);
     s.ori = center;                                                    // :302
     const float j1 = rnd_pm1(state), j2 = rnd_pm1(state);
     s.dir = add3(ray_dir, scale3(mk(j1, j2, 0.0f), 0.001f));           // :303
     s.state = state;
+}
+__device__ __forceinline__ PathStart start_path(const KParams &P, uint64_t path) {
+    PathStart s;
+    s.k = (uint32_t)(path / P.T);
+    s.flat = (uint32_t)(path - (uint64_t)s.k * P.T);
+    start_at(P, s, P.group_first + s.k * P.group_step, P.chunks, P.uni.cam, P.uni.time);
+    return s;
+}
+// The same for a multi-view launch (mm_render_views): the launch's group k is group k mod group_count of view
+// k / group_count, which starts exactly as that group of a single-view dispatch with the view's camera, time and chunks.
+__device__ __forceinline__ PathStart start_view_path(const KParams &P, const ViewRec *views, uint64_t path) {
+    PathStart s;
+    s.k = (uint32_t)(path / P.T);
+    s.flat = (uint32_t)(path - (uint64_t)s.k * P.T);
+    const uint32_t v = s.k / P.group_count, kv = s.k - v * P.group_count;
+    const ViewRec &V = views[v];
+    const mm_camera cam = V.uni.cam;
+    start_at(P, s, P.group_first + kv * P.group_step, P.chunks + V.chunk_off, cam, V.uni.time);
     return s;
 }
 

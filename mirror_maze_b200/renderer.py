@@ -155,6 +155,56 @@ class Renderer:
         self._ck(self._lib.mm_wait(self._ctx, C.byref(cnt)))
         return cnt.as_dict()
 
+    # -- several views in one launch ----------------------------------------------------------------------------------
+    def render_views(self, unis, params, chunk_lists, outs=None, debug=False):
+        """mm_render_views: one launch for len(unis) views of the scene, each with its own uniform (camera, time) and chunk
+        list (chunk_lists[v], grid_x * grid_y chunks each), each into its own persistent view screen.  outs: None, or one entry
+        per view: None, a HostFrame (zero-copy) or a [H, W, 4] float32 array.  Returns (outs, counters dict summed over the
+        views, debug dict | None); the debug arrays are view-major, one row of group_count * chunk_width^2 * spp paths per view."""
+        n = len(unis)
+        if n == 0 or len(chunk_lists) != n or (outs is not None and len(outs) != n):
+            raise ValueError("one uniform and one chunk list (and one output, when given) per view")
+        u_arr = (abi.Uniform * n)(*unis)
+        chunks = np.ascontiguousarray(np.concatenate([np.ascontiguousarray(c, dtype=CHUNK_DTYPE) for c in chunk_lists]))
+        out_arr = None
+        if outs is not None:
+            ptrs = []
+            for o in outs:
+                if o is None:
+                    ptrs.append(None)
+                elif isinstance(o, HostFrame):
+                    ptrs.append(o.ptr)
+                else:
+                    assert o.dtype == np.float32 and o.flags["C_CONTIGUOUS"] and o.size == int(unis[0].view_height) * int(unis[0].view_width) * 4
+                    ptrs.append(o.ctypes.data)
+            out_arr = (C.c_void_p * n)(*ptrs)
+        cnt = Counters()
+        dbg_struct, dbg = None, None
+        if debug:
+            n_groups = params.group_count or params.grid_x * params.grid_y
+            n_paths = n * n_groups * unis[0].chunk_width ** 2 * params.spp
+            dbg = {"first_hit": np.empty(n_paths, np.uint32), "segments": np.empty(n_paths, np.uint32),
+                   "mirror_hits": np.empty(n_paths, np.uint32), "radiance": np.empty((n_paths, 3), np.float32)}
+            dbg_struct = Debug(dbg["first_hit"].ctypes.data_as(C.POINTER(C.c_uint32)),
+                               dbg["segments"].ctypes.data_as(C.POINTER(C.c_uint32)),
+                               dbg["mirror_hits"].ctypes.data_as(C.POINTER(C.c_uint32)),
+                               dbg["radiance"].ctypes.data_as(C.POINTER(C.c_float)))
+        self._ck(self._lib.mm_render_views(self._ctx, u_arr, n, C.byref(params), chunks.ctypes.data, len(chunks), out_arr,
+                                           C.byref(cnt), C.byref(dbg_struct) if dbg_struct else None))
+        self._n_views = n
+        return outs, cnt.as_dict(), dbg
+
+    def present_views(self, outs=None, rgba8=False):
+        """mm_present_views: the present blur of every view screen in one launch (rgba8: the quantising blur of RGBA8 screens),
+        read back asynchronously into outs (None, or one entry per view: None or a HostFrame / pinned address; rgba8 fills
+        the first H*W*4 bytes with the texels).  Done at wait_present()."""
+        arr = None
+        if outs is not None:
+            if len(outs) != getattr(self, "_n_views", len(outs)):
+                raise ValueError("one output (or None) per view of the last render_views")
+            arr = (C.c_void_p * len(outs))(*[None if o is None else (o.ptr if isinstance(o, HostFrame) else int(o)) for o in outs])
+        self._ck(self._lib.mm_present_views(self._ctx, 1 if rgba8 else 0, arr))
+
     def render_multicast_device(self, uniform, params, mc_ptr):
         """mm_render_multicast_device: every finished pixel is one multimem.st to an NVSwitch multicast address."""
         self._ck(self._lib.mm_render_multicast_device(self._ctx, C.byref(uniform), C.byref(params), mc_ptr))

@@ -27,6 +27,7 @@ const _: () = assert!(std::mem::size_of::<Plane>() == 48 && std::mem::size_of::<
 pub const MM_EXCHANGE_PEER: c_int = 0;
 pub const MM_EXCHANGE_NCCL: c_int = 1;
 pub const MM_EXCHANGE_NONE: c_int = 2;
+pub const MM_MAX_VIEWS: u32 = 64;
 
 extern "C" {
     pub fn mm_create(cuda_device: c_int, out: *mut *mut mm_ctx) -> c_int;
@@ -41,6 +42,13 @@ extern "C" {
     pub fn mm_render_async(ctx: *mut mm_ctx, uni: *const Uniform, params: *const Params, chunks: *const Chunk, n_chunks: u32,
                            out_rgba: *mut f32, debug: *const std::ffi::c_void) -> c_int;
     pub fn mm_wait(ctx: *mut mm_ctx, counters: *mut Counters) -> c_int;
+    // several camera views in one launch, each with its own uniform, chunk list and persistent view screen (MM_MAX_VIEWS = 64)
+    pub fn mm_render_views_async(ctx: *mut mm_ctx, unis: *const Uniform, n_views: u32, params: *const Params, chunks: *const Chunk,
+                                 n_chunks: u32, out_rgba: *const *mut f32, debug: *const std::ffi::c_void) -> c_int;
+    pub fn mm_render_views(ctx: *mut mm_ctx, unis: *const Uniform, n_views: u32, params: *const Params, chunks: *const Chunk,
+                           n_chunks: u32, out_rgba: *const *mut f32, counters: *mut Counters, debug: *const std::ffi::c_void) -> c_int;
+    // the blur of every view screen in one launch; out: null or one pinned pointer (or null) per view, done at mm_wait_present
+    pub fn mm_present_views(ctx: *mut mm_ctx, rgba8: u32, out: *const *mut std::ffi::c_void) -> c_int;
     // pin + map a Vec<f32> frame once: the kernel then stores finished pixels straight into it (zero-copy output)
     pub fn mm_host_register(ptr: *mut std::ffi::c_void, bytes: usize) -> c_int;
     pub fn mm_host_unregister(ptr: *mut std::ffi::c_void) -> c_int;
