@@ -70,7 +70,8 @@ typedef struct mm_chunk { uint32_t x, y; } mm_chunk;
  * groups over calls or GPUs gives the bits of a single full-grid call.  group_count = 0 means "all".
  */
 typedef struct mm_params {
-    uint32_t spp;            /* samples per pixel: power of two, 1..256                              */
+    uint32_t spp;            /* samples per pixel: power of two, 1..1024 (512 and 1024: one block of 1024
+                                threads holds two pixels or one; chunk_width^2 * spp <= 2^20 still applies) */
     uint32_t bounce_limit;   /* shaders.metal:294                                                    */
     uint32_t mirror_limit;   /* shaders.metal:295                                                    */
     uint32_t grid_x, grid_y; /* virtual threadgroups per grid (main.rs:646-650)                      */
@@ -100,7 +101,9 @@ typedef struct mm_params {
 #define MM_FLAG_REGROUP     1024u   /* trace with trace_kernel_rg: the default kernel plus warp-level ray compaction — at segment boundaries
                                       the block's live paths are re-formed into warps through shared memory, sorted by ray steepness
                                       |dir.y|, ended paths dropped.  Same bits; fewer instructions (-14 % interior-body executions) but
-                                      measured slower on B200 (profiles/r2_experiments.md), kept as the evidence for that design    */
+                                      measured slower on B200 (profiles/r2_experiments.md), kept as the evidence for that design.
+                                      Its blocks hold at most 256 threads, so above spp 256 the default kernel runs instead
+                                      (with the straggler tail), as MM_FLAG_POOL_KERNEL falls back above spp 64             */
 #define MM_FLAG_NO_TAIL     4096u   /* trace every path to its end in the one-thread-per-path kernel (for comparisons; same bits).  By
                                       default a warp that is past bounce_limit segments with at most 8 live lanes hands those paths to
                                       a second kernel that runs them densely, one thread per path (render_kernel.cu, DESIGN.md §4)  */
@@ -139,7 +142,7 @@ typedef struct mm_debug {
 #define MM_ERR_CUDA          -2   /* a CUDA runtime call failed; see mm_last_error                   */
 #define MM_ERR_NO_SCENE      -3   /* render before mm_upload_scene                                   */
 #define MM_ERR_BVH           -4   /* malformed BVH: child out of range, cycle, depth above MM_MAX_STACK */
-#define MM_ERR_UNSUPPORTED   -5   /* spp not a power of two <= 256, chunk_width^2*spp > limits, ...  */
+#define MM_ERR_UNSUPPORTED   -5   /* spp not a power of two <= 1024, chunk_width^2*spp > limits, ... */
 #define MM_ERR_NOMEM         -6
 
 #define MM_MAX_STACK 52           /* device traversal stack: the reference's 50 entries (unchecked, shaders.metal:123) plus

@@ -288,7 +288,7 @@ int build_launch(mm_ctx *ctx, const mm_uniform *uni, const mm_params *par, bool 
     if (!uni || !par) return fail(ctx, MM_ERR_INVALID, "null uniform or params");
     if (!ctx->have_scene) return fail(ctx, MM_ERR_NO_SCENE, "no scene uploaded");
     const uint32_t spp = par->spp, chunk = uni->chunk_width;
-    if (spp == 0 || (spp & (spp - 1)) || spp > 256) return fail(ctx, MM_ERR_UNSUPPORTED, "spp must be a power of two in 1..256");
+    if (spp == 0 || (spp & (spp - 1)) || spp > kMaxSpp) return fail(ctx, MM_ERR_UNSUPPORTED, "spp must be a power of two in 1..1024");
     if (chunk == 0 || chunk > 64) return fail(ctx, MM_ERR_UNSUPPORTED, "chunk_width must be in 1..64");
     const uint64_t T = (uint64_t)chunk * chunk * spp;
     if (T > (1u << 20)) return fail(ctx, MM_ERR_UNSUPPORTED, "chunk_width^2 * spp too large");
@@ -333,9 +333,10 @@ int build_launch(mm_ctx *ctx, const mm_uniform *uni, const mm_params *par, bool 
     L.views = n_views ? ctx->d_views : nullptr;
     // the multi-view kernels exist for the default kernel only (mm_render_views refuses the flags of the other two)
     if (!n_views && configure_pool(ctx, par, L)) return MM_OK;
-    // opt-in (MM_FLAG_REGROUP, or MM_KERNEL=regroup for tuning runs): the kernel that re-forms the block's warps at segment boundaries
+    // opt-in (MM_FLAG_REGROUP, or MM_KERNEL=regroup for tuning runs): the kernel that re-forms the block's warps at segment
+    // boundaries.  Its largest block is kLargeBlock, so above spp 256 the default kernel runs whatever the flag says.
     const char *env_kernel = getenv("MM_KERNEL");
-    L.choice.regroup = !n_views && ((par->flags & MM_FLAG_REGROUP) || (env_kernel && !strcmp(env_kernel, "regroup")));
+    L.choice.regroup = !n_views && p.spp <= (uint32_t)kLargeBlock && ((par->flags & MM_FLAG_REGROUP) || (env_kernel && !strcmp(env_kernel, "regroup")));
     int bt = block_threads_for(p.spp);
     if (L.choice.regroup) {
         const int want = (int)env_u32("MM_RG_BLOCK", kLargeBlock, 64, kLargeBlock);       // developer override: 64 / 128 / 256

@@ -7,8 +7,10 @@
 //   present pass (:888-893)  ->  mm_present (optional)
 // and writes the frame as a binary PPM (sqrt tone-map already applied by the kernel, as in the shader) or raw fp32.
 //
-//   mm_headless [--maze N] [--width W] [--height H] [--spp S] [--bounces B] [--frames F] [--blur] [--noise file.rgba8]
-//               [--out frame.ppm] [--raw frame.f32] [--gpus N] [--exchange peer|nccl|none] [--pageable]
+//   mm_headless [--maze N] [--width W] [--height H] [--spp S] [--chunk C] [--bounces B] [--frames F] [--blur]
+//               [--noise file.rgba8] [--out frame.ppm] [--raw frame.f32] [--gpus N] [--exchange peer|nccl|none] [--pageable]
+// --chunk C is the uniform's chunk_width (default 4, the reference's): each virtual threadgroup renders a C x C chunk, so
+// --chunk 1 --spp 1024 is the reference's one-pixel-per-threadgroup shape (1024 / C^2 samples fill its 32 x 32 threads).
 // --gpus N > 1 renders through mm_multi (one process, N devices: the frame's groups interleaved over the devices).  The
 // frame buffer is mapped pinned memory from mm_host_alloc (zero-copy output) unless --pageable asks for a plain vector.
 #include <chrono>
@@ -26,7 +28,7 @@ static int fail(mm_ctx *ctx, const char *what, int rc) {
 }
 
 int main(int argc, char **argv) {
-    uint32_t maze = 10, W = 1024, H = 768, spp = 64, bounces = 5, frames = 1;   // the reference's literals
+    uint32_t maze = 10, W = 1024, H = 768, spp = 64, chunk = 4, bounces = 5, frames = 1;   // the reference's literals
     int gpus = 1, exchange = MM_EXCHANGE_PEER;
     bool blur = false, pageable = false;
     std::string out_ppm, out_raw, noise_file;
@@ -37,6 +39,7 @@ int main(int argc, char **argv) {
         else if (a == "--width") W = (uint32_t)std::atoi(next());
         else if (a == "--height") H = (uint32_t)std::atoi(next());
         else if (a == "--spp") spp = (uint32_t)std::atoi(next());
+        else if (a == "--chunk") chunk = (uint32_t)std::atoi(next());
         else if (a == "--bounces") bounces = (uint32_t)std::atoi(next());
         else if (a == "--frames") frames = (uint32_t)std::atoi(next());
         else if (a == "--blur") blur = true;
@@ -84,15 +87,16 @@ int main(int argc, char **argv) {
     }
 
     mm_uniform uni;
-    rc = mm_default_uniform(maze, (float)W, (float)H, 4, 0, &uni);
+    if (chunk == 0 || chunk > W || chunk > H) { std::fprintf(stderr, "--chunk must be in 1..min(width, height)\n"); return 2; }
+    rc = mm_default_uniform(maze, (float)W, (float)H, chunk, 0, &uni);
     if (rc != MM_OK) { std::fprintf(stderr, "mm_default_uniform failed: %d\n", rc); return 1; }
-    const uint32_t n_chunks = mm_gen_chunks((float)W, (float)H, 4, nullptr, 0);
+    const uint32_t n_chunks = mm_gen_chunks((float)W, (float)H, chunk, nullptr, 0);
     std::vector<mm_chunk> chunks(n_chunks);
-    mm_gen_chunks((float)W, (float)H, 4, chunks.data(), n_chunks);
+    mm_gen_chunks((float)W, (float)H, chunk, chunks.data(), n_chunks);
     mm_params par;
     std::memset(&par, 0, sizeof(par));
     par.spp = spp; par.bounce_limit = bounces; par.mirror_limit = 15;
-    par.grid_x = W / 4; par.grid_y = H / 4;                 // one virtual threadgroup per chunk, whole frame
+    par.grid_x = W / chunk; par.grid_y = H / chunk;         // one virtual threadgroup per chunk, whole frame
 
     const size_t frame_floats = (size_t)W * H * 4;
     std::vector<float> frame_vec;
@@ -131,8 +135,8 @@ int main(int argc, char **argv) {
     float kernel_ms = 0.0f;
     if (multi) mm_multi_last_ms(multi, &kernel_ms); else mm_last_ms(ctx, &kernel_ms);
     std::printf("%d GPU(s)%s; ", gpus, multi ? (exchange == MM_EXCHANGE_NCCL ? " [nccl gather]" : exchange == MM_EXCHANGE_NONE ? " [host assembly]" : " [peer stores]") : "");
-    std::printf("maze %ux%u: %u planes, %u nodes; %ux%u x%u spp, %u bounces; %u frame(s): %.3f ms/frame end to end (last kernel %.3f ms), "
-                "%.1f Mrays/s, %llu rays/frame\n", maze, maze, mm_scene_n_planes(scene), mm_scene_n_nodes(scene), W, H, spp, bounces, frames,
+    std::printf("maze %ux%u: %u planes, %u nodes; %ux%u x%u spp, chunk %u, %u bounces; %u frame(s): %.3f ms/frame end to end (last kernel %.3f ms), "
+                "%.1f Mrays/s, %llu rays/frame\n", maze, maze, mm_scene_n_planes(scene), mm_scene_n_nodes(scene), W, H, spp, chunk, bounces, frames,
                 total_ms / frames, kernel_ms, total_rays / total_ms / 1e3, (unsigned long long)cnt.rays);
 
     if (!out_raw.empty()) {

@@ -324,6 +324,21 @@ template <bool CNT, bool DBG, int kBlockThreads>
 __global__ void __launch_bounds__(kBlockThreads, 1024 / kBlockThreads)
 views_ytab_kernel(const __grid_constant__ KParams P, const ViewRec *__restrict__ views) { trace_body<CNT, DBG, true, kBlockThreads, true>(P, views); }
 
+// spp 512 and 1024: the 1024-thread block (kHugeBlock, one block an SM) of the y-table and multi-view kernels.  trace_kernel
+// takes it as a third BLOCK; these three get names of their own, which keeps the instantiation sets of the templates above as
+// they were (tests pin them by name and count).  Same bodies, so the same SASS as a kHugeBlock instantiation would have.
+template <bool CNT, bool DBG>
+__global__ void __launch_bounds__(kHugeBlock, 1)
+trace_ytab_wide_kernel(const __grid_constant__ KParams P) { trace_body<CNT, DBG, true, kHugeBlock>(P); }
+
+template <bool CNT, bool DBG>
+__global__ void __launch_bounds__(kHugeBlock, 1)
+views_wide_kernel(const __grid_constant__ KParams P, const ViewRec *__restrict__ views) { trace_body<CNT, DBG, false, kHugeBlock, true>(P, views); }
+
+template <bool CNT, bool DBG>
+__global__ void __launch_bounds__(kHugeBlock, 1)
+views_ytab_wide_kernel(const __grid_constant__ KParams P, const ViewRec *__restrict__ views) { trace_body<CNT, DBG, true, kHugeBlock, true>(P, views); }
+
 // The paths trace_kernel queued, one thread per path in queue order (dense warps), from where they stopped to their end.  The
 // thread that stores a pixel's last missing sample reduces the pixel's samples in the reference's order and delivers it.
 // YT: the y-table traversal, as in trace_ytab_kernel; the table is the whole dynamic shared memory.  MV: the paths of a
@@ -787,12 +802,14 @@ const void *kptr_rg(int bt) {
 
 template <bool C, bool D>
 const void *kptr(int bt) {
+    if (bt == kHugeBlock) return reinterpret_cast<const void *>(&trace_kernel<C, D, kHugeBlock>);
     return bt == kSmallBlock ? reinterpret_cast<const void *>(&trace_kernel<C, D, kSmallBlock>)
                              : reinterpret_cast<const void *>(&trace_kernel<C, D, kLargeBlock>);
 }
 
 template <bool C, bool D>
 const void *kptr_yt(int bt) {
+    if (bt == kHugeBlock) return reinterpret_cast<const void *>(&trace_ytab_wide_kernel<C, D>);
     return bt == kSmallBlock ? reinterpret_cast<const void *>(&trace_ytab_kernel<C, D, kSmallBlock>)
                              : reinterpret_cast<const void *>(&trace_ytab_kernel<C, D, kLargeBlock>);
 }
@@ -804,6 +821,8 @@ const void *tail_ptr(bool yt) {
 
 template <bool C, bool D>
 const void *kptr_views(int bt, bool yt) {
+    if (bt == kHugeBlock)
+        return yt ? reinterpret_cast<const void *>(&views_ytab_wide_kernel<C, D>) : reinterpret_cast<const void *>(&views_wide_kernel<C, D>);
     if (yt)
         return bt == kSmallBlock ? reinterpret_cast<const void *>(&views_ytab_kernel<C, D, kSmallBlock>)
                                  : reinterpret_cast<const void *>(&views_ytab_kernel<C, D, kLargeBlock>);

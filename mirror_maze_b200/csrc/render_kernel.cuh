@@ -163,13 +163,18 @@ struct KParams {
 
 // Block shapes: 32 warps/SM at <= 64 registers either way.  A block must hold whole pixels (spp | block threads, for the
 // in-block reduction); small blocks retire sooner after their slowest warp (profiles/r1_block_shape.txt), so frames with
-// spp <= kSmallBlock use kSmallBlock threads and only larger sample counts use kLargeBlock.
+// spp <= kSmallBlock use kSmallBlock threads and only larger sample counts use kLargeBlock.  spp 512 and 1024 take the
+// largest block there is, kHugeBlock (two pixels or one a block, one block an SM; DESIGN.md §4).
 #ifndef MM_SMALL_BLOCK
 #define MM_SMALL_BLOCK 64
 #endif
 constexpr int kSmallBlock = MM_SMALL_BLOCK;
 constexpr int kLargeBlock = 256;
-inline int block_threads_for(uint32_t spp) { return spp <= (uint32_t)kSmallBlock ? kSmallBlock : kLargeBlock; }
+constexpr int kHugeBlock = 1024;
+constexpr uint32_t kMaxSpp = kHugeBlock;       // a pixel never spans blocks
+inline int block_threads_for(uint32_t spp) {
+    return spp <= (uint32_t)kSmallBlock ? kSmallBlock : (spp <= (uint32_t)kLargeBlock ? kLargeBlock : kHugeBlock);
+}
 
 // Returns the kernel's static properties for the occupancy query and launch.
 // ytab: trace_ytab_kernel / trace_tail_kernel<..., true> (the y-table traversal) instead of trace_kernel.

@@ -11,6 +11,8 @@ use std::os::raw::{c_char, c_int};
 #[repr(C)] #[derive(Clone, Copy, Default, Debug)] pub struct Camera { pub camera_center: Float3, pub focal_length: f32, pub rotation: Float4, pub viewport: Float2 }
 #[repr(C)] #[derive(Clone, Copy, Default, Debug)] pub struct Uniform { pub cam: Camera, pub view_width: f32, pub view_height: f32, pub chunk_width: u32, pub time: u32 }
 #[repr(C)] #[derive(Clone, Copy, Default, Debug)] pub struct Chunk { pub x: u32, pub y: u32 }
+/// `spp`: a power of two in 1..=1024 (`chunk_width^2 * spp <= 2^20`); `chunk_width = 1, spp = 1024` is the reference's
+/// one-pixel-per-threadgroup dispatch.  Anything else returns `MM_ERR_UNSUPPORTED`.
 #[repr(C)] #[derive(Clone, Copy, Default, Debug)]
 pub struct Params { pub spp: u32, pub bounce_limit: u32, pub mirror_limit: u32, pub grid_x: u32, pub grid_y: u32,
                     pub group_first: u32, pub group_step: u32, pub group_count: u32, pub flags: u32 }
