@@ -167,7 +167,8 @@ constexpr uint32_t kFormMixed = 1u, kFormRcp = 2u, kFormAxis = 4u, kFormYTable =
 // without the divide-free rect test) runs the mixed form, any other the y-table (YT), reciprocal-multiply or plain packed
 // form, with the axis-aligned rect test where the scene has it.  lit: this lane's ray is literal; form: the kForm* bits of
 // the instantiation that ran, written only when FORM (so that the bounce loop compiles exactly as without it).  YT: the host
-// selects it only without MM_FLAG_RCP_SLAB; ytab is the lane's column of the y-table in dynamic shared memory.
+// selects it only without MM_FLAG_RCP_SLAB; ytab is the lane's column of the y-table in dynamic shared memory, as a
+// shared-window address (table_column).
 template <bool CNT, bool YT, bool FORM = false>
 __device__ __forceinline__ Hit warp_traverse(const KParams &P, uint32_t root, const bool &alive, const V3 &ori, const V3 &dir, const float &t,
                                              const uint32_t &slot, Tally &tl, uint32_t ytab, bool &lit, uint32_t &form) {
@@ -242,7 +243,7 @@ template <bool CNT, bool DBG, bool YT, int kBlockThreads, bool MV = false>
 __device__ __forceinline__ void trace_body(const KParams &P, const ViewRec *views = nullptr) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     float *red = reinterpret_cast<float *>(smem_raw);                      // 3 * kBlockThreads floats
-    const uint32_t ytab = YT ? 3u * kBlockThreads * sizeof(float) + (threadIdx.x >> 5) * P.n_yiv * kYEntryStride + (threadIdx.x & 31u) * 8u : 0u;
+    const uint32_t ytab = YT ? table_column(3u * kBlockThreads * sizeof(float) + (threadIdx.x >> 5) * P.n_yiv * kYEntryStride + (threadIdx.x & 31u) * 8u) : 0u;
 
     const uint64_t path = (uint64_t)blockIdx.x * kBlockThreads + threadIdx.x;
     const bool active = path < P.total_paths;
@@ -348,7 +349,7 @@ __device__ __forceinline__ void tail_body(const KParams &P, const ViewRec *views
     const unsigned long long head = P.counters->tail_paths;                // written by trace_kernel, the launch before
     const uint32_t nq = head < P.tail_cap ? (uint32_t)head : P.tail_cap;
     const uint32_t root = P.root_count ? (kLeafBit | P.root_link | (P.root_count << 24)) : P.root_link;
-    const uint32_t ytab = YT ? (threadIdx.x >> 5) * P.n_yiv * kYEntryStride + (threadIdx.x & 31u) * 8u : 0u;
+    const uint32_t ytab = YT ? table_column((threadIdx.x >> 5) * P.n_yiv * kYEntryStride + (threadIdx.x & 31u) * 8u) : 0u;
     const uint32_t words = 4u + 3u * P.spp;
     Tally tl = {0u, 0u, 0u, 0u};
     uint32_t seg = 0, nhits = 0, nliteral = 0;
@@ -416,7 +417,7 @@ probe_rays_kernel(const __grid_constant__ KParams P, const float *__restrict__ r
     const uint32_t i = blockIdx.x * kProbeBlock + threadIdx.x;
     const bool has = i < n;
     const uint32_t root = P.root_count ? (kLeafBit | P.root_link | (P.root_count << 24)) : P.root_link;
-    const uint32_t ytab = YT ? (threadIdx.x >> 5) * P.n_yiv * kYEntryStride + (threadIdx.x & 31u) * 8u : 0u;
+    const uint32_t ytab = YT ? table_column((threadIdx.x >> 5) * P.n_yiv * kYEntryStride + (threadIdx.x & 31u) * 8u) : 0u;
     V3 ori = mk(0.0f, 0.0f, 0.0f), dir = mk(1.0f, 1.0f, 1.0f);
     float t = 1e30f;
     uint32_t slot = 0xFFFFFFFFu;

@@ -111,6 +111,12 @@ __device__ __forceinline__ f2 add2(f2 a, f2 b) { f2 d; asm("add.rn.f32x2 %0, %1,
 __device__ __forceinline__ f2 mul2(f2 a, f2 b) { f2 d; asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b)); return d; }
 __device__ __forceinline__ f2 fma2(f2 a, f2 b, f2 c) { f2 d; asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(a), "l"(b), "l"(c)); return d; }
 
+// 8-byte shared-memory store / load at a 32-bit shared-window address (the y-table).  Through a generic pointer into dynamic
+// shared memory, every access rebuilds the window base (S2UR SR_CgaCtaId, UMOV, UIADD3, ULEA).  Both are volatile, so they
+// keep their program order: a visit's load of a table entry never moves above the fill's store of it.
+__device__ __forceinline__ void sts64(uint32_t a, f2 v) { asm volatile("st.shared.b64 [%0], %1;" : : "r"(a), "l"(v)); }
+__device__ __forceinline__ f2 lds64(uint32_t a) { f2 v; asm volatile("ld.shared.b64 %0, [%1];" : "=l"(v) : "r"(a)); return v; }
+
 // 32-byte read-only load (LDG.E.256, sm_100+): one instruction and one L1 request per half record.
 struct Line32 { f2 x, y, z, w; };
 __device__ __forceinline__ Line32 ldg256(const void *p) {
@@ -301,9 +307,13 @@ constexpr int kRepUnroll = 2;                      // visits per loop trip: 2 me
 struct Hit { float t; uint32_t slot; };
 // AX = true: the scene's rects are all axis-aligned and `rects` points at RectA records (leaf_step_axis).
 // YT = true (only with MIXED = false, RCP = false): `pairs` points at PairRecY records, and the ray's y quotients of the scene's
-// n_yiv y-intervals y_ivals are first written to the lane's column of the y-table, at byte `ytab` of the dynamic shared memory
-// (entry i at ytab + i * kYEntryStride), with the same operations a visit of the other form performs on them.
+// n_yiv y-intervals y_ivals are first written to the lane's column of the y-table, at shared-window address `ytab` (entry i at
+// ytab + i * kYEntryStride), with the same operations a visit of the other form performs on them.  The caller converts the
+// column to that address once per thread (table_column): converted here, at every call, it would cost the y-table kernels a
+// register across the call and a spill.
 extern __shared__ __align__(16) unsigned char mm_dyn_smem[];
+// The shared-window address of byte `offset` of the dynamic shared memory (the y-table column of a lane).
+__device__ __forceinline__ uint32_t table_column(uint32_t offset) { return (uint32_t)__cvta_generic_to_shared(mm_dyn_smem) + offset; }
 template <bool MIXED, bool CNT, bool RCP, bool AX = false, bool YT = false>
 __device__ __noinline__ Hit traverse(const void *__restrict__ pairs, const void *__restrict__ rects, uint32_t root, bool alive,
                                      bool lit, V3 ori, V3 dir, float beam_t, uint32_t beam_slot, Tally *tlp,
@@ -318,12 +328,12 @@ __device__ __noinline__ Hit traverse(const void *__restrict__ pairs, const void 
     if (YT) {
         const f2 no_yy = pack2(-ori.y, -ori.y), nd_yy = pack2(-dir.y, -dir.y), r_yy = pack2(ry, ry), rl_yy = pack2(rly, rly);
         const uint32_t sy = dir.y < 0.0f ? 8u : 0u;
+        // A branch out, not a predicate per slot: the warp issues only the scene's n_yiv slots (5 for every maze).
 #pragma unroll
         for (uint32_t i = 0; i < kMaxYIntervals; i++) {
-            if (i < n_yiv) {
-                const f2 b = __ldg(reinterpret_cast<const f2 *>(reinterpret_cast<const char *>(y_ivals + i) + sy));   // (near.y, far.y)
-                *reinterpret_cast<f2 *>(mm_dyn_smem + ytab + i * kYEntryStride) = quot2<false>(b, no_yy, nd_yy, r_yy, rl_yy);
-            }
+            if (i >= n_yiv) break;
+            const f2 b = __ldg(reinterpret_cast<const f2 *>(reinterpret_cast<const char *>(y_ivals + i) + sy));   // (near.y, far.y)
+            sts64(ytab + i * kYEntryStride, quot2<false>(b, no_yy, nd_yy, r_yy, rl_yy));
         }
         k.no_xy = pack2(-ori.x, -ori.x); k.nd_xy = pack2(-dir.x, -dir.x); k.r_xy = pack2(rx, rx); k.rl_xy = pack2(rlx, rlx);
     } else {
@@ -363,8 +373,7 @@ __device__ __noinline__ Hit traverse(const void *__restrict__ pairs, const void 
                         asm("mov.b64 %0, {%1, %2};" : "=l"(aL) : "r"(z_lo + cur), "r"(hi_z));
                         const Line32 xz = ldg256(reinterpret_cast<const void *>(aXZ));
                         const uint4 lk = __ldg(reinterpret_cast<const uint4 *>(aL));
-                        const f2 y0 = *reinterpret_cast<const f2 *>(mm_dyn_smem + ytab + lk.z);
-                        const f2 y1 = *reinterpret_cast<const f2 *>(mm_dyn_smem + ytab + lk.w);
+                        const f2 y0 = lds64(ytab + lk.z), y1 = lds64(ytab + lk.w);
                         inner_step_ytab<CNT>(xz, y0, y1, make_uint2(lk.x, lk.y), k, t, cur, sp, stack, tl);
                     } else if (!MIXED || !lit) {
                         // 32-B load for (A, B): measured 1.5 % faster than two 16-B loads; folding (Z, link) into a second
