@@ -860,6 +860,7 @@ static int present_impl(mm_ctx *ctx, float *out_rgba, bool q8, uint8_t *out_rgba
     const size_t n_px = (size_t)ctx->screen_w * ctx->screen_h, bytes = n_px * 4 * sizeof(float);
     if (!ctx->d_screen2) CK(cudaMalloc(&ctx->d_screen2, bytes));
     if (out_rgba8 && !ctx->d_screen8) CK(cudaMalloc(&ctx->d_screen8, n_px * 4));
+    if (out_rgba8 && ctx->present_in_flight) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_copy, 0));   // mm_present_async_rgba8's texels have left the device
     CK(launch_blur(ctx->d_screen, ctx->d_screen2, ctx->screen_w, ctx->screen_h, ctx->stream, q8, out_rgba8 ? ctx->d_screen8 : nullptr));
     float *t = ctx->d_screen; ctx->d_screen = ctx->d_screen2; ctx->d_screen2 = t;   // the blurred image is the screen now
     if (out_rgba) CK(cudaMemcpyAsync(out_rgba, ctx->d_screen, bytes, cudaMemcpyDeviceToHost, ctx->stream));

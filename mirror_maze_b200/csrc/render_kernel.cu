@@ -728,11 +728,9 @@ __global__ void div3_selftest_kernel(unsigned long long *mismatches) {
 }
 
 // fragment_shader's 5-tap blur (shaders.metal:214-225), ping-pong.  HBM-bound: 16 B read + 16 B written per pixel (the four
-// neighbour taps hit L1/L2).  One thread handles two horizontally adjacent pixels (8 loads for 2 pixels instead of 10).
-__device__ __forceinline__ void blur_body(const float4 *__restrict__ src, float4 *__restrict__ dst, uint32_t W, uint32_t H, bool q8,
-                                          uchar4 *__restrict__ bytes) {
-    const uint32_t x0 = 2u * (blockIdx.x * blockDim.x + threadIdx.x), y = blockIdx.y;
-    if (x0 >= W || y >= H) return;
+// neighbour taps hit L1/L2).  One thread handles two horizontally adjacent pixels (8 loads for 2 pixels instead of 10) of row y.
+__device__ __forceinline__ void blur_row(const float4 *__restrict__ src, float4 *__restrict__ dst, uint32_t W, uint32_t H, bool q8,
+                                         uchar4 *__restrict__ bytes, uint32_t x0, uint32_t y) {
     const float4 zero = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
     const size_t row = (size_t)y * W;
     const bool two = x0 + 1 < W;
@@ -752,6 +750,14 @@ __device__ __forceinline__ void blur_body(const float4 *__restrict__ src, float4
         bytes[row + x0] = make_uchar4((unsigned char)unorm8(o0.x), (unsigned char)unorm8(o0.y), (unsigned char)unorm8(o0.z), (unsigned char)unorm8(o0.w));
         if (two) bytes[row + x0 + 1] = make_uchar4((unsigned char)unorm8(o1.x), (unsigned char)unorm8(o1.y), (unsigned char)unorm8(o1.z), (unsigned char)unorm8(o1.w));
     }
+}
+// Rows from blockIdx.y in steps of gridDim.y: grid.y is capped at kBlurRows (the hardware allows 65535), the view height is not.
+constexpr uint32_t kBlurRows = 65535;
+__device__ __forceinline__ void blur_body(const float4 *__restrict__ src, float4 *__restrict__ dst, uint32_t W, uint32_t H, bool q8,
+                                          uchar4 *__restrict__ bytes) {
+    const uint32_t x0 = 2u * (blockIdx.x * blockDim.x + threadIdx.x);
+    if (x0 >= W) return;
+    for (uint32_t y = blockIdx.y; y < H; y += gridDim.y) blur_row(src, dst, W, H, q8, bytes, x0, y);
 }
 __global__ void __launch_bounds__(256) blur_kernel(const float4 *__restrict__ src, float4 *__restrict__ dst, uint32_t W, uint32_t H, bool q8,
                                                    uchar4 *__restrict__ bytes) {
@@ -900,7 +906,7 @@ cudaError_t launch_scatter_all(const float *gathered, float *image, const mm_chu
 
 cudaError_t launch_blur(const float *src, float *dst, uint32_t W, uint32_t H, cudaStream_t stream, bool quant8, uint8_t *bytes) {
     if (W == 0 || H == 0) return cudaSuccess;
-    dim3 grid((W + 511) / 512, H);                                            // two pixels per thread
+    dim3 grid((W + 511) / 512, std::min(H, kBlurRows));                       // two pixels per thread
     blur_kernel<<<grid, 256, 0, stream>>>(reinterpret_cast<const float4 *>(src), reinterpret_cast<float4 *>(dst), W, H, quant8,
                                           reinterpret_cast<uchar4 *>(bytes));
     return cudaGetLastError();
@@ -908,7 +914,7 @@ cudaError_t launch_blur(const float *src, float *dst, uint32_t W, uint32_t H, cu
 
 cudaError_t launch_blur_views(const float *src, float *dst, uint32_t W, uint32_t H, uint32_t n, cudaStream_t stream, bool quant8, uint8_t *bytes) {
     if (W == 0 || H == 0 || n == 0) return cudaSuccess;
-    dim3 grid((W + 511) / 512, H, n);                                         // two pixels per thread, one z slice per screen
+    dim3 grid((W + 511) / 512, std::min(H, kBlurRows), n);                    // two pixels per thread, one z slice per screen
     blur_views_kernel<<<grid, 256, 0, stream>>>(reinterpret_cast<const float4 *>(src), reinterpret_cast<float4 *>(dst), W, H, quant8,
                                                 reinterpret_cast<uchar4 *>(bytes));
     return cudaGetLastError();

@@ -6,7 +6,8 @@ import torch
 import mirror_maze_b200 as mm
 
 r = mm.Renderer(0)
-peak = json.load(open(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "MEASURED_PEAKS.json"))).get("hbm_gbs", 6650.0)
+peaks_path = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "MEASURED_PEAKS.json")
+peak = json.load(open(peaks_path)).get("hbm_gbs", 6650.0) if os.path.exists(peaks_path) else 6650.0   # the file is written per machine, not committed
 stream = torch.cuda.Stream()
 r.set_stream(stream.cuda_stream)
 for W, H in ((1920, 1080), (3840, 2160), (7680, 4320)):
